@@ -2,7 +2,7 @@
 """bench.py — alignment-evaluation throughput (similarity + CSLS + rank -> Hits@k / MR / MRR) on synthetic
 DBP15K/FBDB15K-shaped data, the headline metric of BASELINE.json, on N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl snag|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl snag|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -63,6 +63,8 @@ DEFAULT_WORKLOAD = "c4_1m"
 SEED = 3408                       # the reference's scripted seed (run.sh:2)
 CPU_SAMPLE_N = 8192               # bounded sample for the CPU legs: a CPU_SAMPLE_N x CPU_SAMPLE_N sub-problem (~1 s per pass on
                                   # 16 host threads: 4 passes of the cpu_baseline leg, K + W passes of the reference arm)
+DUMP_ROWS = 512                   # --dump-outputs: gradient rows kept per table of a training slice (fixed, seeded choice), so
+                                  # that the default line (c4_1m + c5_train + c1_train) writes about 53 MB
 
 
 # ================================================================================================ helpers
@@ -144,6 +146,18 @@ def synth_tables(n: int, d: int, sigma: float, device, chunk: int = 65536):
     return emb, left, right
 
 
+def dump_outputs(out_dir: str, prefix: str, arrays: dict):
+    """--dump-outputs: writes every tensor of `arrays` as out_dir/<prefix>.<name>.npy, floating point as float32 and
+    integers (ranks) as float64, which holds every int32 exactly."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for nm, t in arrays.items():
+        t = t.detach().cpu()
+        a = t.float().numpy() if t.is_floating_point() else t.to(torch.float64).numpy()
+        np.save(os.path.join(out_dir, f"{prefix}.{nm}.npy"), a)
+
+
 # ================================================================================================ CPU legs
 def cpu_port_sample(n_s: int, d: int, k: int, sigma: float, steps: int, warmup: int):
     """Times the oracle port (oracle/snag_oracle.c, all host threads) on an n_s x n_s sub-problem of the workload."""
@@ -206,7 +220,7 @@ def run_reference(args, name, n, d, k, sigma, desc):
     if rank != 0:
         return                      # under torchrun only rank 0 times the CPU arm; the others exit 0 without work
     n_s = min(CPU_SAMPLE_N, n)
-    cb = cpu_port_sample(n_s, d, k, sigma, max(1, args.steps), max(0, args.warmup))
+    cb = cpu_port_sample(n_s, d, k, sigma, args.steps, args.warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_step"], "higher_is_better": True,
@@ -332,7 +346,7 @@ def eval_bench(ctx, args, name):
 
     n, d, k, sigma, desc = WORKLOADS[name]
     world, rank, dev, group, peaks = ctx.world, ctx.rank, ctx.dev, ctx.group, ctx.peaks
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
     emb, left, right = synth_tables(n, d, sigma, dev)
     dpad = ops.round_up(d, 64)
     sweep_events = []                       # (name, start, end) per fused-sweep launch inside the timed region
@@ -359,6 +373,9 @@ def eval_bench(ctx, args, name):
         e1.record()
         ctx.barrier()
     ops.SWEEP_EVENT_SINK = None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, name, {"rank_l2r": res.rank_l2r, "rank_r2l": res.rank_r2l, "nv1": res.nv1,
+                                               "nv2": res.nv2, "g": res.g})
     ms_per_step = ctx.max_over_ranks(e0.elapsed_time(e1) / K)
     launches_per_step = res.launches + 2
     # per-kernel durations of the fused sweeps (this rank), algorithmic flops = 2 * rows * cols * D per launch
@@ -395,12 +412,12 @@ def eval_bench(ctx, args, name):
         torch.cuda.synchronize()
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         g0.record()
-        for _ in range(20):
+        for _ in range(K):
             o = evaluate.evaluate_alignment(emb, left, right, csls=True, csls_k=k)
         g1.record()
         torch.cuda.synchronize()
         same = bool(torch.equal(o["ranks"].rank_l2r, res.rank_l2r) and torch.equal(o["ranks"].rank_r2l, res.rank_r2l))
-        out["graph_replay"] = {"ms_per_step": g0.elapsed_time(g1) / 20, "cuda_graph": bool(o["ranks"].info.get("cuda_graph")),
+        out["graph_replay"] = {"ms_per_step": g0.elapsed_time(g1) / K, "cuda_graph": bool(o["ranks"].info.get("cuda_graph")),
                                "ranks_equal_eager": same,
                                "note": "evaluate_alignment(final_emb, test_left, test_right): input copy + one graph launch "
                                        "+ one 32-byte status read + host Hits/MR/MRR, per evaluation"}
@@ -423,16 +440,15 @@ def eval_bench(ctx, args, name):
     def step_e2e():
         return evaluate.evaluate_alignment_host(host[0, :c1 - c0], host[1, :c1 - c0], n, c0, csls=True, csls_k=k, group=group)
 
-    n_e2e = 2 if n >= 500_000 else 5
     o = step_e2e()
     ctx.barrier()
     t0 = time.perf_counter()
-    for _ in range(n_e2e):
+    for _ in range(K):
         o = step_e2e()
     ctx.barrier()
-    dt = ctx.max_over_ranks((time.perf_counter() - t0) / n_e2e)
+    dt = ctx.max_over_ranks((time.perf_counter() - t0) / K)
     out["e2e"] = {"value": n * n / dt, "unit": UNIT, "h2d_bytes_per_step": int(2 * (c1 - c0) * d * 4),
-                  "d2h_bytes_per_step": int(2 * n * 4), "ms_per_step": dt * 1e3, "steps": n_e2e,
+                  "d2h_bytes_per_step": int(2 * n * 4), "ms_per_step": dt * 1e3, "steps": K,
                   "streamed": bool(o.get("streamed")), "cpus_bound_to_gpu_numa": ctx.cpu_affinity,
                   "note": "per rank: H2D of its slice of both fp32 tables from pinned memory (+ NVLink all-gather of the bf16 "
                           "operands when sharded), evaluation, D2H of both rank vectors, host Hits/MR/MRR; on one GPU the "
@@ -525,12 +541,13 @@ def cpu_icl_sample(B_s, M, dm, steps, B_full=None):
 
 def train_bench(ctx, args, name, cpu_leg=True):
     """The loss-layer slice `name` (2 + 2M icl_loss calls, forward + backward) on ctx.world GPUs -> bench-line fields."""
+    import numpy as np
     import torch
     from snag_b200 import loss as sloss, ops
 
     B, M, dm, desc = TRAIN_WORKLOADS[name]
     world, rank, dev, group, peaks = ctx.world, ctx.rank, ctx.dev, ctx.group, ctx.peaks
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
     streams, hidden, joint, joint_fz, wn, links, leaves = _train_tables(B, M, dm, dev)
     layer = sloss.SnagLossLayer(tau=0.1, ab_weight=0.5).to(dev)       # --awloss 0 (config.py:114): the reference's default
     links_pinned = torch.from_numpy(links).pin_memory()
@@ -592,9 +609,15 @@ def train_bench(ctx, args, name, cpu_leg=True):
             ctx.barrier()
             e0.record()
             for _ in range(K):
-                step(False)
+                loss = step(False)
             e1.record()
             ctx.barrier()
+        if args.dump_outputs and grads_mode == "local" and rank == 0:
+            rows = torch.from_numpy(np.sort(np.random.RandomState(SEED + 2).choice(wn.shape[0], DUMP_ROWS, replace=False)))
+            named = [(f"stream{m}", t) for m, t in enumerate(streams)] + [(f"hidden{m}", t) for m, t in enumerate(hidden)]
+            named += [("joint", joint), ("joint_fz", joint_fz), ("weight_norm", wn)]
+            dump_outputs(args.dump_outputs, name, {"loss": loss.reshape(1), **{f"grad_{nm}": t.grad[rows.to(dev)]
+                                                                                for nm, t in named if t is not None}})
         ms = ctx.max_over_ranks(e0.elapsed_time(e1) / K)
         # end to end: the step's input (the batch of links) comes from pinned host memory, the loss goes back to the host
         step(True)
@@ -901,7 +924,9 @@ def run_train(args, name):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="steps of every GPU timed loop: the device-resident steps, the end-to-end steps and the CUDA-graph "
+                         "replays of the small evaluations (a short window makes the last two noisier)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default=os.environ.get("SNAG_BENCH_WORKLOAD", DEFAULT_WORKLOAD), choices=sorted(WORKLOADS) + sorted(TRAIN_WORKLOADS))
     ap.add_argument("--impl", default="snag", choices=["snag", "reference"])
@@ -911,7 +936,17 @@ def main():
     ap.add_argument("--no-context", action="store_true", help="skip the snag_step / reference_gpu_eager context legs")
     ap.add_argument("--profile-run", action="store_true",
                     help="only the device-resident timed region (for runs under ncu); e2e and CPU legs are skipped")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each GPU workload computed as DIR/<workload>.<name>.npy: the rank "
+                         "vectors, CSLS neighbourhood means and ground-truth distances of an evaluation; the loss and a "
+                         f"fixed sample of {DUMP_ROWS} rows of every input gradient of a training slice. Rank 0 writes what it "
+                         "received: with --gpus N > 1 a training gradient holds only the rows of rank 0's own anchors "
+                         "(zeros elsewhere), not the full gradient")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "snag":
+        ap.error("--dump-outputs writes the outputs of --impl snag")
     if args.workload in TRAIN_WORKLOADS:
         run_train(args, args.workload)
         return

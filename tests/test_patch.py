@@ -5,6 +5,7 @@ from __future__ import annotations
 
 import inspect
 import logging
+import math
 import os
 import sys
 import types
@@ -93,6 +94,25 @@ def test_signatures_match_reference():
     assert _sig(importlib.import_module("model.SNAG_tools").MformerFusion.forward) == _sig(fusion.MformerFusion_forward)
     from snag_b200 import seeds
     assert _sig(importlib.import_module("src.data").visual_pivot_induction) == _sig(seeds.visual_pivot_induction)
+
+
+def test_signatures_match_the_recorded_reference_signatures():
+    """Without a reference checkout: the call signatures SURVEY.md §(a) recorded from the reference (model/SNAG_loss.py,
+    src/utils.py:202,417, main.py:359) — parameter names, order and defaults — against the mirrors."""
+    from snag_b200 import evaluate, loss, runner
+    P = inspect.Parameter.POSITIONAL_OR_KEYWORD
+    E = inspect.Parameter.empty
+    recorded = {
+        loss.icl_loss.forward: [("self", E), ("emb", E), ("train_links", E), ("neg_l", None), ("neg_r", None),
+                                ("weight_norm", None), ("norm", True)],
+        loss.ial_loss.forward: [("self", E), ("src_emb", E), ("tar_emb", E), ("train_links", E), ("norm", True)],
+        evaluate.pairwise_distances: [("x", E), ("y", None)],
+        evaluate.csls_sim: [("sim_mat", E), ("k", E)],
+        runner._test: [("self", E), ("test_left", E), ("test_right", E), ("last_epoch", False), ("save_name", ""),
+                       ("loss", None)],
+    }
+    for f, want in recorded.items():
+        assert _sig(f) == [(n, P, d) for n, d in want], f.__qualname__
 
 
 @needs_ref
@@ -215,6 +235,75 @@ def test_mformer_fusion_mirror_on_cpu(monkeypatch, name):
                                   use_intermediate=1)
     mod = tools.MformerFusion(args, modal_num=M, with_weight=1)
     mod.load_state_dict(torch.load(io.BytesIO(fx["state"].tobytes())))
+    mod.eval()
+
+    def cpu_tail(embs, weight_norm, weight_norm_fz):
+        j, jf = oracle.joint_fuse([e.detach().numpy() for e in embs], weight_norm.detach().numpy(),
+                                  weight_norm_fz.detach().numpy())
+        return torch.from_numpy(j), torch.from_numpy(jf)
+    monkeypatch.setattr(fusion, "joint_embeddings", cpu_tail)
+    embs = [torch.from_numpy(fx[f"emb{m}"]) for m in range(M)] + [None] * (6 - M)
+    with torch.no_grad():
+        joint, joint_fz, hidden, weight_norm = fusion.MformerFusion_forward(mod, embs)
+    np.testing.assert_allclose(weight_norm.numpy(), fx["weight_norm"], rtol=0, atol=1e-6)
+    np.testing.assert_allclose(hidden.numpy(), fx["hidden"], rtol=0, atol=1e-5)
+    np.testing.assert_allclose(joint.numpy(), fx["joint"], rtol=0, atol=2e-6)
+    np.testing.assert_allclose(joint_fz.numpy(), fx["joint_fz"], rtol=0, atol=2e-6)
+
+
+class _BertSelfAttention(torch.nn.Module):
+    def __init__(self, D):
+        super().__init__()
+        self.query, self.key, self.value = torch.nn.Linear(D, D), torch.nn.Linear(D, D), torch.nn.Linear(D, D)
+
+
+class _DenseNorm(torch.nn.Module):
+    def __init__(self, d_in, D):
+        super().__init__()
+        self.dense, self.LayerNorm = torch.nn.Linear(d_in, D), torch.nn.LayerNorm(D, eps=1e-12)
+
+
+class _BertLayer(torch.nn.Module):
+    """A BERT encoder layer (post-LayerNorm, eps 1e-12, erf GELU) under the parameter names of the reference's
+    fusion_layer. With the weights stored in the fusion golden files it reproduces the hidden states the reference
+    recorded there exactly, so it can stand in for the reference's layer where no reference checkout exists."""
+
+    def __init__(self, D, heads):
+        super().__init__()
+        self.heads = heads
+        self.attention = torch.nn.Module()
+        self.attention.self, self.attention.output = _BertSelfAttention(D), _DenseNorm(D, D)
+        self.intermediate = torch.nn.Module()
+        self.intermediate.dense = torch.nn.Linear(D, 2 * D)
+        self.output = _DenseNorm(2 * D, D)
+
+    def forward(self, x, output_attentions=False):
+        N, M, D = x.shape
+        sa, hd = self.attention.self, D // self.heads
+        split = lambda t: t.view(N, M, self.heads, hd).permute(0, 2, 1, 3)
+        q, k, v = split(sa.query(x)), split(sa.key(x)), split(sa.value(x))
+        probs = torch.softmax(q @ k.transpose(-1, -2) / math.sqrt(hd), dim=-1)
+        ctx = (probs @ v).permute(0, 2, 1, 3).reshape(N, M, D)
+        a = self.attention.output.LayerNorm(self.attention.output.dense(ctx) + x)
+        y = self.output.LayerNorm(self.output.dense(torch.nn.functional.gelu(self.intermediate.dense(a))) + a)
+        return (y, probs) if output_attentions else (y,)
+
+
+@pytest.mark.parametrize("name", ["fusion_m4_d64", "fusion_m6_d96"])
+def test_mformer_fusion_mirror_on_recorded_reference_outputs(monkeypatch, name):
+    """Without a reference checkout: the drop-in MformerFusion.forward, run on a module that carries the reference
+    module's stored weights (fusion_layer through _BertLayer, weight_raw), reproduces the outputs the reference's forward
+    recorded in the golden file, with the CUDA tail replaced by the oracle's restatement as in the test above."""
+    import io
+    from snag_b200 import fusion
+    from tests.conftest import load_golden
+    fx = load_golden(name)
+    M, D, heads = int(fx["M"]), int(fx["D"]), int(fx["heads"])
+    mod = torch.nn.Module()
+    mod.args = types.SimpleNamespace(num_attention_heads=heads)
+    mod.fusion_layer = torch.nn.ModuleList([_BertLayer(D, heads)])
+    mod.weight_raw = torch.nn.Parameter(torch.zeros(6))
+    mod.load_state_dict(torch.load(io.BytesIO(fx["state"].tobytes())), strict=True)
     mod.eval()
 
     def cpu_tail(embs, weight_norm, weight_norm_fz):
