@@ -352,6 +352,47 @@ int snag_l1_distance(const float* x, const float* y, int64_t n1, int64_t n2, int
  * column j. Used by the --distance 1 path, where no contraction exists to fuse the counting into. */
 int snag_matrix_rank(const float* d, int64_t n, int64_t ld, int32_t* cnt_row, int32_t* cnt_col, void* stream);
 
+/* ---- fused --distance 1 evaluation (no n x n matrix; the same generator as the L2 sweeps drives it) ------------------ */
+/* Operands X [n1][Dp], Y [n2][Dp] are fp32 rows zero padded to Dp (a multiple of 8), 16-byte aligned; xn / yn are the
+ * rows' L1 norms (sum of |x_k|, fp32). The CUDA-core sweep computes d~_ij = sum_k |x_ik - y_jk| in fp32 with packed adds
+ * and |d~ - d| <= (ceil(Dp / 32) + 18) 2^-24 1.01 (xn_i + yn_j) against the canonical d = fp32 of the fp64 index-order
+ * sum (scipy's cdist). snag_l1_plan: number of partial lists per row (n_lists) of an [n_rows x n_cols] sweep. */
+int snag_l1_plan(int32_t n_rows, int32_t n_cols, int32_t Dp, int32_t* n_lists);
+/* part / part_idx [n_lists][n1][SNAG_KT]: per list, the SNAG_KT largest c~ = 1 - d~ of every row (ascending, -inf / -1
+ * padded) and their columns — the input of snag_topk_merge_mean, as from snag_eval_rowtopk. */
+int snag_l1_rowtopk(const float* X, const float* Y, int32_t n1, int32_t n2, int32_t Dp, float* part, int32_t* part_idx,
+                    void* stream);
+/* Rank counts with a deferral band, as snag_eval_rank_band: dist~ = 1 - ((2 (1 - d~) - nv1_i) - nv2_j) (use_csls) or d~
+ * is compared with g_row[i] and g_col[j]; clear "less" is counted into cnt_row / cnt_col, elements within the pair's
+ * error bound are appended to band[] (x = row | direction flags << 30, y = column; *band_cnt may exceed band_cap: re-run
+ * with a larger list) for snag_l1_band_rescore. top4_val / top4_idx (both NULL or [n_lists][n1][4]): each row's 4
+ * nearest (x = -dist~, column gid) per list, for snag_top4_merge. Zero *band_cnt first. */
+int snag_l1_rank_band(const float* X, const float* Y, const float* xn, const float* yn, const float* nv1, const float* nv2,
+                      const float* g_row, const float* g_col, int32_t row_gid0, int32_t col_gid0, int32_t n1, int32_t n2,
+                      int32_t Dp, int32_t use_csls, int32_t* cnt_row, int32_t* cnt_col, float* top4_val, int32_t* top4_idx,
+                      uint64_t* band, uint32_t* band_cnt, uint32_t band_cap, void* stream);
+/* Canonical CSLS neighbourhood means of the rows of A from their merged sweep candidates (as snag_topk_rescore, with
+ * bn_max = the largest L1 norm of B); unverifiable rows are appended to flagged[] for snag_l1_topk_exhaustive. */
+int snag_l1_topk_rescore(const float* A, const float* B, int32_t Dp, int64_t n_rows, const float* an, float bn_max,
+                         const int32_t* cand_idx, const float* cand_val, int32_t k, float* nv, int32_t* flagged,
+                         int32_t* flagged_cnt, int32_t flagged_cap, void* stream);
+int snag_l1_topk_exhaustive(const float* A, const float* B, int32_t Dp, int64_t n_b, const int32_t* flagged,
+                            const int32_t* flagged_cnt, int32_t flagged_cap, int32_t k, float* nv, void* stream);
+/* g[p] = canonical (CSLS) distance of pair (x_p, y_p) */
+int snag_l1_pair_score(const float* X, const float* Y, int32_t Dp, int64_t n, const float* nv1, const float* nv2,
+                       int32_t use_csls, float* g, void* stream);
+/* the deferred elements of snag_l1_rank_band judged canonically with the stable-sort tie-break */
+int snag_l1_band_rescore(const float* X, const float* Y, int32_t Dp, const float* nv1, const float* nv2, const float* g_row,
+                         const float* g_col, int32_t row_gid0, int32_t col_gid0, int32_t use_csls, const uint64_t* band,
+                         const uint32_t* band_cnt, uint32_t band_cap, int32_t* cnt_row, int32_t* cnt_col, void* stream);
+/* cand [n_rows][4] merged sweep candidates (ids into Y, 0x7fffffff = empty) -> canonical distances ascending (id
+ * ascending on ties); rows whose 4th sweep candidate cannot rule out an outsider in the canonical top 3 (yn_max / nv2_absmax:
+ * the largest L1 norm of Y and |nv2|) are appended to flagged[] (n_rows entries, *flagged_cnt zeroed by the caller) and
+ * rescanned against all n_b rows of Y in the same call. */
+int snag_l1_top3_rescore(const float* X, const float* Y, int32_t Dp, int64_t n_rows, int64_t n_b, const float* xn, float yn_max,
+                         const float* nv1, const float* nv2, float nv2_absmax, int32_t use_csls, const int32_t* cand, float* oval,
+                         int32_t* oidx, int32_t* flagged, int32_t* flagged_cnt, void* stream);
+
 /* ---- mutual nearest neighbours (iterative-learning link mining) ------------------------------- */
 /* The argmin pair of model/SNAG.py:192-208 (Iter_new_links: torch.argmin over the rows and over the columns of
  * pairwise_distances(final_emb[left], final_emb[right])) without forming the distance matrix.

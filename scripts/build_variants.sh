@@ -6,7 +6,7 @@ mkdir -p snag_b200/_variants
 build() {  # name, extra flags
   name=$1; shift
   objs=""
-  for f in abi bw_kernels sim_kernels icl_fused icl_fwd_sym; do
+  for f in abi bw_kernels sim_kernels icl_fused icl_fwd_sym l1_sweep; do
     nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC --expt-relaxed-constexpr "$@" \
       -c snag_b200/csrc/$f.cu -o snag_b200/_variants/${name}_$f.o &
     objs="$objs snag_b200/_variants/${name}_$f.o"

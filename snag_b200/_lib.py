@@ -38,6 +38,15 @@ _SIGNATURES = {
     "snag_normalize_bwd_scatter_many": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp],
     "snag_l1_distance": [_vp, _vp, _i64, _i64, _i32, _i64, _i64, _vp, _i64, _vp],
     "snag_matrix_rank": [_vp, _i64, _i64, _vp, _vp, _vp],
+    "snag_l1_plan": [_i32, _i32, _i32, C.POINTER(_i32)],
+    "snag_l1_rowtopk": [_vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp],
+    "snag_l1_rank_band": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp,
+                          _vp, _u32, _vp],
+    "snag_l1_topk_rescore": [_vp, _vp, _i32, _i64, _vp, _f32, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _vp],
+    "snag_l1_topk_exhaustive": [_vp, _vp, _i32, _i64, _vp, _vp, _i32, _i32, _vp, _vp],
+    "snag_l1_pair_score": [_vp, _vp, _i32, _i64, _vp, _vp, _i32, _vp, _vp],
+    "snag_l1_band_rescore": [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _u32, _vp, _vp, _vp],
+    "snag_l1_top3_rescore": [_vp, _vp, _i32, _i64, _i64, _vp, _f32, _vp, _vp, _f32, _i32, _vp, _vp, _vp, _vp, _vp, _vp],
     "snag_icl_bwd_fused": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _f32, _i32, _i64, _vp],
     "snag_sim_write": [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _i64, _vp],
     "snag_sim_write_t": [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _i64, _i64, _vp],

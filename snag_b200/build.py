@@ -18,7 +18,7 @@ PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 BUILD_DIR = PKG_DIR / "_build"
 LIB_PATH = PKG_DIR / "libsnag_b200.so"
-SOURCES = ["abi.cu", "bw_kernels.cu", "sim_kernels.cu", "icl_fused.cu", "icl_fwd_sym.cu"]
+SOURCES = ["abi.cu", "bw_kernels.cu", "sim_kernels.cu", "icl_fused.cu", "icl_fwd_sym.cu", "l1_sweep.cu"]
 HEADERS = ["common.cuh", "simgemm.cuh", "snag_internal.h", "../../include/snag_b200.h"]
 
 NVCC_FLAGS = [

@@ -108,6 +108,51 @@ int snag_l1_distance(const float* x, const float* y, int64_t n1, int64_t n2, int
 int snag_matrix_rank(const float* d, int64_t n, int64_t ld, int32_t* cnt_row, int32_t* cnt_col, void* stream) {
   return launch_matrix_rank(d, n, ld, cnt_row, cnt_col, S(stream));
 }
+
+int snag_l1_plan(int32_t n_rows, int32_t n_cols, int32_t Dp, int32_t* n_lists) {
+  SimPlan pl;
+  const int rc = l1_plan(n_rows, n_cols, Dp, &pl);
+  if (rc) return rc;
+  if (n_lists) *n_lists = pl.n_lists;
+  return SNAG_OK;
+}
+int snag_l1_rowtopk(const float* X, const float* Y, int32_t n1, int32_t n2, int32_t Dp, float* part, int32_t* part_idx,
+                    void* stream) {
+  return launch_l1_rowtopk(X, Y, n1, n2, Dp, part, part_idx, S(stream));
+}
+int snag_l1_rank_band(const float* X, const float* Y, const float* xn, const float* yn, const float* nv1, const float* nv2,
+                      const float* g_row, const float* g_col, int32_t row_gid0, int32_t col_gid0, int32_t n1, int32_t n2,
+                      int32_t Dp, int32_t use_csls, int32_t* cnt_row, int32_t* cnt_col, float* top4_val, int32_t* top4_idx,
+                      uint64_t* band, uint32_t* band_cnt, uint32_t band_cap, void* stream) {
+  return launch_l1_rank_band(X, Y, xn, yn, nv1, nv2, g_row, g_col, row_gid0, col_gid0, n1, n2, Dp, use_csls, cnt_row, cnt_col,
+                             top4_val, top4_idx, reinterpret_cast<uint2*>(band), band_cnt, band_cap, S(stream));
+}
+int snag_l1_topk_rescore(const float* A, const float* B, int32_t Dp, int64_t n_rows, const float* an, float bn_max,
+                         const int32_t* cand_idx, const float* cand_val, int32_t k, float* nv, int32_t* flagged,
+                         int32_t* flagged_cnt, int32_t flagged_cap, void* stream) {
+  return launch_l1_topk_rescore(A, B, Dp, n_rows, an, bn_max, cand_idx, cand_val, k, nv, flagged, flagged_cnt, flagged_cap,
+                                S(stream));
+}
+int snag_l1_topk_exhaustive(const float* A, const float* B, int32_t Dp, int64_t n_b, const int32_t* flagged,
+                            const int32_t* flagged_cnt, int32_t flagged_cap, int32_t k, float* nv, void* stream) {
+  return launch_l1_topk_exhaustive(A, B, Dp, n_b, flagged, flagged_cnt, flagged_cap, k, nv, S(stream));
+}
+int snag_l1_pair_score(const float* X, const float* Y, int32_t Dp, int64_t n, const float* nv1, const float* nv2,
+                       int32_t use_csls, float* g, void* stream) {
+  return launch_l1_pair_score(X, Y, Dp, n, nv1, nv2, use_csls, g, S(stream));
+}
+int snag_l1_band_rescore(const float* X, const float* Y, int32_t Dp, const float* nv1, const float* nv2, const float* g_row,
+                         const float* g_col, int32_t row_gid0, int32_t col_gid0, int32_t use_csls, const uint64_t* band,
+                         const uint32_t* band_cnt, uint32_t band_cap, int32_t* cnt_row, int32_t* cnt_col, void* stream) {
+  return launch_l1_band_rescore(X, Y, Dp, nv1, nv2, g_row, g_col, row_gid0, col_gid0, use_csls,
+                                reinterpret_cast<const uint2*>(band), band_cnt, band_cap, cnt_row, cnt_col, S(stream));
+}
+int snag_l1_top3_rescore(const float* X, const float* Y, int32_t Dp, int64_t n_rows, int64_t n_b, const float* xn, float yn_max,
+                         const float* nv1, const float* nv2, float nv2_absmax, int32_t use_csls, const int32_t* cand, float* oval,
+                         int32_t* oidx, int32_t* flagged, int32_t* flagged_cnt, void* stream) {
+  return launch_l1_top3_rescore(X, Y, Dp, n_rows, n_b, xn, yn_max, nv1, nv2, nv2_absmax, use_csls, cand, oval, oidx, flagged,
+                                flagged_cnt, S(stream));
+}
 int32_t snag_icl_bwd_fused_splits(int32_t n_prob, int32_t B, int32_t Bp, int32_t row_blocks) {
   return icl_bwd_fused_splits(n_prob, B, Bp, row_blocks);
 }

@@ -56,6 +56,26 @@ int launch_normalize_bwd_scatter_many(int n_prob, const float* const* emb, const
 int launch_l1_distance(const float* x, const float* y, long long n1, long long n2, int D, long long ldx, long long ldy,
                        float* out, long long ldo, cudaStream_t st);
 int launch_matrix_rank(const float* d, long long n, long long ld, int* cnt_row, int* cnt_col, cudaStream_t st);
+// fused --distance 1 evaluation (l1_sweep.cu)
+int l1_plan(int n_rows, int n_cols, int Dp, SimPlan* plan);
+int launch_l1_rowtopk(const float* X, const float* Y, int n1, int n2, int Dp, float* part, int* part_idx, cudaStream_t st);
+int launch_l1_rank_band(const float* X, const float* Y, const float* xn, const float* yn, const float* nv1, const float* nv2,
+                        const float* g_row, const float* g_col, int row_gid0, int col_gid0, int n1, int n2, int Dp,
+                        int use_csls, int* cnt_row, int* cnt_col, float* top4_val, int* top4_idx, uint2* band,
+                        unsigned int* band_cnt, unsigned int band_cap, cudaStream_t st);
+int launch_l1_topk_rescore(const float* A, const float* B, int Dp, long long n_rows, const float* an, float bn_max,
+                           const int* cand_idx, const float* cand_val, int k, float* nv, int* flagged, int* flagged_cnt,
+                           int flagged_cap, cudaStream_t st);
+int launch_l1_topk_exhaustive(const float* A, const float* B, int Dp, long long n_b, const int* flagged, const int* flagged_cnt,
+                              int flagged_cap, int k, float* nv, cudaStream_t st);
+int launch_l1_pair_score(const float* X, const float* Y, int Dp, long long n, const float* nv1, const float* nv2, int use_csls,
+                         float* g, cudaStream_t st);
+int launch_l1_band_rescore(const float* X, const float* Y, int Dp, const float* nv1, const float* nv2, const float* g_row,
+                           const float* g_col, int row_gid0, int col_gid0, int use_csls, const uint2* band,
+                           const unsigned int* band_cnt, unsigned int band_cap, int* cnt_row, int* cnt_col, cudaStream_t st);
+int launch_l1_top3_rescore(const float* X, const float* Y, int Dp, long long n_rows, long long n_b, const float* xn,
+                           float yn_max, const float* nv1, const float* nv2, float nv2_absmax, int use_csls, const int* cand,
+                           float* oval, int* oidx, int* flagged, int* flagged_cnt, cudaStream_t st);
 // fused ICL backward for Dpad <= 320 (icl_fused.cu)
 int icl_bwd_fused_splits(int n_prob, int B, int Bp, int row_blocks);
 int launch_icl_bwd_fused(int n_prob, const __nv_bfloat16* const* S3, const float* const* cr_a, const float* const* cr_b,

@@ -731,24 +731,64 @@ def evaluate_alignment_materialised(final_emb: torch.Tensor, test_left: torch.Te
 
 
 def evaluate_alignment_l1(final_emb: torch.Tensor, test_left: torch.Tensor, test_right: torch.Tensor, csls: bool = True,
-                          csls_k: int = 10, want_top3: bool = False) -> dict:
+                          csls_k: int = 10, want_top3: bool = False, group=None) -> dict:
     """Runner._test with --distance 1 (main.py:379, 387-429). The reference normalises on the device, moves both sides
-    to the host and calls scipy's cdist(metric="cityblock"); the L1 distance is not a contraction, so nothing here is
-    fused: one CUDA kernel materialises the [n, n] fp32 matrix (fp64 index-order sums, like the oracle), the
-    materialised csls_sim kernels apply CSLS and a counting kernel produces both rank vectors."""
+    to the host and calls scipy's cdist(metric="cityblock"). Here the rows are normalised and gathered in torch (the same
+    operands), and the evaluation is the fused one of evaluate_alignment with the L1 kernels of snag_b200.l1: a CUDA-core
+    sweep in fp32 whose verdicts inside its error bound are re-judged with the canonical arithmetic (fp64 index-order
+    sums rounded once, the reference's fp32 CSLS chain), so ranks, nv1 / nv2, g and the prediction ids equal the
+    reference's without the [n, n] matrix. With `group` every rank passes the same final_emb, sweeps its own shard of the
+    targets and gets the full metrics. CSLS neighbourhoods larger than the KT candidates of the fused sweep are evaluated
+    on the materialised matrix (single GPU)."""
     n = test_left.numel()
     if test_right.numel() != n:
         raise ValueError("test_left and test_right must pair up")
+    if csls and csls_k > n:
+        raise ValueError(f"csls_k={csls_k} exceeds the number of evaluated pairs n={n}")
+    materialised = csls and not 1 <= csls_k <= KT
+    if materialised and group is not None:
+        raise SnagError(f"csls_k={csls_k} > {KT}: the materialised evaluation is not sharded")
+    if not final_emb.is_cuda:
+        raise SnagError("evaluate_alignment_l1: final_emb must live on the GPU (there is no CPU path)")
     fe = torch.nn.functional.normalize(final_emb.float())                       # main.py:379
-    x = fe.index_select(0, test_left.to(torch.int64)).contiguous()
-    y = fe.index_select(0, test_right.to(torch.int64)).contiguous()
+    left, right = test_left.to(torch.int64), test_right.to(torch.int64)
+    if materialised:
+        return _evaluate_l1_materialised(fe, left, right, csls_k, want_top3)
+    from . import l1
+    X, xn = l1.prep(fe, left)
+    Y, yn = l1.prep(fe, right)
+    if group is None:
+        world, rank = 1, 0
+    else:
+        import torch.distributed as dist
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+    gen = _align_ranks_steps(l1, X, Y, xn, yn, n, csls_k, csls, want_top3, world, rank, two_sweep=False)
+    if world == 1:
+        try:
+            next(gen)
+        except StopIteration as stop:
+            res = stop.value
+        else:
+            raise AssertionError("single-rank evaluation requested a collective")
+    else:
+        res = _drive_with_torch_distributed(gen, group)
+    res.info["distance"] = 1
+    return {"l2r": metrics_from_ranks(res.rank_l2r), "r2l": metrics_from_ranks(res.rank_r2l), "ranks": res,
+            "launches": res.launches + 2}
+
+
+def _evaluate_l1_materialised(fe: torch.Tensor, left: torch.Tensor, right: torch.Tensor, csls_k: int, want_top3: bool) -> dict:
+    """CSLS with csls_k > KT on --distance 1: the reference's composition on the materialised [n, n] fp32 matrix
+    (fp64 index-order L1 sums, csls_sim on 1 - distance, counting ranks with the stable-sort tie-break)."""
+    n = left.numel()
+    free, _total = torch.cuda.mem_get_info(fe.device)
+    if 3 * 4 * n * n > free:
+        raise SnagError(f"csls_k={csls_k} > {KT} needs the materialised {n} x {n} matrix, which does not fit this device")
+    x = fe.index_select(0, left).contiguous()
+    y = fe.index_select(0, right).contiguous()
     dist = _cuda_ops.l1_distance(x, y)
-    nv1 = nv2 = None
-    if csls:
-        if csls_k > n:
-            raise ValueError(f"csls_k={csls_k} exceeds the number of evaluated pairs n={n}")
-        out, nv1, nv2 = _cuda_ops.csls_sim_matrix(1 - dist, int(csls_k))         # main.py:393
-        dist = 1 - out
+    out, nv1, nv2 = _cuda_ops.csls_sim_matrix(1 - dist, int(csls_k))             # main.py:393
+    dist = 1 - out
     rank_l2r, rank_r2l = _cuda_ops.matrix_rank(dist)
     top3_idx = top3_val = None
     if want_top3:
