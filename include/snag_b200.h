@@ -80,6 +80,14 @@ int snag_rowblend_bwd(const float* g_out, const uint8_t* mask, float* g_in, int6
  * (src/utils.py:210-212). out is uint16_t* = raw bf16. */
 int snag_prep_bf16(const float* emb, int64_t ld, const int64_t* idx, int32_t n, int32_t D, int32_t normalize,
                    uint16_t* out, int32_t Dpad, float* norm2, void* stream);
+/* Prologue of the fp32 evaluation (precision="fp32"). rows [n, Dpad] fp32 (16-byte aligned) = the values snag_prep_bf16
+ * rounds, bit for bit (same normalisation arithmetic), zero padded; split [n, 3 Dpad] bf16 (128-byte aligned) = the
+ * three-term split h = bf16(x), m = bf16(x - h) laid out as [m | h | h] for side 0 (sources) and [h | m | h] for side 1
+ * (targets): a sweep over a side-0 and a side-1 operand (in either order) contracts m_x h_y + h_x m_y + h_x h_y, which
+ * leaves out only m_x m_y and the split's residuals (|x y - that| <= 3 * 2^-16 |x y|). norm2[r] = ||rows[r]||^2 in fp64,
+ * in index order, rounded once. Any sweep below accepts split operands (Dpad argument = 3 Dpad). */
+int snag_prep_split(const float* emb, int64_t ld, const int64_t* idx, int32_t n, int32_t D, int32_t normalize, int32_t side,
+                    float* rows, uint16_t* split, int32_t Dpad, float* norm2, void* stream);
 /* ---- fusion-output (joint) embeddings, model/SNAG_tools.py:44-49 ------------------------------ */
 /* joint[i, off_m + c] = w_ent[i, m] * e_m[i, c] / max(||e_m[i]||, 1e-12) and joint_fz[...] = w_glob[m] * (same), for the
  * M <= 6 present modalities concatenated along the row (off_m = widths[0] + .. + widths[m-1]). embs / widths are HOST
@@ -333,6 +341,36 @@ int snag_top4_merge(const float* val, const int32_t* idx, int32_t n_lists, int64
 int snag_top3_rescore(const uint16_t* X, const uint16_t* Y, int32_t Dpad, int64_t n_rows, const float* xn, const float* yn,
                       const float* nv1, const float* nv2, int32_t use_csls, const int32_t* cand, float* oval, int32_t* oidx,
                       void* stream);
+/* The canonical kernels above over fp32 rows [n, Dpad] (snag_prep_split's `rows`, 16-byte aligned) instead of bf16
+ * operands: same arguments, same arithmetic (an fp32 x fp32 product is exact in fp64, so the fp64 index-order sum
+ * rounded once is still the oracle's s_ij). The fp32 evaluation's sweeps run on the split operands and every verdict
+ * inside their error bound is re-judged here. */
+int snag_topk_rescore_f32(const float* A, const float* B, int32_t Dpad, int64_t n_rows, const float* an, const float* bn,
+                          const int32_t* cand_idx, const float* cand_val, int32_t k, float delta, const float* outsider_bound,
+                          float* nv, int32_t* flagged, int32_t* flagged_cnt, int32_t flagged_cap, float* best_d,
+                          int32_t* best_idx, void* stream);
+int snag_topk_exhaustive_f32(const float* A, const float* B, int32_t Dpad, int64_t n_b, const float* an, const float* bn,
+                             const int32_t* flagged, const int32_t* flagged_cnt, int32_t flagged_cap, int32_t k, float* nv,
+                             float* best_d, int32_t* best_idx, void* stream);
+int snag_pair_score_f32(const float* X, const float* Y, int32_t Dpad, int64_t n, const float* xn, const float* yn,
+                        const float* nv1, const float* nv2, int32_t use_csls, float* g, float* s_out, void* stream);
+int snag_band_rescore_f32(const float* X, const float* Y, int32_t Dpad, const float* xn, const float* yn, const float* nv1,
+                          const float* nv2, const float* g_row, const float* g_col, int32_t row_gid0, int32_t col_gid0,
+                          int32_t use_csls, const uint64_t* band, const uint32_t* band_cnt, uint32_t band_cap, int32_t* cnt_row,
+                          int32_t* cnt_col, void* stream);
+int snag_band_rescore_rows_f32(const float* X, const float* Y, int32_t Dpad, const float* xn, const float* yn,
+                               const float* nv1, const float* nv2, const float* g_row, const float* g_col,
+                               const int32_t* row_gids, int32_t col_gid0, int32_t use_csls, int32_t swapped,
+                               const uint64_t* band, const uint32_t* band_cnt, uint32_t band_cap, int32_t* cnt_row,
+                               int32_t* cnt_col, void* stream);
+int snag_rank_exhaustive_f32(const float* A, const float* B, int32_t Dpad, int64_t n_b, const float* an, const float* bn,
+                             const float* nva, const float* nvb, const float* g, const int32_t* rows, int32_t n_rows,
+                             int32_t a_gid0, int32_t b_gid0, int32_t use_csls, int32_t swapped, int32_t* cnt, void* stream);
+int snag_pairs_dot_f32(const float* X, const float* Y, int32_t Dpad, const int32_t* rows, const int32_t* cols, int64_t n_pairs,
+                       float* s_out, void* stream);
+int snag_top3_rescore_f32(const float* X, const float* Y, int32_t Dpad, int64_t n_rows, const float* xn, const float* yn,
+                          const float* nv1, const float* nv2, int32_t use_csls, const int32_t* cand, float* oval, int32_t* oidx,
+                          void* stream);
 
 /* csls_sim (src/utils.py:417-435) on a MATERIALISED fp32 similarity matrix [n1, ld]: nv1[i] / nv2[j] = mean of the k
  * largest entries of row i / column j; out[i,j] = (2*sim[i,j] - nv1[i]) - nv2[j] (out may be NULL to get only the

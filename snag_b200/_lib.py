@@ -31,6 +31,7 @@ _SIGNATURES = {
     "snag_rowblend_fwd": [_vp, _vp, _vp, _vp, _i64, _i32, _f32, _f32, _vp],
     "snag_rowblend_bwd": [_vp, _vp, _vp, _i64, _i32, _f32, _vp],
     "snag_prep_bf16": [_vp, _i64, _vp, _i32, _i32, _i32, _vp, _i32, _vp, _vp],
+    "snag_prep_split": [_vp, _i64, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp],
     "snag_joint_fuse_fwd": [_vp, _vp, _i32, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _vp],
     "snag_joint_fuse_bwd": [_vp, _vp, _vp, _i32, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp],
     "snag_normalize_bwd_scatter": [_vp, _i64, _vp, _i32, _i32, _i32, _vp, _i64, _i32, _i64, _vp, _i64, _vp],
@@ -80,6 +81,15 @@ _SIGNATURES = {
     "snag_pairs_dot": [_vp, _vp, _i32, _vp, _vp, _i64, _vp, _vp],
     "snag_top4_merge": [_vp, _vp, _i32, _i64, _vp, _vp, _vp],
     "snag_top3_rescore": [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
+    "snag_topk_rescore_f32": [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _f32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp],
+    "snag_topk_exhaustive_f32": [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp],
+    "snag_pair_score_f32": [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp],
+    "snag_band_rescore_f32": [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _u32, _vp, _vp, _vp],
+    "snag_band_rescore_rows_f32": [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _u32, _vp,
+                                   _vp, _vp],
+    "snag_rank_exhaustive_f32": [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp],
+    "snag_pairs_dot_f32": [_vp, _vp, _i32, _vp, _vp, _i64, _vp, _vp],
+    "snag_top3_rescore_f32": [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
     "snag_csls_sim": [_vp, _i64, _i64, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp],
     "snag_mutual_nn": [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp],
     "snag_icl_rowsum": [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _f32, _vp, _vp, _vp],

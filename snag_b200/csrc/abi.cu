@@ -66,6 +66,12 @@ int snag_prep_bf16(const float* emb, int64_t ld, const int64_t* idx, int32_t n, 
                           reinterpret_cast<__nv_bfloat16*>(out), Dpad, norm2, S(stream));
 }
 
+int snag_prep_split(const float* emb, int64_t ld, const int64_t* idx, int32_t n, int32_t D, int32_t normalize, int32_t side,
+                    float* rows, uint16_t* split, int32_t Dpad, float* norm2, void* stream) {
+  return launch_prep_split(emb, ld, reinterpret_cast<const long long*>(idx), n, D, normalize, side, rows,
+                           reinterpret_cast<__nv_bfloat16*>(split), Dpad, norm2, S(stream));
+}
+
 int snag_joint_fuse_fwd(const float* const* embs, const int32_t* widths, int32_t M, int64_t N, const float* w_ent, int64_t ldw,
                         const float* w_glob, float* joint, float* joint_fz, int64_t ld_out, void* stream) {
   return launch_joint_fuse_fwd(embs, widths, M, N, w_ent, ldw, w_glob, joint, joint_fz, ld_out, S(stream));
@@ -285,6 +291,56 @@ int snag_top3_rescore(const uint16_t* X, const uint16_t* Y, int32_t Dpad, int64_
                       const float* nv1, const float* nv2, int32_t use_csls, const int32_t* cand, float* oval, int32_t* oidx,
                       void* stream) {
   return launch_top3_rescore(BF(X), BF(Y), Dpad, n_rows, xn, yn, nv1, nv2, use_csls, cand, oval, oidx, S(stream));
+}
+
+/* fp32 rows (precision="fp32" evaluation): the canonical kernels above instantiated for float */
+int snag_topk_rescore_f32(const float* A, const float* B, int32_t Dpad, int64_t n_rows, const float* an, const float* bn,
+                          const int32_t* cand_idx, const float* cand_val, int32_t k, float delta, const float* outsider_bound,
+                          float* nv, int32_t* flagged, int32_t* flagged_cnt, int32_t flagged_cap, float* best_d,
+                          int32_t* best_idx, void* stream) {
+  return launch_topk_rescore(A, B, Dpad, n_rows, an, bn, cand_idx, cand_val, k, delta, outsider_bound, nv, flagged,
+                             flagged_cnt, flagged_cap, best_d, best_idx, S(stream));
+}
+int snag_topk_exhaustive_f32(const float* A, const float* B, int32_t Dpad, int64_t n_b, const float* an, const float* bn,
+                             const int32_t* flagged, const int32_t* flagged_cnt, int32_t flagged_cap, int32_t k, float* nv,
+                             float* best_d, int32_t* best_idx, void* stream) {
+  return launch_topk_exhaustive(A, B, Dpad, n_b, an, bn, flagged, flagged_cnt, flagged_cap, k, nv, best_d, best_idx, S(stream));
+}
+int snag_pair_score_f32(const float* X, const float* Y, int32_t Dpad, int64_t n, const float* xn, const float* yn,
+                        const float* nv1, const float* nv2, int32_t use_csls, float* g, float* s_out, void* stream) {
+  return launch_pair_score(X, Y, Dpad, n, xn, yn, nv1, nv2, use_csls, g, s_out, S(stream));
+}
+int snag_band_rescore_f32(const float* X, const float* Y, int32_t Dpad, const float* xn, const float* yn, const float* nv1,
+                          const float* nv2, const float* g_row, const float* g_col, int32_t row_gid0, int32_t col_gid0,
+                          int32_t use_csls, const uint64_t* band, const uint32_t* band_cnt, uint32_t band_cap, int32_t* cnt_row,
+                          int32_t* cnt_col, void* stream) {
+  return launch_band_rescore(X, Y, Dpad, xn, yn, nv1, nv2, g_row, g_col, row_gid0, col_gid0, use_csls,
+                             reinterpret_cast<const uint2*>(band), band_cnt, band_cap, cnt_row, cnt_col, S(stream));
+}
+int snag_band_rescore_rows_f32(const float* X, const float* Y, int32_t Dpad, const float* xn, const float* yn,
+                               const float* nv1, const float* nv2, const float* g_row, const float* g_col,
+                               const int32_t* row_gids, int32_t col_gid0, int32_t use_csls, int32_t swapped,
+                               const uint64_t* band, const uint32_t* band_cnt, uint32_t band_cap, int32_t* cnt_row,
+                               int32_t* cnt_col, void* stream) {
+  if (!row_gids) return SNAG_ERR_ARG;
+  return launch_band_rescore(X, Y, Dpad, xn, yn, nv1, nv2, g_row, g_col, 0, col_gid0, use_csls,
+                             reinterpret_cast<const uint2*>(band), band_cnt, band_cap, cnt_row, cnt_col, S(stream), row_gids,
+                             swapped);
+}
+int snag_rank_exhaustive_f32(const float* A, const float* B, int32_t Dpad, int64_t n_b, const float* an, const float* bn,
+                             const float* nva, const float* nvb, const float* g, const int32_t* rows, int32_t n_rows,
+                             int32_t a_gid0, int32_t b_gid0, int32_t use_csls, int32_t swapped, int32_t* cnt, void* stream) {
+  return launch_rank_exhaustive(A, B, Dpad, n_b, an, bn, nva, nvb, g, rows, n_rows, a_gid0, b_gid0, use_csls, swapped, cnt,
+                                S(stream));
+}
+int snag_pairs_dot_f32(const float* X, const float* Y, int32_t Dpad, const int32_t* rows, const int32_t* cols, int64_t n_pairs,
+                       float* s_out, void* stream) {
+  return launch_pairs_dot(X, Y, Dpad, rows, cols, n_pairs, s_out, S(stream));
+}
+int snag_top3_rescore_f32(const float* X, const float* Y, int32_t Dpad, int64_t n_rows, const float* xn, const float* yn,
+                          const float* nv1, const float* nv2, int32_t use_csls, const int32_t* cand, float* oval, int32_t* oidx,
+                          void* stream) {
+  return launch_top3_rescore(X, Y, Dpad, n_rows, xn, yn, nv1, nv2, use_csls, cand, oval, oidx, S(stream));
 }
 
 int64_t snag_csls_workspace_bytes(int64_t n1, int64_t n2) { return csls_workspace_floats(n1, n2) * 4; }

@@ -2,6 +2,7 @@
 // column mean/std, entity-row blend (fwd/bwd), CSLS candidate merge, ground-truth ("diagonal") scores,
 // and the materialised CSLS drop-in. All vectorised, coalesced, grid sized from the SM count.
 #include <mutex>
+#include <type_traits>
 #include "common.cuh"
 #include "snag_internal.h"
 
@@ -339,6 +340,54 @@ __global__ void __launch_bounds__(256) prep_bf16_kernel(const float* __restrict_
   if (lane == 0 && norm2) norm2[warp] = static_cast<float>(acc);
 }
 
+// Prologue of the fp32 evaluation: the rows prep_bf16 rounds, kept in fp32 (the canonical re-scores read them), and a
+// three-term bf16 split of them for the tensor-core sweeps: h = bf16(x), m = bf16(x - h) (x - h is exact in fp32), laid
+// out as [m | h | h] for sources (side 0) and [h | m | h] for targets (side 1), so that one bf16 contraction of width
+// 3 Dpad forms m_x h_y + h_x m_y + h_x h_y in either operand order. The normalisation repeats prep_row's arithmetic
+// step for step — each lane's fp32 sum of squares over its columns (float4 path or scalar path under the same
+// condition), the same butterfly, the same __fdiv_rn — so x is bit for bit what prep_bf16 rounds and h is its output.
+__global__ void __launch_bounds__(256) prep_split_kernel(const float* __restrict__ emb, long long ld,
+                                                         const long long* __restrict__ idx, int n, int D, int normalize,
+                                                         int side, float* __restrict__ rows, __nv_bfloat16* __restrict__ split,
+                                                         int Dpad) {
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (warp >= n) return;
+  const float* src = emb + (idx ? idx[warp] : static_cast<long long>(warp)) * ld;
+  float denom = 1.0f;
+  if (normalize) {
+    const bool vec4 = (D % 4 == 0) && (ld % 4 == 0) && ((reinterpret_cast<uintptr_t>(emb) & 15) == 0);
+    float ss = 0.f;
+    if (vec4) {
+      const float4* s4 = reinterpret_cast<const float4*>(src);
+      for (int c4 = lane; c4 < (D >> 2); c4 += 32) {
+        const float4 t = __ldg(s4 + c4);
+        ss = __fmaf_rn(t.x, t.x, ss); ss = __fmaf_rn(t.y, t.y, ss); ss = __fmaf_rn(t.z, t.z, ss); ss = __fmaf_rn(t.w, t.w, ss);
+      }
+    } else {
+      for (int c = lane; c < D; c += 32) { const float v = __ldg(src + c); ss = __fmaf_rn(v, v, ss); }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    denom = fmaxf(sqrtf(ss), 1e-12f);
+  }
+  float* row = rows + static_cast<long long>(warp) * Dpad;
+  __nv_bfloat16* sp = split + static_cast<long long>(warp) * 3 * Dpad;
+  __nv_bfloat16* h0 = sp + (side ? 0 : Dpad);
+  __nv_bfloat16* m0 = sp + (side ? Dpad : 0);
+  __nv_bfloat16* h1 = sp + 2 * Dpad;
+  for (int c = lane; c < Dpad; c += 32) {
+    float v = 0.f;
+    if (c < D) v = normalize ? __fdiv_rn(__ldg(src + c), denom) : __ldg(src + c);
+    const __nv_bfloat16 h = __float2bfloat16_rn(v);
+    const __nv_bfloat16 m = __float2bfloat16_rn(__fsub_rn(v, __bfloat162float(h)));
+    row[c] = v;
+    h0[c] = h;
+    m0[c] = m;
+    h1[c] = h;
+  }
+}
+
 // ------------------------------------------------------------------------------------------------
 // Batched prologue / epilogue of the loss layer: the 2 + 2M icl_loss calls of a step share the batch of links, so the
 // stacked operands of ALL calls are built by one launch and the gradients of all calls go back through one launch
@@ -669,6 +718,33 @@ __device__ __forceinline__ float canonical_dot(const __nv_bfloat16* __restrict__
   }
   return static_cast<float>(acc);
 }
+// The same for fp32 rows (the fp32 evaluation): an fp32 x fp32 product is exact in fp64 as well, so fma(double, double,
+// acc) in index order is still the oracle's arithmetic. Same pipelining: 64 bytes of each row per trip (16 elements).
+__device__ __forceinline__ float canonical_dot(const float* __restrict__ x, const float* __restrict__ y, int Dpad) {
+  const float4* xr = reinterpret_cast<const float4*>(x);
+  const float4* yr = reinterpret_cast<const float4*>(y);
+  const int n = Dpad / 4;                        // 16-byte words per row; a multiple of 16
+  double acc = 0.0;
+  float4 a[4], b[4];
+#pragma unroll
+  for (int u = 0; u < 4; ++u) { a[u] = __ldg(xr + u); b[u] = __ldg(yr + u); }
+  for (int c = 0; c < n; c += 4) {
+    float4 na[4], nb[4];
+    const int cn = c + 4 < n ? c + 4 : c;
+#pragma unroll
+    for (int u = 0; u < 4; ++u) { na[u] = __ldg(xr + cn + u); nb[u] = __ldg(yr + cn + u); }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      acc = fma(static_cast<double>(a[u].x), static_cast<double>(b[u].x), acc);
+      acc = fma(static_cast<double>(a[u].y), static_cast<double>(b[u].y), acc);
+      acc = fma(static_cast<double>(a[u].z), static_cast<double>(b[u].z), acc);
+      acc = fma(static_cast<double>(a[u].w), static_cast<double>(b[u].w), acc);
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) { a[u] = na[u]; b[u] = nb[u]; }
+  }
+  return static_cast<float>(acc);
+}
 // the reference's fp32 chain from s to the (CSLS) distance, one rounding per op (simgemm.cuh has the same two helpers)
 __device__ __forceinline__ float canonical_dist(float s, float xn, float yn, float nv1, float nv2, int use_csls) {
   const float d = fmaxf(__fmaf_rn(-2.0f, s, __fadd_rn(xn, yn)), 0.0f);
@@ -758,7 +834,8 @@ __global__ void __launch_bounds__(128) topk_merge_mean_kernel(const float* __res
 // Unverified rows (plateaus of near-equal scores wider than KT - k) are appended to `flagged` for the exhaustive
 // pass below. One warp handles two rows: 16 lanes per row, one candidate per lane.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) topk_rescore_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* __restrict__ B,
+template <typename T>
+__global__ void __launch_bounds__(128) topk_rescore_kernel(const T* __restrict__ A, const T* __restrict__ B,
                                                            int Dpad, long long n_rows, const float* __restrict__ an,
                                                            const float* __restrict__ bn, const int* __restrict__ cand_idx,
                                                            const float* __restrict__ cand_val, int k, float delta,
@@ -823,7 +900,8 @@ __global__ void __launch_bounds__(128) topk_rescore_kernel(const __nv_bfloat16* 
 
 // Exhaustive canonical neighbourhood of the flagged rows: one block per flagged row, threads stride over all rows of
 // B keeping their own k largest canonical scores; lists are merged through shared memory.
-__global__ void __launch_bounds__(256) topk_exhaustive_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* __restrict__ B,
+template <typename T>
+__global__ void __launch_bounds__(256) topk_exhaustive_kernel(const T* __restrict__ A, const T* __restrict__ B,
                                                               int Dpad, long long n_b, const float* __restrict__ an,
                                                               const float* __restrict__ bn, const int* __restrict__ flagged,
                                                               const int* __restrict__ flagged_cnt, int flagged_cap, int k,
@@ -877,29 +955,35 @@ __global__ void __launch_bounds__(256) topk_exhaustive_kernel(const __nv_bfloat1
 // in fp64 in index order and rounded once to fp32 (the oracle's definition of s_pp), then the same
 // fp32 chain as the fused epilogue. One thread per pair; 16-byte loads.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) pair_score_kernel(const __nv_bfloat16* __restrict__ X, const __nv_bfloat16* __restrict__ Y,
+template <typename T>
+__global__ void __launch_bounds__(128) pair_score_kernel(const T* __restrict__ X, const T* __restrict__ Y,
                                                          int Dpad, long long n, const float* __restrict__ xn,
                                                          const float* __restrict__ yn, const float* __restrict__ nv1,
                                                          const float* __restrict__ nv2, int use_csls, float* __restrict__ g,
                                                          float* __restrict__ s_out) {
   const long long p = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
   if (p >= n) return;
-  const uint4* xr = reinterpret_cast<const uint4*>(X + p * Dpad);
-  const uint4* yr = reinterpret_cast<const uint4*>(Y + p * Dpad);
-  double acc = 0.0;
-  for (int c = 0; c < Dpad / 8; ++c) {
-    const uint4 a = __ldg(xr + c), b = __ldg(yr + c);
-    const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, bw[4] = {b.x, b.y, b.z, b.w};
+  float s;
+  if constexpr (std::is_same<T, float>::value) {
+    s = canonical_dot(X + p * Dpad, Y + p * Dpad, Dpad);
+  } else {
+    const uint4* xr = reinterpret_cast<const uint4*>(X + p * Dpad);
+    const uint4* yr = reinterpret_cast<const uint4*>(Y + p * Dpad);
+    double acc = 0.0;
+    for (int c = 0; c < Dpad / 8; ++c) {
+      const uint4 a = __ldg(xr + c), b = __ldg(yr + c);
+      const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, bw[4] = {b.x, b.y, b.z, b.w};
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      // bf16 -> fp32 is a 16-bit shift; low half first (little endian = lower column index)
-      const float a0 = __uint_as_float(aw[e] << 16), a1 = __uint_as_float(aw[e] & 0xffff0000u);
-      const float b0 = __uint_as_float(bw[e] << 16), b1 = __uint_as_float(bw[e] & 0xffff0000u);
-      acc = fma(static_cast<double>(a0), static_cast<double>(b0), acc);
-      acc = fma(static_cast<double>(a1), static_cast<double>(b1), acc);
+      for (int e = 0; e < 4; ++e) {
+        // bf16 -> fp32 is a 16-bit shift; low half first (little endian = lower column index)
+        const float a0 = __uint_as_float(aw[e] << 16), a1 = __uint_as_float(aw[e] & 0xffff0000u);
+        const float b0 = __uint_as_float(bw[e] << 16), b1 = __uint_as_float(bw[e] & 0xffff0000u);
+        acc = fma(static_cast<double>(a0), static_cast<double>(b0), acc);
+        acc = fma(static_cast<double>(a1), static_cast<double>(b1), acc);
+      }
     }
+    s = static_cast<float>(acc);
   }
-  const float s = static_cast<float>(acc);
   if (s_out) s_out[p] = s;
   const float t = __fadd_rn(xn[p], yn[p]);
   const float d = fmaxf(__fmaf_rn(-2.0f, s, t), 0.0f);
@@ -914,7 +998,8 @@ __global__ void __launch_bounds__(128) pair_score_kernel(const __nv_bfloat16* __
 // inside the band is judged here with the canonical arithmetic and the stable-sort tie-break (main.py:400-429 with
 // torch.sort(stable=True)): one thread per element.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) band_rescore_kernel(const __nv_bfloat16* __restrict__ X, const __nv_bfloat16* __restrict__ Y,
+template <typename T>
+__global__ void __launch_bounds__(128) band_rescore_kernel(const T* __restrict__ X, const T* __restrict__ Y,
                                                            int Dpad, const float* __restrict__ xn, const float* __restrict__ yn,
                                                            const float* __restrict__ nv1, const float* __restrict__ nv2,
                                                            const float* __restrict__ g_row, const float* __restrict__ g_col,
@@ -1036,7 +1121,8 @@ __global__ void __launch_bounds__(256) rank_judge_kernel(const uint2* __restrict
 }
 
 constexpr int RX_ROWS = 8;       // listed rows one block of rank_exhaustive handles together (B is read once for all of them)
-__global__ void __launch_bounds__(256) rank_exhaustive_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* __restrict__ B,
+template <typename T>
+__global__ void __launch_bounds__(256) rank_exhaustive_kernel(const T* __restrict__ A, const T* __restrict__ B,
                                                               int Dpad, long long n_b, const float* __restrict__ an,
                                                               const float* __restrict__ bn, const float* __restrict__ nva,
                                                               const float* __restrict__ nvb, const float* __restrict__ g,
@@ -1048,7 +1134,7 @@ __global__ void __launch_bounds__(256) rank_exhaustive_kernel(const __nv_bfloat1
   const int nr = min(RX_ROWS, n_rows - r0);
   for (int t = threadIdx.x; t < RX_ROWS * Dpad; t += blockDim.x) {
     const int r = t / Dpad, c = t - r * Dpad;
-    a_s[t] = r < nr ? __bfloat162float(A[static_cast<long long>(rows[r0 + r]) * Dpad + c]) : 0.f;
+    a_s[t] = r < nr ? static_cast<float>(A[static_cast<long long>(rows[r0 + r]) * Dpad + c]) : 0.f;
   }
   if (threadIdx.x < RX_ROWS) cnt_s[threadIdx.x] = 0;
   __syncthreads();
@@ -1066,27 +1152,36 @@ __global__ void __launch_bounds__(256) rank_exhaustive_kernel(const __nv_bfloat1
   const long long per = (n_b + gridDim.y - 1) / gridDim.y;
   const long long j0 = blockIdx.y * per, j1 = min(n_b, j0 + per);
   for (long long j = j0 + threadIdx.x; j < j1; j += blockDim.x) {
-    const uint4* br = reinterpret_cast<const uint4*>(B + j * Dpad);
     double acc[RX_ROWS];
 #pragma unroll
     for (int r = 0; r < RX_ROWS; ++r) acc[r] = 0.0;
     for (int c = 0; c < Dpad / 8; ++c) {
-      const uint4 b = __ldg(br + c);
-      const uint32_t bw[4] = {b.x, b.y, b.z, b.w};
       float bf[8];
+      if constexpr (std::is_same<T, float>::value) {
+        const float4* br = reinterpret_cast<const float4*>(B + j * Dpad);
+        const float4 b0 = __ldg(br + 2 * c), b1 = __ldg(br + 2 * c + 1);
+        bf[0] = b0.x; bf[1] = b0.y; bf[2] = b0.z; bf[3] = b0.w; bf[4] = b1.x; bf[5] = b1.y; bf[6] = b1.z; bf[7] = b1.w;
+      } else {
+        const uint4 b = __ldg(reinterpret_cast<const uint4*>(B + j * Dpad) + c);
+        const uint32_t bw[4] = {b.x, b.y, b.z, b.w};
 #pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        bf[2 * e] = __uint_as_float(bw[e] << 16);
-        bf[2 * e + 1] = __uint_as_float(bw[e] & 0xffff0000u);
+        for (int e = 0; e < 4; ++e) {
+          bf[2 * e] = __uint_as_float(bw[e] << 16);
+          bf[2 * e + 1] = __uint_as_float(bw[e] & 0xffff0000u);
+        }
       }
 #pragma unroll
       for (int r = 0; r < RX_ROWS; ++r) {
         const float4 a0 = *reinterpret_cast<const float4*>(a_s + r * Dpad + c * 8);
         const float4 a1 = *reinterpret_cast<const float4*>(a_s + r * Dpad + c * 8 + 4);
         const float af[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-        // a bf16 x bf16 product is exact in fp32, so exact product + one fp64 rounding == fma(double a, double b, acc)
 #pragma unroll
-        for (int e = 0; e < 8; ++e) acc[r] = __dadd_rn(acc[r], static_cast<double>(__fmul_rn(af[e], bf[e])));
+        for (int e = 0; e < 8; ++e) {
+          if constexpr (std::is_same<T, float>::value)
+            acc[r] = fma(static_cast<double>(af[e]), static_cast<double>(bf[e]), acc[r]);   // exact product in fp64
+          else   // a bf16 x bf16 product is exact in fp32, so exact product + one fp64 rounding == fma(double a, double b, acc)
+            acc[r] = __dadd_rn(acc[r], static_cast<double>(__fmul_rn(af[e], bf[e])));
+        }
       }
     }
     const float b_n = bn[j], b_nv = use_csls ? nvb[j] : 0.f;
@@ -1112,12 +1207,22 @@ __global__ void __launch_bounds__(256) rank_exhaustive_kernel(const __nv_bfloat1
 
 // canonical dot products of an explicit list of (row of X, row of Y) pairs — the re-score of the similarity entries a
 // thresholded sweep collected (unsupervised seed induction, src/data.py:367-375)
-__global__ void __launch_bounds__(128) pairs_dot_kernel(const __nv_bfloat16* __restrict__ X, const __nv_bfloat16* __restrict__ Y,
+template <typename T>
+__global__ void __launch_bounds__(128) pairs_dot_kernel(const T* __restrict__ X, const T* __restrict__ Y,
                                                         int Dpad, const int* __restrict__ rows, const int* __restrict__ cols,
                                                         long long n_pairs, float* __restrict__ s_out) {
   const long long p = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
   if (p >= n_pairs) return;
   s_out[p] = canonical_dot(X + static_cast<long long>(rows[p]) * Dpad, Y + static_cast<long long>(cols[p]) * Dpad, Dpad);
+}
+
+// ||row||^2 of fp32 rows in fp64, in index order, rounded once (oracle_norm2): the canonical dot of the row with itself.
+// (prep_row adds lane-strided partial sums: in that order fp64 sums of fp32 squares round differently now and then.)
+__global__ void __launch_bounds__(128) row_norm2_kernel(const float* __restrict__ rows, int Dpad, long long n,
+                                                        float* __restrict__ norm2) {
+  const long long p = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+  if (p >= n) return;
+  norm2[p] = canonical_dot(rows + p * Dpad, rows + p * Dpad, Dpad);
 }
 
 // merge per-list top-4 candidate lists of each row (x descending = nearest first, column id ascending on ties)
@@ -1153,7 +1258,8 @@ __global__ void __launch_bounds__(128) top4_merge_kernel(const float* __restrict
 
 // canonical distances of each row's (up to) four nearest candidates, sorted ascending (column id ascending on ties):
 // entries 0..2 are ret1..ret3 of the prediction file (main.py:411)
-__global__ void __launch_bounds__(128) top3_rescore_kernel(const __nv_bfloat16* __restrict__ X, const __nv_bfloat16* __restrict__ Y,
+template <typename T>
+__global__ void __launch_bounds__(128) top3_rescore_kernel(const T* __restrict__ X, const T* __restrict__ Y,
                                                            int Dpad, long long n_rows, const float* __restrict__ xn,
                                                            const float* __restrict__ yn, const float* __restrict__ nv1,
                                                            const float* __restrict__ nv2, int use_csls,
@@ -1385,7 +1491,8 @@ int launch_col_cand_finalize(const long long* offs, const int* hist, const float
                                                                              cand_idx, overflow);
   return static_cast<int>(cudaGetLastError());
 }
-int launch_topk_rescore(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad, long long n_rows, const float* an,
+template <typename T>
+int launch_topk_rescore(const T* A, const T* B, int Dpad, long long n_rows, const float* an,
                         const float* bn, const int* cand_idx, const float* cand_val, int k, float delta,
                         const float* outsider_bound, float* nv, int* flagged, int* flagged_cnt, int flagged_cap,
                         float* best_d, int* best_idx, cudaStream_t st) {
@@ -1394,19 +1501,20 @@ int launch_topk_rescore(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad
   if ((best_d == nullptr) != (best_idx == nullptr)) return SNAG_ERR_ARG;
   if (k < 1 || k > KT_LIST || (Dpad % 64)) return SNAG_ERR_SHAPE;
   const long long threads = n_rows * 16;
-  topk_rescore_kernel<<<static_cast<unsigned>((threads + 127) / 128), 128, 0, st>>>(A, B, Dpad, n_rows, an, bn, cand_idx,
+  topk_rescore_kernel<T><<<static_cast<unsigned>((threads + 127) / 128), 128, 0, st>>>(A, B, Dpad, n_rows, an, bn, cand_idx,
                                                                                    cand_val, k, delta, outsider_bound, nv, flagged,
                                                                                    flagged_cnt, flagged_cap, best_d, best_idx);
   return static_cast<int>(cudaGetLastError());
 }
-int launch_topk_exhaustive(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad, long long n_b, const float* an,
+template <typename T>
+int launch_topk_exhaustive(const T* A, const T* B, int Dpad, long long n_b, const float* an,
                            const float* bn, const int* flagged, const int* flagged_cnt, int flagged_cap, int k, float* nv,
                            float* best_d, int* best_idx, cudaStream_t st) {
   if (!A || !B || !an || !bn || !flagged || !flagged_cnt || !nv || n_b <= 0 || flagged_cap < 1) return SNAG_ERR_ARG;
   if ((best_d == nullptr) != (best_idx == nullptr)) return SNAG_ERR_ARG;
   if (k < 1 || k > KT_LIST || (Dpad % 64)) return SNAG_ERR_SHAPE;
   const int grid = flagged_cap < num_sms() * 4 ? flagged_cap : num_sms() * 4;
-  topk_exhaustive_kernel<<<grid, 256, 0, st>>>(A, B, Dpad, n_b, an, bn, flagged, flagged_cnt, flagged_cap, k, nv, best_d, best_idx);
+  topk_exhaustive_kernel<T><<<grid, 256, 0, st>>>(A, B, Dpad, n_b, an, bn, flagged, flagged_cnt, flagged_cap, k, nv, best_d, best_idx);
   return static_cast<int>(cudaGetLastError());
 }
 static inline int grid_for(long long work_items, int block, int num_sms, int ctas_per_sm);
@@ -1714,6 +1822,17 @@ int launch_prep_bf16(const float* emb, long long ld, const long long* idx, int n
   return static_cast<int>(cudaGetLastError());
 }
 
+int launch_prep_split(const float* emb, long long ld, const long long* idx, int n, int D, int normalize, int side,
+                      float* rows, __nv_bfloat16* split, int Dpad, float* norm2, cudaStream_t st) {
+  if (!emb || !rows || !split || !norm2 || n <= 0 || D <= 0 || (side != 0 && side != 1)) return SNAG_ERR_ARG;
+  if (Dpad < D || (Dpad % 64) != 0) return SNAG_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(rows) & 15) || (reinterpret_cast<uintptr_t>(split) & 127)) return SNAG_ERR_ALIGN;
+  const long long threads = static_cast<long long>(n) * 32;
+  prep_split_kernel<<<static_cast<int>((threads + 255) / 256), 256, 0, st>>>(emb, ld, idx, n, D, normalize, side, rows, split, Dpad);
+  row_norm2_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(rows, Dpad, n, norm2);
+  return static_cast<int>(cudaGetLastError());
+}
+
 int launch_icl_stack_prep(int n_prob, const float* const* emb, const long long* ld, const int* D, __nv_bfloat16* const* out,
                           const int* Dpad, const long long* idx_l, const long long* idx_r, int B, int Bp, int normalize,
                           cudaStream_t st) {
@@ -1826,16 +1945,18 @@ int launch_topk_merge_mean(const float* part, const int* part_idx, int n_lists, 
   return static_cast<int>(cudaGetLastError());
 }
 
-int launch_pair_score(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, long long n, const float* xn, const float* yn,
+template <typename T>
+int launch_pair_score(const T* X, const T* Y, int Dpad, long long n, const float* xn, const float* yn,
                       const float* nv1, const float* nv2, int use_csls, float* g, float* s_out, cudaStream_t st) {
   if (!X || !Y || !xn || !yn || !g || n <= 0) return SNAG_ERR_ARG;
   if (use_csls && (!nv1 || !nv2)) return SNAG_ERR_ARG;
   if (Dpad % 64) return SNAG_ERR_SHAPE;
-  pair_score_kernel<<<static_cast<int>((n + 127) / 128), 128, 0, st>>>(X, Y, Dpad, n, xn, yn, nv1, nv2, use_csls, g, s_out);
+  pair_score_kernel<T><<<static_cast<int>((n + 127) / 128), 128, 0, st>>>(X, Y, Dpad, n, xn, yn, nv1, nv2, use_csls, g, s_out);
   return static_cast<int>(cudaGetLastError());
 }
 
-int launch_band_rescore(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, const float* xn, const float* yn,
+template <typename T>
+int launch_band_rescore(const T* X, const T* Y, int Dpad, const float* xn, const float* yn,
                         const float* nv1, const float* nv2, const float* g_row, const float* g_col, int row_gid0, int col_gid0,
                         int use_csls, const uint2* band, const unsigned int* band_cnt, unsigned int band_cap, int* cnt_row,
                         int* cnt_col, cudaStream_t st, const int* row_gids, int swapped) {
@@ -1843,7 +1964,7 @@ int launch_band_rescore(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad
   if (use_csls && (!nv1 || !nv2)) return SNAG_ERR_ARG;
   if (Dpad % 64) return SNAG_ERR_SHAPE;
   // grid-stride over the device-side count: no host round trip
-  band_rescore_kernel<<<num_sms() * 16, 128, 0, st>>>(X, Y, Dpad, xn, yn, nv1, nv2, g_row, g_col, row_gid0, col_gid0, use_csls,
+  band_rescore_kernel<T><<<num_sms() * 16, 128, 0, st>>>(X, Y, Dpad, xn, yn, nv1, nv2, g_row, g_col, row_gid0, col_gid0, use_csls,
                                                       band, band_cnt, band_cap, cnt_row, cnt_col, row_gids, swapped);
   return static_cast<int>(cudaGetLastError());
 }
@@ -1867,7 +1988,8 @@ int launch_rank_judge(const uint2* rk_stream, const int* rk_stream_row, const in
   return static_cast<int>(cudaGetLastError());
 }
 
-int launch_rank_exhaustive(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad, long long n_b, const float* an,
+template <typename T>
+int launch_rank_exhaustive(const T* A, const T* B, int Dpad, long long n_b, const float* an,
                            const float* bn, const float* nva, const float* nvb, const float* g, const int* rows, int n_rows,
                            int a_gid0, int b_gid0, int use_csls, int swapped, int* cnt, cudaStream_t st) {
   if (!A || !B || !an || !bn || !g || !rows || !cnt || n_rows < 1 || n_b < 1) return SNAG_ERR_ARG;
@@ -1877,23 +1999,24 @@ int launch_rank_exhaustive(const __nv_bfloat16* A, const __nv_bfloat16* B, int D
   if (smem > 200 * 1024) return SNAG_ERR_SHAPE;
   static std::once_flag once;
   std::call_once(once, [] {
-    cudaFuncSetAttribute(rank_exhaustive_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(rank_exhaustive_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   });
   const int gx = (n_rows + RX_ROWS - 1) / RX_ROWS;
   int gy = (num_sms() * 4 + gx - 1) / gx;                  // enough blocks to fill the machine when few rows are listed
   const long long max_gy = (n_b + 255) / 256;
   if (gy > max_gy) gy = static_cast<int>(max_gy);
   if (gy < 1) gy = 1;
-  rank_exhaustive_kernel<<<dim3(gx, gy), 256, smem, st>>>(A, B, Dpad, n_b, an, bn, nva, nvb, g, rows, n_rows, a_gid0, b_gid0,
+  rank_exhaustive_kernel<T><<<dim3(gx, gy), 256, smem, st>>>(A, B, Dpad, n_b, an, bn, nva, nvb, g, rows, n_rows, a_gid0, b_gid0,
                                                           use_csls, swapped, cnt);
   return static_cast<int>(cudaGetLastError());
 }
 
-int launch_pairs_dot(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, const int* rows, const int* cols,
+template <typename T>
+int launch_pairs_dot(const T* X, const T* Y, int Dpad, const int* rows, const int* cols,
                      long long n_pairs, float* s_out, cudaStream_t st) {
   if (!X || !Y || !rows || !cols || !s_out || n_pairs <= 0) return SNAG_ERR_ARG;
   if (Dpad % 64) return SNAG_ERR_SHAPE;
-  pairs_dot_kernel<<<static_cast<unsigned>((n_pairs + 127) / 128), 128, 0, st>>>(X, Y, Dpad, rows, cols, n_pairs, s_out);
+  pairs_dot_kernel<T><<<static_cast<unsigned>((n_pairs + 127) / 128), 128, 0, st>>>(X, Y, Dpad, rows, cols, n_pairs, s_out);
   return static_cast<int>(cudaGetLastError());
 }
 
@@ -1903,13 +2026,14 @@ int launch_top4_merge(const float* val, const int* idx, int n_lists, long long n
   return static_cast<int>(cudaGetLastError());
 }
 
-int launch_top3_rescore(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, long long n_rows, const float* xn,
+template <typename T>
+int launch_top3_rescore(const T* X, const T* Y, int Dpad, long long n_rows, const float* xn,
                         const float* yn, const float* nv1, const float* nv2, int use_csls, const int* cand, float* oval,
                         int* oidx, cudaStream_t st) {
   if (!X || !Y || !xn || !yn || !cand || !oval || !oidx || n_rows <= 0) return SNAG_ERR_ARG;
   if (use_csls && (!nv1 || !nv2)) return SNAG_ERR_ARG;
   if (Dpad % 64) return SNAG_ERR_SHAPE;
-  top3_rescore_kernel<<<static_cast<int>((n_rows + 127) / 128), 128, 0, st>>>(X, Y, Dpad, n_rows, xn, yn, nv1, nv2, use_csls,
+  top3_rescore_kernel<T><<<static_cast<int>((n_rows + 127) / 128), 128, 0, st>>>(X, Y, Dpad, n_rows, xn, yn, nv1, nv2, use_csls,
                                                                             cand, oval, oidx);
   return static_cast<int>(cudaGetLastError());
 }
@@ -1920,5 +2044,27 @@ int launch_icl_finalize(const float* rowsum_part, int n_chunks, int B, int Bp, c
   icl_finalize_kernel<<<(B + 255) / 256, 256, 0, st>>>(rowsum_part, n_chunks, B, Bp, pos, inv_tau, lse, nll);
   return static_cast<int>(cudaGetLastError());
 }
+
+// the canonical kernels for both row types: bf16 operands (default evaluation) and fp32 rows (precision="fp32")
+#define SNAG_CANONICAL_INSTANTIATE(T)                                                                                       \
+  template int launch_topk_rescore<T>(const T*, const T*, int, long long, const float*, const float*, const int*,         \
+                                      const float*, int, float, const float*, float*, int*, int*, int, float*, int*,        \
+                                      cudaStream_t);                                                                        \
+  template int launch_topk_exhaustive<T>(const T*, const T*, int, long long, const float*, const float*, const int*,      \
+                                         const int*, int, int, float*, float*, int*, cudaStream_t);                         \
+  template int launch_pair_score<T>(const T*, const T*, int, long long, const float*, const float*, const float*,        \
+                                    const float*, int, float*, float*, cudaStream_t);                                       \
+  template int launch_band_rescore<T>(const T*, const T*, int, const float*, const float*, const float*, const float*,   \
+                                      const float*, const float*, int, int, int, const uint2*, const unsigned int*,         \
+                                      unsigned int, int*, int*, cudaStream_t, const int*, int);                             \
+  template int launch_rank_exhaustive<T>(const T*, const T*, int, long long, const float*, const float*, const float*,   \
+                                         const float*, const float*, const int*, int, int, int, int, int, int*,             \
+                                         cudaStream_t);                                                                     \
+  template int launch_pairs_dot<T>(const T*, const T*, int, const int*, const int*, long long, float*, cudaStream_t);    \
+  template int launch_top3_rescore<T>(const T*, const T*, int, long long, const float*, const float*, const float*,      \
+                                      const float*, int, const int*, float*, int*, cudaStream_t);
+SNAG_CANONICAL_INSTANTIATE(__nv_bfloat16)
+SNAG_CANONICAL_INSTANTIATE(float)
+#undef SNAG_CANONICAL_INSTANTIATE
 
 }  // namespace snag

@@ -37,6 +37,8 @@ int launch_rowblend_fwd(const float* e, const float* noise, const uint8_t* mask,
 int launch_rowblend_bwd(const float* g_out, const uint8_t* mask, float* g_in, long long N, int D, float a, cudaStream_t st);
 int launch_prep_bf16(const float* emb, long long ld, const long long* idx, int n, int D, int normalize,
                      __nv_bfloat16* out, int Dpad, float* norm2, cudaStream_t st);
+int launch_prep_split(const float* emb, long long ld, const long long* idx, int n, int D, int normalize, int side,
+                      float* rows, __nv_bfloat16* split, int Dpad, float* norm2, cudaStream_t st);
 int launch_joint_fuse_fwd(const float* const* embs, const int* widths, int M, long long N, const float* w_ent, long long ldw,
                           const float* w_glob, float* joint, float* joint_fz, long long ld_out, cudaStream_t st);
 int launch_joint_fuse_bwd(const float* const* embs, float* const* d_embs, const int* widths, int M, long long N,
@@ -92,23 +94,29 @@ int launch_icl_sym_finalize(const float* total, const float* pos, int n_prob, in
                             cudaStream_t st);
 int launch_topk_merge_mean(const float* part, const int* part_idx, int n_lists, long long n_rows, int k, float* nv,
                            float* cand_out, int* cand_idx_out, cudaStream_t st);
-int launch_topk_rescore(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad, long long n_rows, const float* an,
+template <typename T>
+int launch_topk_rescore(const T* A, const T* B, int Dpad, long long n_rows, const float* an,
                         const float* bn, const int* cand_idx, const float* cand_val, int k, float delta,
                         const float* outsider_bound, float* nv, int* flagged, int* flagged_cnt, int flagged_cap,
                         float* best_d, int* best_idx, cudaStream_t st);
-int launch_topk_exhaustive(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad, long long n_b, const float* an,
+template <typename T>
+int launch_topk_exhaustive(const T* A, const T* B, int Dpad, long long n_b, const float* an,
                            const float* bn, const int* flagged, const int* flagged_cnt, int flagged_cap, int k, float* nv,
                            float* best_d, int* best_idx, cudaStream_t st);
-int launch_pair_score(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, long long n, const float* xn, const float* yn,
+template <typename T>
+int launch_pair_score(const T* X, const T* Y, int Dpad, long long n, const float* xn, const float* yn,
                       const float* nv1, const float* nv2, int use_csls, float* g, float* s_out, cudaStream_t st);
-int launch_band_rescore(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, const float* xn, const float* yn,
+template <typename T>
+int launch_band_rescore(const T* X, const T* Y, int Dpad, const float* xn, const float* yn,
                         const float* nv1, const float* nv2, const float* g_row, const float* g_col, int row_gid0, int col_gid0,
                         int use_csls, const uint2* band, const unsigned int* band_cnt, unsigned int band_cap, int* cnt_row,
                         int* cnt_col, cudaStream_t st, const int* row_gids = nullptr, int swapped = 0);
-int launch_pairs_dot(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, const int* rows, const int* cols,
+template <typename T>
+int launch_pairs_dot(const T* X, const T* Y, int Dpad, const int* rows, const int* cols,
                      long long n_pairs, float* s_out, cudaStream_t st);
 int launch_top4_merge(const float* val, const int* idx, int n_lists, long long n_rows, float* oval, int* oidx, cudaStream_t st);
-int launch_top3_rescore(const __nv_bfloat16* X, const __nv_bfloat16* Y, int Dpad, long long n_rows, const float* xn,
+template <typename T>
+int launch_top3_rescore(const T* X, const T* Y, int Dpad, long long n_rows, const float* xn,
                         const float* yn, const float* nv1, const float* nv2, int use_csls, const int* cand, float* oval,
                         int* oidx, cudaStream_t st);
 int launch_icl_finalize(const float* rowsum_part, int n_chunks, int B, int Bp, const float* pos, float inv_tau, float* lse,
@@ -161,7 +169,8 @@ int launch_rank_judge(const uint2* rk_stream, const int* rk_stream_row, const in
                       const float* R, const float* Rp, const float* C, const float* Cp, const unsigned char* row_ok,
                       const unsigned char* col_ok, float eps, int row_gid0, int col_gid0, int* cnt_row, int* cnt_col,
                       uint2* band, unsigned int* band_cnt, unsigned int band_cap, int* overflow, cudaStream_t st);
-int launch_rank_exhaustive(const __nv_bfloat16* A, const __nv_bfloat16* B, int Dpad, long long n_b, const float* an,
+template <typename T>
+int launch_rank_exhaustive(const T* A, const T* B, int Dpad, long long n_b, const float* an,
                            const float* bn, const float* nva, const float* nvb, const float* g, const int* rows, int n_rows,
                            int a_gid0, int b_gid0, int use_csls, int swapped, int* cnt, cudaStream_t st);
 int launch_col_threshold(const float* cand, long long n, int k, const float* yn, float* colthr, float* colb, cudaStream_t st);

@@ -660,13 +660,26 @@ def _graphed(final_emb, test_left, test_right, csls, csls_k, want_top3, normaliz
     return g(final_emb, test_left, test_right)
 
 
+PRECISIONS = ("bf16", "fp32")
+EVAL_PRECISION = "bf16"     # what Runner._test evaluates with (python -m snag_b200.patch --eval-precision fp32 sets it)
+
+
+def _check_precision(precision: str) -> None:
+    if precision not in PRECISIONS:
+        raise ValueError(f"precision={precision!r}: expected one of {PRECISIONS}")
+
+
 def evaluate_alignment(final_emb: torch.Tensor, test_left: torch.Tensor, test_right: torch.Tensor, csls: bool = True,
                        csls_k: int = 10, want_top3: bool = False, normalize: bool = True, group=None,
-                       graph: bool | None = None) -> dict:
+                       graph: bool | None = None, precision: str = "bf16") -> dict:
     """The evaluation a user of the reference gets from Runner._test, as a function:
     final_emb [N, D] fp32 (device), test_left/right LongTensor [n] -> metrics for both directions.
     graph (default: on for a single GPU and fewer than TWO_SWEEP_MIN_N pairs): replay the evaluation as one CUDA graph
-    captured on the first call with this shape — the reference evaluates the same test set after every epoch."""
+    captured on the first call with this shape — the reference evaluates the same test set after every epoch.
+    precision: "bf16" (default) ranks the normalised rows rounded to bf16; "fp32" ranks the unrounded fp32 rows, as the
+    reference does (snag_b200.fp32: split-bf16 sweeps, canonical re-scores on the fp32 rows), so that ranks, nv1 / nv2,
+    g and Hits@k / MR / MRR equal the reference's bit for bit. fp32 needs csls_k <= KT and runs without the CUDA graph."""
+    _check_precision(precision)
     n = test_left.numel()
     if test_right.numel() != n:
         raise ValueError("test_left and test_right must pair up")
@@ -674,8 +687,12 @@ def evaluate_alignment(final_emb: torch.Tensor, test_left: torch.Tensor, test_ri
         raise ValueError(f"csls_k={csls_k}")
     if csls and csls_k > n:
         raise ValueError(f"csls_k={csls_k} exceeds the number of evaluated pairs n={n}")
+    if precision == "fp32" and csls and csls_k > KT:
+        raise SnagError(f"precision='fp32' with csls_k={csls_k} > {KT}: the materialised evaluation is bf16 only")
     if not final_emb.is_cuda:
         raise SnagError("evaluate_alignment: final_emb must live on the GPU (there is no CPU path)")
+    if precision == "fp32":
+        return _evaluate_fp32(final_emb, test_left, test_right, csls, csls_k, want_top3, normalize, group)
     if csls and csls_k > KT:
         # the fused sweeps keep KT candidates per entity; larger neighbourhoods (the reference takes any k) are evaluated
         # on the materialised matrix
@@ -697,6 +714,34 @@ def evaluate_alignment(final_emb: torch.Tensor, test_left: torch.Tensor, test_ri
         "ranks": res,
         "launches": res.launches + 2,
     }
+
+
+def _evaluate_fp32(final_emb, test_left, test_right, csls: bool, csls_k: int, want_top3: bool, normalize: bool, group) -> dict:
+    """evaluate_alignment(precision="fp32"): the fused evaluation with the kernel backend snag_b200.fp32."""
+    from . import fp32
+    n = test_left.numel()
+    X, xn = fp32.prep(final_emb, test_left.to(torch.int64).contiguous(), normalize, 0)
+    Y, yn = fp32.prep(final_emb, test_right.to(torch.int64).contiguous(), normalize, 1)
+    if float(torch.maximum(xn[:n].max(), yn[:n].max()).item()) > 8.0:
+        raise SnagError("the fused evaluation expects L2-normalised rows (evaluate_alignment(normalize=True))")
+    if group is None:
+        world, rank = 1, 0
+    else:
+        import torch.distributed as dist
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+    gen = _align_ranks_steps(fp32, X, Y, xn, yn, n, csls_k, csls, want_top3, world, rank)
+    if world == 1:
+        try:
+            next(gen)
+        except StopIteration as stop:
+            res = stop.value
+        else:
+            raise AssertionError("single-rank evaluation requested a collective")
+    else:
+        res = _drive_with_torch_distributed(gen, group)
+    res.info["precision"] = "fp32"
+    return {"l2r": metrics_from_ranks(res.rank_l2r), "r2l": metrics_from_ranks(res.rank_r2l), "ranks": res,
+            "launches": res.launches + 4}
 
 
 def evaluate_alignment_materialised(final_emb: torch.Tensor, test_left: torch.Tensor, test_right: torch.Tensor, csls: bool = True,
@@ -900,14 +945,19 @@ def _stream_in_with_prepasses(src_rows, tgt_rows, n: int, csls_k: int, normalize
 
 
 def evaluate_alignment_host(src_rows: torch.Tensor, tgt_rows: torch.Tensor, n: int, row0: int = 0, csls: bool = True,
-                            csls_k: int = 10, normalize: bool = True, group=None, device=None, stream_in: bool | None = None) -> dict:
+                            csls_k: int = 10, normalize: bool = True, group=None, device=None, stream_in: bool | None = None,
+                            precision: str = "bf16") -> dict:
     """End-to-end entry point from HOST memory: `src_rows` / `tgt_rows` are (ideally pinned) fp32 [m, D] host tensors
     holding pairs row0 .. row0+m of the n evaluated pairs — all of them on a single GPU, or this rank's contiguous
     slice (ceil(n / world) pairs per rank) when `group` is given. Copies them to the device, normalises and rounds
     them, exchanges the bf16 operands over NCCL so that every rank holds both tables, runs the sharded fused
     evaluation, brings the ranks back and reduces them to Hits@k / MR / MRR on the host.
     stream_in (default: single GPU, CSLS, n >= TWO_SWEEP_MIN_N): transfer the tables in chunks and run the prologue and
-    the sample pre-passes on the chunks as they arrive (_stream_in_with_prepasses); the result is bit-identical."""
+    the sample pre-passes on the chunks as they arrive (_stream_in_with_prepasses); the result is bit-identical.
+    precision: "bf16" only (the fp32 evaluation takes device tables: evaluate_alignment(precision="fp32"))."""
+    _check_precision(precision)
+    if precision != "bf16":
+        raise SnagError("evaluate_alignment_host evaluates bf16 operands only: use evaluate_alignment(precision='fp32')")
     if device is None:
         device = torch.device("cuda", torch.cuda.current_device())
     m, d = src_rows.shape

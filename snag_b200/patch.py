@@ -1,8 +1,13 @@
 """Drop-in installation into an UNMODIFIED checkout of zjukg/SNAG (SNAG_MMEA).
 
-    python -m snag_b200.patch /path/to/SNAG_MMEA [main.py flags ...]      # runs main.py with the hot path replaced
+    python -m snag_b200.patch [--eval-precision fp32] /path/to/SNAG_MMEA [main.py flags ...]
+                                                      # runs main.py with the hot path replaced
 or, from Python:
     import snag_b200.patch as sp; sp.patch()         # after SNAG_MMEA is on sys.path, before Runner is built
+
+--eval-precision fp32 (patch(eval_precision="fp32")): Runner._test ranks the unrounded fp32 embeddings, as the reference
+does, instead of their bf16 rounding (snag_b200.evaluate.EVAL_PRECISION); the flag is consumed before main.py parses
+its arguments.
 
 patch() assigns attributes — main.py, model/*.py and src/*.py stay byte-identical:
     model.SNAG_loss.icl_loss / ial_loss / CustomMultiLossLayer            -> snag_b200.loss
@@ -42,9 +47,13 @@ def unpatch() -> int:
     return n
 
 
-def patch(main_module: types.ModuleType | None = None) -> list[str]:
-    """Install the replacements into whichever reference modules are importable; returns what was patched."""
+def patch(main_module: types.ModuleType | None = None, eval_precision: str | None = None) -> list[str]:
+    """Install the replacements into whichever reference modules are importable; returns what was patched.
+    eval_precision ("bf16" or "fp32", None = leave as is): what Runner._test evaluates with."""
     done = []
+    if eval_precision is not None:
+        evaluate._check_precision(eval_precision)
+        evaluate.EVAL_PRECISION = eval_precision
 
     def _set(mod, name, value, label=None):
         # obj.__dict__ rather than getattr: a function stored on a class must be put back as the plain function
@@ -96,7 +105,26 @@ def patch(main_module: types.ModuleType | None = None) -> list[str]:
     return done
 
 
-def run_main(reference_dir: str, argv: list[str]) -> None:
+def parse_args(argv: list[str]) -> tuple[str | None, str, list[str]]:
+    """(eval_precision or None, reference directory, main.py's arguments) from this module's command line: the options
+    of snag_b200.patch precede the reference directory; everything after it belongs to main.py."""
+    precision = None
+    i = 0
+    while i < len(argv) and argv[i].startswith("--eval-precision"):
+        if argv[i] == "--eval-precision":
+            if i + 1 >= len(argv):
+                raise SystemExit("--eval-precision needs a value (bf16 or fp32)")
+            precision, i = argv[i + 1], i + 2
+        else:
+            precision, i = argv[i].split("=", 1)[1], i + 1
+        if precision not in evaluate.PRECISIONS:
+            raise SystemExit(f"--eval-precision {precision}: expected one of {evaluate.PRECISIONS}")
+    if i >= len(argv):
+        raise SystemExit(__doc__)
+    return precision, argv[i], list(argv[i + 1:])
+
+
+def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = None) -> None:
     """Execute the reference's main.py (unchanged on disk) with the hot path patched in: the module body is executed
     first, the patch is applied (Runner now exists), then the `if __name__ == "__main__":` block runs."""
     reference_dir = os.path.abspath(reference_dir)
@@ -104,7 +132,7 @@ def run_main(reference_dir: str, argv: list[str]) -> None:
     sys.path.insert(0, reference_dir)
     os.chdir(reference_dir)
     sys.argv = [path] + list(argv)
-    patch()                                           # model.*, src.* before main.py binds their names
+    patch(eval_precision=eval_precision)              # model.*, src.* before main.py binds their names
     tree = ast.parse(open(path).read(), filename=path)
     body, tail = [], []
     for node in tree.body:
@@ -121,6 +149,5 @@ def run_main(reference_dir: str, argv: list[str]) -> None:
 
 
 if __name__ == "__main__":
-    if len(sys.argv) < 2:
-        raise SystemExit(__doc__)
-    run_main(sys.argv[1], sys.argv[2:])
+    _precision, _ref_dir, _argv = parse_args(sys.argv[1:])
+    run_main(_ref_dir, _argv, _precision)

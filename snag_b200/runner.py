@@ -44,7 +44,7 @@ def _test(self, test_left, test_right, last_epoch=False, save_name="", loss=None
             # and both ranking loops (:400-429) in one call; the normalisation happens on the gathered rows only
             out = evaluate.evaluate_alignment(final_emb.float().contiguous(), test_left, test_right,
                                               csls=self.args.csls is True, csls_k=self.args.csls_k,
-                                              want_top3=bool(last_epoch))
+                                              want_top3=bool(last_epoch), precision=evaluate.EVAL_PRECISION)
     top_k = [1, 10, 50]
     l2r, r2l = out["l2r"], out["r2l"]
     acc_l2r, mean_l2r, mrr_l2r = l2r.acc, l2r.mr, l2r.mrr
