@@ -195,9 +195,10 @@ int snag_sim_write_t_mn(const uint16_t* XT, int32_t xt_ld, const uint16_t* Y, in
 /* Measurement aid: the same TMA + tcgen05 sweep with the accumulators dropped (no epilogue, no output).
  * Times the mainloop alone so that bench.py can attribute a sweep's time to mainloop vs fused epilogue. */
 int snag_sim_mainloop_only(const uint16_t* X, const uint16_t* Y, int32_t n1, int32_t n2, int32_t Dpad, void* stream);
-/* Development aid: counters = zeroed device buffer of 2*snag_num_sms()*4 uint64 (or NULL to switch off). While set, the UMMA-
+/* Development aid: counters = zeroed device buffer of 4*snag_num_sms()*4 uint64 (or NULL to switch off). While set, the UMMA-
  * issuing thread of every CTA of every sweep records {total cycles, cycles waiting for a free accumulator stage
- * (epilogue-bound), cycles waiting for operands (TMA-bound), tiles}. Process-global, not thread-safe. */
+ * (epilogue-bound), cycles waiting for operands (TMA-bound), tiles}; the fused evaluation sweeps add their flag and
+ * per-test counters (scripts/onepass_attrib.py reads them). Process-global, not thread-safe. */
 int snag_debug_counters(uint64_t* counters);
 /* CSLS sweep 1 (src/utils.py:431-432 without the matrix): for every row of X the SNAG_KT largest
  * c_ij = 1 - d_ij over the columns of each chunk. part: fp32 [n_lists][n1][SNAG_KT] (n_lists from

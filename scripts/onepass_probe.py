@@ -18,7 +18,7 @@ X, xn = ops.prep_bf16(emb, left, True)
 Y, yn = ops.prep_bf16(emb, right, True)
 del emb
 sms = ops.num_sms()
-dbg = torch.zeros((2 * sms, 4), dtype=torch.int64, device=dev)
+dbg = torch.zeros((4 * sms, 4), dtype=torch.int64, device=dev)   # rows 2*sms.. : EpiOnePass per-test counters
 records = []
 
 

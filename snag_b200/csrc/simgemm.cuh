@@ -58,9 +58,11 @@ struct SimShape {
   int a_mn;             // 1: the X operand is given TRANSPOSED — tmX maps a [K rows, n_rows columns] matrix (box 64 x 64) and
                         // the A tile is read MN-major (the gradient GEMMs contract over the rows of the stacked embeddings,
                         // which are stored with the output dimension contiguous; no transposed copy is made)
-  unsigned long long* dbg;   // optional [2*gridDim.x][4] cycle counters (zeroed by the caller) or null. Row cta: UMMA issuer
+  unsigned long long* dbg;   // optional [4*gridDim.x][4] cycle counters (zeroed by the caller) or null. Row cta: UMMA issuer
                              // total, its wait for a free accumulator stage, sum over epilogue warps of strip time,
-                             // tiles. Row gridDim.x + cta: sum over epilogue warps of commit + barrier time.
+                             // tiles. Row gridDim.x + cta: sum over epilogue warps of commit + barrier time, then the
+                             // fused evaluation epilogues' flag counters; rows 2*gridDim.x.. : EpiRowColTopKT's per-test
+                             // counters.
 };
 
 struct EpiCtx {
@@ -119,11 +121,12 @@ struct EpiWG { static constexpr int value = NUM_EPI_WG; };
 template <class E>
 struct EpiWG<E, std::void_t<decltype(E::kWG)>> { static constexpr int value = E::kWG; };
 
-// optional per-CTA hook run by the epilogue threads after their last unit: Epi::kernel_end(params, ctx)
+// optional per-CTA hook run by the epilogue threads after their last unit: Epi::kernel_end(params, shape, ctx)
 template <class E, class = void>
 struct HasKernelEnd : std::false_type {};
 template <class E>
-struct HasKernelEnd<E, decltype(E::kernel_end(std::declval<const typename E::Params&>(), std::declval<const EpiCtx&>()), void())>
+struct HasKernelEnd<E, decltype(E::kernel_end(std::declval<const typename E::Params&>(), std::declval<const SimShape&>(),
+                                              std::declval<const EpiCtx&>()), void())>
     : std::true_type {};
 
 template <class Epi>
@@ -348,7 +351,7 @@ sim_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUte
       }
       Epi::unit_end(ep, shp, cx, st);
     }
-    if constexpr (HasKernelEnd<Epi>::value) Epi::kernel_end(ep, cx);
+    if constexpr (HasKernelEnd<Epi>::value) Epi::kernel_end(ep, shp, cx);
     if (dbg && lane == 0) {      // summed over the epilogue warps: cycles consuming strips / cycles in commit + barrier
       atomicAdd(shp.dbg + blockIdx.x * 4 + 2, static_cast<unsigned long long>(c_proc));
       atomicAdd(shp.dbg + (gridDim.x + blockIdx.x) * 4 + 0, static_cast<unsigned long long>(c_bar));
@@ -625,8 +628,8 @@ struct EpiRowTopK {
 //     bandwidth kernels bucket the streams by column afterwards. (Letting the row owner re-check its own flagged
 //     columns through 32 predicated blocks needs no staging but measured 10-20 % slower.)
 // ------------------------------------------------------------------------------------------------
-// r[q] for a WARP-UNIFORM run-time q: a switch the compiler turns into an indexed branch (BRX) — every lane takes the same
-// case, so there is no divergence and no local-memory spill of the register strip
+// r[q] for a run-time q: a switch the compiler turns into a branch tree, so the register strip is never spilled to local
+// memory; lanes that ask for different q take different leaves, one after the other
 __device__ __forceinline__ uint32_t strip_value(const uint32_t (&r)[32], int q) {
   uint32_t v = 0;
   switch (q) {
@@ -711,19 +714,26 @@ struct EpiRowColTopKT {
   static constexpr int kHalfOff = kVecs * BN + BN / 32;             // 16-byte aligned: (kVecs*256 + 8) * 4 bytes
   static constexpr int kVecStride = kHalfOff + (kRank ? 3 : 1) * (BN / 2);
   static constexpr int kCntOff = 2 * kVecStride;         // int: candidates appended by this CTA so far (+1: rank stream)
-  static __device__ __forceinline__ void kernel_end(const Params& p, const EpiCtx& cx) {
+  // diagnostics (shp.dbg set): what the exact tests made of the flagged elements, unsigned counters per CTA: accepted by
+  // the row top-k test, appended as column candidates, above the l2r / r2l rank threshold, accepted by none of them
+  enum { kDbgRow, kDbgCol, kDbgL2r, kDbgR2l, kDbgNone, kDbgN };
+  static constexpr int kDbgOff = kCntOff + 2;
+  static __device__ __forceinline__ void kernel_end(const Params& p, const SimShape& shp, const EpiCtx& cx) {
     named_bar_sync(1, NUM_EPI_THREADS);
     if (cx.tid == 0) {
       p.stream_cnt[blockIdx.x] = *reinterpret_cast<const int*>(cx.scratch + kCntOff);
       if (kRank) p.rk_cnt[blockIdx.x] = *reinterpret_cast<const int*>(cx.scratch + kCntOff + 1);
+      if (shp.dbg != nullptr) {            // rows 2*gridDim.x + cta: row, col, l2r, r2l; 3*gridDim.x + cta: none
+        const unsigned* d = reinterpret_cast<const unsigned*>(cx.scratch + kDbgOff);
+        for (int t = 0; t < kDbgN; ++t) shp.dbg[((2 + t / 4) * gridDim.x + blockIdx.x) * 4 + t % 4] = d[t];
+      }
     }
   }
   static __device__ __forceinline__ void unit_begin(const Params& p, const SimShape&, const EpiCtx& cx, State& st) {
-    static_assert(kCntOff + 2 <= EPI_VEC_FLOATS, "scratch too small");
+    static_assert(kDbgOff + kDbgN <= EPI_VEC_FLOATS, "scratch too small");
     static_assert((kHalfOff % 4) == 0 && (kVecStride % 4) == 0, "fp16x2 vectors must be 16-byte aligned");
     if (cx.useq == 0 && cx.tid == 0) {                     // ordered by the tile barrier
-      *reinterpret_cast<int*>(cx.scratch + kCntOff) = 0;
-      *reinterpret_cast<int*>(cx.scratch + kCntOff + 1) = 0;
+      for (int t = 0; t < 2 + kDbgN; ++t) reinterpret_cast<int*>(cx.scratch + kCntOff)[t] = 0;
     }
     st.xn = cx.row_ok ? p.xn[cx.row] : 0.f;
     st.a = cx.row_ok ? 0.5f * st.xn : INFINITY;          // padding rows never produce column candidates
@@ -829,63 +839,87 @@ struct EpiRowColTopKT {
       fm |= __hgt2_mask(h, m) & ((1u << pq) | (0x10000u << pq));
     }
     if (!__any_sync(0xffffffffu, fm != 0)) return;
-    // Slow path, warp-uniform: walk the columns ANY row of this warp flagged; the column index is the same for all lanes,
-    // so the accumulator is fetched from the register strip through an indexed (uniform) branch, and the flagging rows
-    // run the exact tests. No shared-memory staging, no transposition: top-k insertion touches only the row's own
-    // registers and the two appends are stateless, so the row owner does all three. (Measured alternatives: staging the
-    // strip in shared memory + handing column candidates to a column-owning lane: -20 % SM clock at the 1 kW power cap;
-    // re-reading the column from TMEM with tcgen05.ld.x1: ~1 200 cycles per flagged column, epilogue-bound.)
-    uint32_t um = __reduce_or_sync(0xffffffffu, fm);
-    if (shp.dbg != nullptr) {               // diagnostics: flagged strips / flagged columns / flagged elements of this CTA
+    // Slow path. Each lane walks the columns IT flagged, so the warp iterates max over lanes of popc(fm) times (the union
+    // of the flagged columns, walked by the whole warp, is several times longer when the flags sit in different rows and
+    // columns, as they mostly do). The accumulator comes out of the register strip through an indexed branch that
+    // diverges only over the distinct columns of one step; no shared-memory staging, no transposition. The row owner
+    // runs all the exact tests: top-k insertion touches only its own registers, and the appends are warp-aggregated
+    // (stream_slot). (Measured alternatives: staging the strip in shared memory + handing column candidates to a
+    // column-owning lane: -20 % SM clock at the 1 kW power cap; re-reading the column from TMEM with tcgen05.ld.x1:
+    // ~1 200 cycles per flagged column, epilogue-bound.)
+    const bool dbg = shp.dbg != nullptr;
+    if (dbg) {                              // diagnostics: flagged strips / flagged columns / flagged elements of this CTA
       const int nf = __reduce_add_sync(0xffffffffu, __popc(fm));
+      const uint32_t um = __reduce_or_sync(0xffffffffu, fm);
       if (cx.lane == 0) {
         atomicAdd(shp.dbg + (gridDim.x + blockIdx.x) * 4 + 1, 1ull);
         atomicAdd(shp.dbg + (gridDim.x + blockIdx.x) * 4 + 2, static_cast<unsigned long long>(__popc(um)));
         atomicAdd(shp.dbg + (gridDim.x + blockIdx.x) * 4 + 3, static_cast<unsigned long long>(nf));
       }
     }
-    while (um != 0) {
-      const int b = __ffs(um) - 1;
-      um &= um - 1;
-      const int q = b < 16 ? 2 * b : 2 * (b - 16) + 1;
-      const float sv = __uint_as_float(strip_value(r, q));          // q is warp-uniform: an indexed branch, no divergence
-      if (((fm >> b) & 1u) != 0) {
-      const float ynq = yn_s[q];
-      float x = 0.f;
-      const bool want_row = sv > thr, want_col = sv > __fadd_rn(st.a, cb_s[q]);
-      if (want_row || want_col) x = __fsub_rn(1.0f, sqdist_from_dot(sv, st.xn, ynq));
-      if (want_row && x > st.top[0]) topk_list_insert<true>(st.top, st.topi, x, ct * BN + c * 32 + q);
-      if (want_col && x >= ct_s[q]) {
-        // column candidate (column, c, row): appended to this CTA's private stream, a shared-memory counter hands out
-        // the slot (no global-atomic round trip on the epilogue's critical path); a later pass buckets the streams by
-        // column. The counter saturates just above the capacity (overflow is detected by cnt > cap; letting it run on
-        // could wrap 32 bits when nearly everything is streamed).
-        volatile int* cc = reinterpret_cast<volatile int*>(cx.scratch + kCntOff);
-        if (*cc <= p.cta_cap) {
-          const int slot = atomicAdd(reinterpret_cast<int*>(cx.scratch + kCntOff), 1);
-          if (slot < p.cta_cap) {
-            const long long o = static_cast<long long>(blockIdx.x) * p.cta_cap + slot;
-            p.stream[o] = make_uint2(static_cast<uint32_t>(ct * BN + c * 32 + q), __float_as_uint(x));
-            p.stream_row[o] = cx.row;
-          }
+    const uint32_t col0 = static_cast<uint32_t>(ct * BN + c * 32);
+    int* cnt = reinterpret_cast<int*>(cx.scratch + kCntOff);
+    do {
+      bool app_col = false, app_rk = false;
+      uint32_t col = 0, dflags = 0;
+      float sv = 0.f, x = 0.f;
+      if (fm != 0) {
+        const int b = __ffs(fm) - 1;
+        fm &= fm - 1;
+        const int q = b < 16 ? 2 * b : 2 * (b - 16) + 1;
+        col = col0 + q;
+        sv = __uint_as_float(strip_value(r, q));
+        const bool want_row = sv > thr, want_col = sv > __fadd_rn(st.a, cb_s[q]);
+        if (want_row || want_col) x = __fsub_rn(1.0f, sqdist_from_dot(sv, st.xn, yn_s[q]));
+        const bool acc_row = want_row && x > st.top[0];
+        if (acc_row) topk_list_insert<true>(st.top, st.topi, x, static_cast<int>(col));
+        app_col = want_col && x >= ct_s[q];
+        if (kRank && !(SNAG_OPX & 4)) {
+          const float t_l2r = __fadd_rn(st.rk_r, kc_s[q]), t_r2l = __fadd_rn(st.rk_rp, kp_s[q]);
+          app_rk = sv > fminf(t_l2r, t_r2l);
+          if (dbg) dflags = (sv > t_l2r ? 1u << kDbgL2r : 0u) | (sv > t_r2l ? 1u << kDbgR2l : 0u);
+        }
+        if (dbg) {
+          dflags |= (acc_row ? 1u << kDbgRow : 0u) | (app_col ? 1u << kDbgCol : 0u);
+          if (dflags == 0) dflags = 1u << kDbgNone;
         }
       }
-      if (kRank && !(SNAG_OPX & 4)) {
-        if (sv > fminf(__fadd_rn(st.rk_r, kc_s[q]), __fadd_rn(st.rk_rp, kp_s[q]))) {
-          // rank candidate: (column, tensor-core s, row)
-          volatile int* kc = reinterpret_cast<volatile int*>(cx.scratch + kCntOff + 1);
-          if (*kc <= p.rk_cap) {
-            const int slot = atomicAdd(reinterpret_cast<int*>(cx.scratch + kCntOff + 1), 1);
-            if (slot < p.rk_cap) {
-              const long long o = static_cast<long long>(blockIdx.x) * p.rk_cap + slot;
-              p.rk_stream[o] = make_uint2(static_cast<uint32_t>(ct * BN + c * 32 + q), __float_as_uint(sv));
-              p.rk_stream_row[o] = cx.row;
-            }
-          }
+      // column candidate (column, c, row); rank candidate (column, tensor-core s, row)
+      int slot = stream_slot(app_col, cnt, p.cta_cap, cx.lane);
+      if (slot >= 0) {
+        const long long o = static_cast<long long>(blockIdx.x) * p.cta_cap + slot;
+        p.stream[o] = make_uint2(col, __float_as_uint(x));
+        p.stream_row[o] = cx.row;
+      }
+      if (kRank) {
+        slot = stream_slot(app_rk, cnt + 1, p.rk_cap, cx.lane);
+        if (slot >= 0) {
+          const long long o = static_cast<long long>(blockIdx.x) * p.rk_cap + slot;
+          p.rk_stream[o] = make_uint2(col, __float_as_uint(sv));
+          p.rk_stream_row[o] = cx.row;
         }
       }
+      if (dbg) {
+#pragma unroll
+        for (int t = 0; t < kDbgN; ++t) {
+          const int v = __popc(__ballot_sync(0xffffffffu, (dflags >> t) & 1u));
+          if (cx.lane == 0 && v != 0) atomicAdd(reinterpret_cast<unsigned*>(cx.scratch + kDbgOff) + t, static_cast<unsigned>(v));
+        }
       }
-    }
+    } while (__any_sync(0xffffffffu, fm != 0));
+  }
+  // Slot of this lane's entry in a CTA-private stream (-1: nothing to append, or the stream is full). One shared-memory
+  // atomicAdd per warp hands out consecutive slots to the lanes with pred set, in lane order. The counter stops growing
+  // once it exceeds cap (overflow is detected by count > cap; letting it run on could wrap 32 bits when nearly everything
+  // is streamed). Warp-collective: every lane of the warp calls it.
+  static __device__ __forceinline__ int stream_slot(bool pred, int* cnt, int cap, int lane) {
+    const uint32_t bal = __ballot_sync(0xffffffffu, pred);
+    if (bal == 0) return -1;
+    const int leader = __ffs(bal) - 1;
+    int base = 0;
+    if (lane == leader) base = *reinterpret_cast<volatile int*>(cnt) <= cap ? atomicAdd(cnt, __popc(bal)) : cap;
+    base = __shfl_sync(0xffffffffu, base, leader) + __popc(bal & ((1u << lane) - 1u));
+    return pred && base < cap ? base : -1;
   }
   static __device__ __forceinline__ void tile_end(const Params&, const SimShape&, const EpiCtx&, State&, int, int) {}
   static __device__ __forceinline__ void unit_end(const Params& p, const SimShape& shp, const EpiCtx& cx, State& st) {
@@ -926,7 +960,7 @@ struct EpiRowColTopKF32 {
   static constexpr int kVecStride = 3 * BN + BN / 32;
   static constexpr int kXnOff = 2 * kVecStride;
   static constexpr int kCntOff = kXnOff + 2 * BM;        // int: candidates appended by this CTA so far
-  static __device__ __forceinline__ void kernel_end(const Params& p, const EpiCtx& cx) {
+  static __device__ __forceinline__ void kernel_end(const Params& p, const SimShape&, const EpiCtx& cx) {
     named_bar_sync(1, NUM_EPI_THREADS);
     if (cx.tid == 0) p.stream_cnt[blockIdx.x] = *reinterpret_cast<const int*>(cx.scratch + kCntOff);
   }
