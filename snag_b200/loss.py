@@ -71,13 +71,18 @@ class AutomaticWeightedLoss(nn.Module):
         return loss_sum
 
 
-MAX_INV_TAU = 80.0     # exp((s - 1)/tau) must not underflow for every term of a row: (s - 1)/tau >= -2/tau > -87.3 * 2
+# The kernels evaluate E = ex2.approx.ftz((s - 1) log2(e) / tau), which flushes results below 2^-126 to zero, and the
+# backward scales each row by g exp(1/tau - lse) / tau <= g / (tau E_min) in fp32. For bf16-rounded unit rows
+# s >= -(1 + 2^-8)^2, so no term of a row underflows while 2 (1 + 2^-8)^2 log2(e) / tau <= 126 (1/tau <= 43.3), and
+# the row scale stays finite for 1/tau <= 40 (exp(2 (1 + 2^-8)^2 40) 40 < 2^128).
+MAX_INV_TAU = 40.0
 
 
 def _check_tau(tau: float) -> float:
     """The fused sweeps evaluate exp(s/tau - 1/tau) with the fixed maximum 1/tau (rows are unit norm) instead of a
-    running row maximum; for 1/tau beyond ~80 a row whose similarities are all <= 0 would underflow to a zero row sum
-    (the reference's log_softmax never does). Refuse such temperatures instead of returning inf."""
+    running row maximum; beyond MAX_INV_TAU a row whose similarities are all negative enough (one anchor anti-correlated
+    with the batch) would underflow to a zero row sum, where the reference's log_softmax stays finite. Refuse such
+    temperatures instead of returning inf."""
     inv_tau = float(1.0 / tau)
     if not 0.0 < inv_tau <= MAX_INV_TAU:
         raise ValueError(f"tau={tau}: the fused contrastive kernels support 1/tau in (0, {MAX_INV_TAU:g}] "
