@@ -21,6 +21,7 @@ import torch
 
 from . import ops as _cuda_ops
 from ._lib import KT, SnagError
+from .ops import round_up
 
 TOP_K = (1, 10, 50)   # main.py:380
 
@@ -39,10 +40,6 @@ class AlignRanks:
     top3_val: torch.Tensor | None = None
     launches: int = 0                 # kernels of libsnag_b200.so launched by this rank
     info: dict = field(default_factory=dict)
-
-
-def round_up(x: int, m: int) -> int:
-    return (x + m - 1) // m * m
 
 
 def shard_bounds(n: int, world: int, rank: int, align: int = 256) -> tuple[int, int]:
@@ -412,6 +409,30 @@ def _drive_with_torch_distributed(gen, group):
         return stop.value
 
 
+def _world_rank(group) -> tuple[int, int]:
+    if group is None:
+        return 1, 0
+    import torch.distributed as dist
+    return dist.get_world_size(group), dist.get_rank(group)
+
+
+def _run_steps(gen, group=None):
+    """The result of an _align_ranks_steps generator: through torch.distributed with a group, else on this rank alone."""
+    if group is not None:
+        return _drive_with_torch_distributed(gen, group)
+    try:
+        next(gen)
+    except StopIteration as stop:
+        return stop.value
+    raise AssertionError("single-rank evaluation requested a collective")
+
+
+def _result(res: AlignRanks, launches: int, **extra) -> dict:
+    """What the evaluate_alignment* entry points return: Hits@k / MR / MRR of both directions and the ranks."""
+    return {"l2r": metrics_from_ranks(res.rank_l2r), "r2l": metrics_from_ranks(res.rank_r2l), "ranks": res,
+            "launches": launches, **extra}
+
+
 def simulate_sharded(make_gen, world: int):
     """Run `world` rank generators in lockstep inside one process (used by tests and single-GPU checks of the
     sharding logic): make_gen(rank) -> generator as produced by _align_ranks_steps."""
@@ -480,13 +501,7 @@ def _align_ranks_lazy(be, X, Y, xn, yn, n, csls_k, use_csls, want_top3):
     """Single-rank, three-sweep evaluation without any host synchronisation until ONE read of four counters at the end
     (what makes the evaluation of a reference-sized test set — 10 500 pairs, every epoch with --eval_epoch 1 — launch
     bound otherwise: ~8 round trips). Returns None when the read shows that an assumption did not hold."""
-    gen = _align_ranks_steps(be, X, Y, xn, yn, n, csls_k, use_csls, want_top3, 1, 0, False, lazy=True)
-    try:
-        next(gen)
-    except StopIteration as stop:
-        res = stop.value
-    else:
-        raise AssertionError("single-rank evaluation requested a collective")
+    res = _run_steps(_align_ranks_steps(be, X, Y, xn, yn, n, csls_k, use_csls, want_top3, 1, 0, False, lazy=True))
     status = _pending_status(res, xn, yn, n).cpu()        # the one synchronisation
     if not _resolve_pending(res, status):
         return None
@@ -519,11 +534,7 @@ def align_ranks(X: torch.Tensor, Y: torch.Tensor, xn: torch.Tensor, yn: torch.Te
     # from that instead of silently weakening the guarantee. Squared norms up to 8 are let through for small exact
     # (dyadic) test inputs.
     be = _cuda_ops if _backend is None else _backend     # test seam: host-logic tests run the generator on a CPU stand-in
-    if group is None:
-        world, rank = 1, 0
-    else:
-        import torch.distributed as dist
-        world, rank = dist.get_world_size(group), dist.get_rank(group)
+    world, rank = _world_rank(group)
     if lazy is None:
         lazy = world == 1 and _backend is None and n < TWO_SWEEP_MIN_N
     if lazy:
@@ -534,15 +545,8 @@ def align_ranks(X: torch.Tensor, Y: torch.Tensor, xn: torch.Tensor, yn: torch.Te
         raise SnagError("align_ranks expects L2-normalised rows (evaluate_alignment(normalize=True))")
     if pre is not None and (world != 1 or not use_csls or two_sweep_plan(n, csls_k) is None or not two_sweep):
         raise ValueError("pre-computed sample pre-passes apply to the single-rank two-sweep CSLS path only")
-    gen = _align_ranks_steps(be, X, Y, xn, yn, n, csls_k, use_csls, want_top3, world, rank, two_sweep, one_pass=one_pass,
-                             pre=pre)
-    if world == 1:
-        try:
-            next(gen)
-        except StopIteration as stop:
-            return stop.value
-        raise AssertionError("single-rank evaluation requested a collective")
-    return _drive_with_torch_distributed(gen, group)
+    return _run_steps(_align_ranks_steps(be, X, Y, xn, yn, n, csls_k, use_csls, want_top3, world, rank, two_sweep,
+                                         one_pass=one_pass, pre=pre), group)
 
 
 # =================================================================================================
@@ -596,12 +600,8 @@ class _GraphedEvaluation:
         def run():
             X, xn = _cuda_ops.prep_bf16(self.emb, self.left, self.normalize)
             Y, yn = _cuda_ops.prep_bf16(self.emb, self.right, self.normalize)
-            gen = _align_ranks_steps(_cuda_ops, X, Y, xn, yn, n, csls_k, csls, want_top3, 1, 0, False, lazy=True)
-            try:
-                next(gen)
-            except StopIteration as stop:
-                return stop.value, _pending_status(stop.value, xn, yn, n)
-            raise AssertionError("single-rank evaluation requested a collective")
+            res = _run_steps(_align_ranks_steps(_cuda_ops, X, Y, xn, yn, n, csls_k, csls, want_top3, 1, 0, False, lazy=True))
+            return res, _pending_status(res, xn, yn, n)
 
         self._run = run
 
@@ -669,6 +669,20 @@ def _check_precision(precision: str) -> None:
         raise ValueError(f"precision={precision!r}: expected one of {PRECISIONS}")
 
 
+def _check_eval_args(what: str, final_emb, test_left, test_right, csls: bool, csls_k: int) -> int:
+    """The refusals evaluate_alignment and evaluate_alignment_l1 share; returns the number of pairs n."""
+    n = test_left.numel()
+    if test_right.numel() != n:
+        raise ValueError("test_left and test_right must pair up")
+    if csls and csls_k < 1:
+        raise ValueError(f"csls_k={csls_k}")
+    if csls and csls_k > n:
+        raise ValueError(f"csls_k={csls_k} exceeds the number of evaluated pairs n={n}")
+    if not final_emb.is_cuda:
+        raise SnagError(f"{what}: final_emb must live on the GPU (there is no CPU path)")
+    return n
+
+
 def evaluate_alignment(final_emb: torch.Tensor, test_left: torch.Tensor, test_right: torch.Tensor, csls: bool = True,
                        csls_k: int = 10, want_top3: bool = False, normalize: bool = True, group=None,
                        graph: bool | None = None, precision: str = "bf16") -> dict:
@@ -680,17 +694,9 @@ def evaluate_alignment(final_emb: torch.Tensor, test_left: torch.Tensor, test_ri
     reference does (snag_b200.fp32: split-bf16 sweeps, canonical re-scores on the fp32 rows), so that ranks, nv1 / nv2,
     g and Hits@k / MR / MRR equal the reference's bit for bit. fp32 needs csls_k <= KT and runs without the CUDA graph."""
     _check_precision(precision)
-    n = test_left.numel()
-    if test_right.numel() != n:
-        raise ValueError("test_left and test_right must pair up")
-    if csls and csls_k < 1:
-        raise ValueError(f"csls_k={csls_k}")
-    if csls and csls_k > n:
-        raise ValueError(f"csls_k={csls_k} exceeds the number of evaluated pairs n={n}")
     if precision == "fp32" and csls and csls_k > KT:
         raise SnagError(f"precision='fp32' with csls_k={csls_k} > {KT}: the materialised evaluation is bf16 only")
-    if not final_emb.is_cuda:
-        raise SnagError("evaluate_alignment: final_emb must live on the GPU (there is no CPU path)")
+    n = _check_eval_args("evaluate_alignment", final_emb, test_left, test_right, csls, csls_k)
     if precision == "fp32":
         return _evaluate_fp32(final_emb, test_left, test_right, csls, csls_k, want_top3, normalize, group)
     if csls and csls_k > KT:
@@ -703,17 +709,11 @@ def evaluate_alignment(final_emb: torch.Tensor, test_left: torch.Tensor, test_ri
         res = _graphed(final_emb.contiguous(), test_left.to(torch.int64), test_right.to(torch.int64), csls, csls_k,
                        want_top3, normalize)
         if res is not None:
-            return {"l2r": metrics_from_ranks(res.rank_l2r), "r2l": metrics_from_ranks(res.rank_r2l), "ranks": res,
-                    "launches": res.launches + 2}
+            return _result(res, res.launches + 2)
     X, xn = _cuda_ops.prep_bf16(final_emb, test_left.to(torch.int64).contiguous(), normalize)
     Y, yn = _cuda_ops.prep_bf16(final_emb, test_right.to(torch.int64).contiguous(), normalize)
     res = align_ranks(X, Y, xn, yn, n, csls_k, csls, want_top3, group)
-    return {
-        "l2r": metrics_from_ranks(res.rank_l2r),
-        "r2l": metrics_from_ranks(res.rank_r2l),
-        "ranks": res,
-        "launches": res.launches + 2,
-    }
+    return _result(res, res.launches + 2)
 
 
 def _evaluate_fp32(final_emb, test_left, test_right, csls: bool, csls_k: int, want_top3: bool, normalize: bool, group) -> dict:
@@ -724,24 +724,9 @@ def _evaluate_fp32(final_emb, test_left, test_right, csls: bool, csls_k: int, wa
     Y, yn = fp32.prep(final_emb, test_right.to(torch.int64).contiguous(), normalize, 1)
     if float(torch.maximum(xn[:n].max(), yn[:n].max()).item()) > 8.0:
         raise SnagError("the fused evaluation expects L2-normalised rows (evaluate_alignment(normalize=True))")
-    if group is None:
-        world, rank = 1, 0
-    else:
-        import torch.distributed as dist
-        world, rank = dist.get_world_size(group), dist.get_rank(group)
-    gen = _align_ranks_steps(fp32, X, Y, xn, yn, n, csls_k, csls, want_top3, world, rank)
-    if world == 1:
-        try:
-            next(gen)
-        except StopIteration as stop:
-            res = stop.value
-        else:
-            raise AssertionError("single-rank evaluation requested a collective")
-    else:
-        res = _drive_with_torch_distributed(gen, group)
+    res = _run_steps(_align_ranks_steps(fp32, X, Y, xn, yn, n, csls_k, csls, want_top3, *_world_rank(group)), group)
     res.info["precision"] = "fp32"
-    return {"l2r": metrics_from_ranks(res.rank_l2r), "r2l": metrics_from_ranks(res.rank_r2l), "ranks": res,
-            "launches": res.launches + 4}
+    return _result(res, res.launches + 4)
 
 
 def evaluate_alignment_materialised(final_emb: torch.Tensor, test_left: torch.Tensor, test_right: torch.Tensor, csls: bool = True,
@@ -754,12 +739,23 @@ def evaluate_alignment_materialised(final_emb: torch.Tensor, test_left: torch.Te
     if group is not None:
         raise SnagError(f"csls_k={csls_k} > {KT}: the materialised evaluation is not sharded")
     n = test_left.numel()
-    free, _total = torch.cuda.mem_get_info(final_emb.device)
+
+    def distances():
+        X, xn = _cuda_ops.prep_bf16(final_emb, test_left.to(torch.int64).contiguous(), normalize)
+        Y, yn = _cuda_ops.prep_bf16(final_emb, test_right.to(torch.int64).contiguous(), normalize)
+        return _cuda_ops.sim_write(X, Y, xn, yn, n, n, mode=1)                       # main.py:386
+
+    return _materialised(distances, n, final_emb.device, csls, csls_k, want_top3,
+                         {"materialised": True, "csls_k": int(csls_k)})
+
+
+def _materialised(distances, n: int, device, csls: bool, csls_k: int, want_top3: bool, info: dict) -> dict:
+    """The reference's composition on the materialised [n, n] fp32 matrix that distances() builds: csls_sim on
+    1 - distance, counting ranks of the diagonal with the stable-sort tie-break, and the top 3 of a stable sort."""
+    free, _total = torch.cuda.mem_get_info(device)
     if 3 * 4 * n * n > free:
         raise SnagError(f"csls_k={csls_k} > {KT} needs the materialised {n} x {n} matrix, which does not fit this device")
-    X, xn = _cuda_ops.prep_bf16(final_emb, test_left.to(torch.int64).contiguous(), normalize)
-    Y, yn = _cuda_ops.prep_bf16(final_emb, test_right.to(torch.int64).contiguous(), normalize)
-    dist = _cuda_ops.sim_write(X, Y, xn, yn, n, n, mode=1)                            # main.py:386
+    dist = distances()
     nv1 = nv2 = None
     if csls:
         out, nv1, nv2 = _cuda_ops.csls_sim_matrix(1 - dist, int(csls_k))              # main.py:393
@@ -770,9 +766,7 @@ def evaluate_alignment_materialised(final_emb: torch.Tensor, test_left: torch.Te
     if want_top3:
         order = torch.sort(dist, dim=1, stable=True)
         top3_idx, top3_val = order[1][:, :3].to(torch.int32), order[0][:, :3]
-    res = AlignRanks(rank_l2r, rank_r2l, nv1, nv2, torch.diagonal(dist).clone(), top3_idx, top3_val, 7,
-                     {"materialised": True, "csls_k": int(csls_k)})
-    return {"l2r": metrics_from_ranks(rank_l2r), "r2l": metrics_from_ranks(rank_r2l), "ranks": res, "launches": 7}
+    return _result(AlignRanks(rank_l2r, rank_r2l, nv1, nv2, torch.diagonal(dist).clone(), top3_idx, top3_val, 7, info), 7)
 
 
 def evaluate_alignment_l1(final_emb: torch.Tensor, test_left: torch.Tensor, test_right: torch.Tensor, csls: bool = True,
@@ -785,63 +779,23 @@ def evaluate_alignment_l1(final_emb: torch.Tensor, test_left: torch.Tensor, test
     reference's without the [n, n] matrix. With `group` every rank passes the same final_emb, sweeps its own shard of the
     targets and gets the full metrics. CSLS neighbourhoods larger than the KT candidates of the fused sweep are evaluated
     on the materialised matrix (single GPU)."""
-    n = test_left.numel()
-    if test_right.numel() != n:
-        raise ValueError("test_left and test_right must pair up")
-    if csls and csls_k > n:
-        raise ValueError(f"csls_k={csls_k} exceeds the number of evaluated pairs n={n}")
     materialised = csls and not 1 <= csls_k <= KT
     if materialised and group is not None:
         raise SnagError(f"csls_k={csls_k} > {KT}: the materialised evaluation is not sharded")
-    if not final_emb.is_cuda:
-        raise SnagError("evaluate_alignment_l1: final_emb must live on the GPU (there is no CPU path)")
+    n = _check_eval_args("evaluate_alignment_l1", final_emb, test_left, test_right, csls, csls_k)
     fe = torch.nn.functional.normalize(final_emb.float())                       # main.py:379
     left, right = test_left.to(torch.int64), test_right.to(torch.int64)
-    if materialised:
-        return _evaluate_l1_materialised(fe, left, right, csls_k, want_top3)
+    if materialised:            # fp64 index-order L1 sums
+        return _materialised(lambda: _cuda_ops.l1_distance(fe.index_select(0, left).contiguous(),
+                                                             fe.index_select(0, right).contiguous()),
+                             n, fe.device, True, csls_k, want_top3, {"distance": 1, "materialised": True})
     from . import l1
     X, xn = l1.prep(fe, left)
     Y, yn = l1.prep(fe, right)
-    if group is None:
-        world, rank = 1, 0
-    else:
-        import torch.distributed as dist
-        world, rank = dist.get_world_size(group), dist.get_rank(group)
-    gen = _align_ranks_steps(l1, X, Y, xn, yn, n, csls_k, csls, want_top3, world, rank, two_sweep=False)
-    if world == 1:
-        try:
-            next(gen)
-        except StopIteration as stop:
-            res = stop.value
-        else:
-            raise AssertionError("single-rank evaluation requested a collective")
-    else:
-        res = _drive_with_torch_distributed(gen, group)
+    res = _run_steps(_align_ranks_steps(l1, X, Y, xn, yn, n, csls_k, csls, want_top3, *_world_rank(group), two_sweep=False),
+                     group)
     res.info["distance"] = 1
-    return {"l2r": metrics_from_ranks(res.rank_l2r), "r2l": metrics_from_ranks(res.rank_r2l), "ranks": res,
-            "launches": res.launches + 2}
-
-
-def _evaluate_l1_materialised(fe: torch.Tensor, left: torch.Tensor, right: torch.Tensor, csls_k: int, want_top3: bool) -> dict:
-    """CSLS with csls_k > KT on --distance 1: the reference's composition on the materialised [n, n] fp32 matrix
-    (fp64 index-order L1 sums, csls_sim on 1 - distance, counting ranks with the stable-sort tie-break)."""
-    n = left.numel()
-    free, _total = torch.cuda.mem_get_info(fe.device)
-    if 3 * 4 * n * n > free:
-        raise SnagError(f"csls_k={csls_k} > {KT} needs the materialised {n} x {n} matrix, which does not fit this device")
-    x = fe.index_select(0, left).contiguous()
-    y = fe.index_select(0, right).contiguous()
-    dist = _cuda_ops.l1_distance(x, y)
-    out, nv1, nv2 = _cuda_ops.csls_sim_matrix(1 - dist, int(csls_k))             # main.py:393
-    dist = 1 - out
-    rank_l2r, rank_r2l = _cuda_ops.matrix_rank(dist)
-    top3_idx = top3_val = None
-    if want_top3:
-        order = torch.sort(dist, dim=1, stable=True)
-        top3_idx, top3_val = order[1][:, :3].to(torch.int32), order[0][:, :3]
-    res = AlignRanks(rank_l2r, rank_r2l, nv1, nv2, torch.diagonal(dist).clone(), top3_idx, top3_val, 7,
-                     {"distance": 1, "materialised": True})
-    return {"l2r": metrics_from_ranks(rank_l2r), "r2l": metrics_from_ranks(rank_r2l), "ranks": res, "launches": 7}
+    return _result(res, res.launches + 2)
 
 
 STREAM_CHUNK_ROWS = 65536      # rows per host -> device chunk of the streamed entry point (315 MB at D = 1200: ~6 ms of PCIe 5)
@@ -981,10 +935,7 @@ def evaluate_alignment_host(src_rows: torch.Tensor, tgt_rows: torch.Tensor, n: i
             raise ValueError("stream_in applies to the single-GPU two-sweep CSLS evaluation (n >= TWO_SWEEP_MIN_N)")
         X, Y, xn, yn, pre, launches = _stream_in_with_prepasses(src_rows, tgt_rows, n, csls_k, normalize, device, plan2[0])
         res = align_ranks(X, Y, xn, yn, n, csls_k, csls, False, None, pre=pre)
-        l2r = res.rank_l2r.cpu()
-        r2l = res.rank_r2l.cpu()
-        return {"l2r": metrics_from_ranks(l2r), "r2l": metrics_from_ranks(r2l), "ranks": res,
-                "launches": res.launches + launches, "streamed": True}
+        return _result(res, res.launches + launches, streamed=True)
     xs = src_rows.to(device, non_blocking=True)
     ys = tgt_rows.to(device, non_blocking=True)
     dpad = round_up(d, 64)
@@ -1011,10 +962,7 @@ def evaluate_alignment_host(src_rows: torch.Tensor, tgt_rows: torch.Tensor, n: i
         dist.all_gather_into_tensor(xn, xnl, group=group)
         dist.all_gather_into_tensor(yn, ynl, group=group)
     res = align_ranks(X, Y, xn[:n].contiguous(), yn[:n].contiguous(), n, csls_k, csls, False, group)
-    l2r = res.rank_l2r.cpu()
-    r2l = res.rank_r2l.cpu()
-    return {"l2r": metrics_from_ranks(l2r), "r2l": metrics_from_ranks(r2l), "ranks": res,
-            "launches": res.launches + launches}
+    return _result(res, res.launches + launches)
 
 
 # =================================================================================================

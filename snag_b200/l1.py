@@ -9,7 +9,7 @@ import ctypes
 import torch
 
 from ._lib import KT, SnagError, call, current_stream, ptr
-from .ops import _need, round_up
+from .ops import _band_retry, _need, round_up
 from .ops import num_sms, top4_merge, topk_merge_mean  # noqa: F401  (the generator calls them as be.*)
 
 LAST_TOPK_INFO: dict = {}
@@ -106,27 +106,22 @@ def eval_rank(X, Y, xn, yn, nv1, nv2, g_row, g_col, row_gid0: int, col_gid0: int
         nl = n_lists(n1, n2, X.shape[1])
         t3v = torch.empty((nl, n1, 4), dtype=torch.float32, device=dev)
         t3i = torch.empty((nl, n1, 4), dtype=torch.int32, device=dev)
-    cap = max(BAND_MIN_CAP, BAND_PER_ROW * (n1 + n2))
-    row_save, col_save = cnt_row.clone(), cnt_col.clone()
-    while True:
-        band = torch.empty((cap,), dtype=torch.int64, device=dev)
-        band_cnt = torch.zeros((1,), dtype=torch.int32, device=dev)
+
+    def attempt(band, band_cnt, cap):
         call("snag_l1_rank_band", ptr(X), ptr(Y), ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col), row_gid0,
              col_gid0, n1, n2, X.shape[1], int(use_csls), ptr(cnt_row), ptr(cnt_col), ptr(t3v), ptr(t3i), ptr(band),
              ptr(band_cnt), cap, st)
         call("snag_l1_band_rescore", ptr(X), ptr(Y), X.shape[1], ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col), row_gid0, col_gid0,
              int(use_csls), ptr(band), ptr(band_cnt), cap, ptr(cnt_row), ptr(cnt_col), st)
-        deferred = int(band_cnt.item()) & 0xFFFFFFFF
-        LAST_RANK_INFO.clear()
-        LAST_RANK_INFO.update(deferred=deferred, cap=cap, mode="band")
-        if deferred <= cap:
-            return t3v, t3i
-        if cap >= BAND_MAX_CAP:
-            raise SnagError(f"{deferred} elements of the L1 rank sweep are within the error bound of a ground-truth "
-                            f"distance (nearly all ties): more than the deferral list can hold")
-        cnt_row.copy_(row_save)               # the list overflowed: undo the partial counts and retry
-        cnt_col.copy_(col_save)
-        cap = min(BAND_MAX_CAP, max(cap * 4, round_up(deferred + deferred // 8, 1024)))
+
+    deferred, cap = _band_retry(attempt, max(BAND_MIN_CAP, BAND_PER_ROW * (n1 + n2)), (cnt_row, cnt_col), grow=4,
+                                max_cap=BAND_MAX_CAP, clamp=True)
+    LAST_RANK_INFO.clear()
+    LAST_RANK_INFO.update(deferred=deferred, cap=cap, mode="band")
+    if deferred > cap:
+        raise SnagError(f"{deferred} elements of the L1 rank sweep are within the error bound of a ground-truth "
+                        f"distance (nearly all ties): more than the deferral list can hold")
+    return t3v, t3i
 
 
 def top3_rescore(X, Y, xn, yn, nv1, nv2, use_csls: bool, cand: torch.Tensor):

@@ -147,6 +147,49 @@ def _check_operand(t: torch.Tensor, name: str) -> None:
         raise ValueError(f"{name}: base pointer must be 128-byte aligned")
 
 
+def _suffix(X: torch.Tensor, Y: torch.Tensor, names: str = "XY") -> str:
+    """Suffix of the canonical entry points for the row type of X and Y: "" (snag_X) for bf16 operands (prep_bf16),
+    "_f32" (snag_X_f32) for the fp32 rows of fp32.prep ([n, multiple of 64], 16-byte aligned)."""
+    for t, nm in ((X, names[0]), (Y, names[1])):
+        if isinstance(t, torch.Tensor) and t.dtype == torch.float32:
+            _need(t, torch.float32, nm, 2)
+            if t.shape[1] % 64 or t.data_ptr() % 16:
+                raise ValueError(f"{nm}: fp32 rows must be [n, multiple of 64] and 16-byte aligned")
+        else:
+            _check_operand(t, nm)
+    if X.dtype != Y.dtype:
+        raise TypeError(f"{names[0]} and {names[1]} must have the same dtype")
+    return "" if X.dtype == torch.bfloat16 else "_f32"
+
+
+def _band_retry(attempt, cap: int, counters: tuple, grow: int = 1, max_cap: int | None = None, clamp: bool = False,
+                sync: bool = True):
+    """The deferral-list protocol of the band sweeps. attempt(band, band_cnt, cap) enqueues a sweep or judge that lists
+    the elements it cannot decide in `band` (band_cnt counts them all, also those past cap) and their canonical
+    re-score, both adding to `counters`. After an overflow the counters are restored and the attempt repeats with
+    max(grow x cap, 9/8 of the count rounded up to 1024) entries, clamped to max_cap when `clamp`. Returns (deferred,
+    cap) of the last attempt; deferred > cap (counters restored) when the list would have to grow past max_cap or,
+    clamped, a list of max_cap overflowed. sync=False: one attempt, no host synchronisation (CUDA-graph capture);
+    returns the DEVICE band_cnt and cap, and the caller must check deferred <= cap before trusting the counters."""
+    dev = counters[0].device
+    saved = [t.clone() for t in counters] if sync else None
+    while True:
+        band = torch.empty((cap,), dtype=torch.int64, device=dev)
+        band_cnt = torch.zeros((1,), dtype=torch.int32, device=dev)
+        attempt(band, band_cnt, cap)
+        if not sync:
+            return band_cnt, cap
+        deferred = int(band_cnt.item()) & 0xFFFFFFFF
+        if deferred <= cap:
+            return deferred, cap
+        for t, s in zip(counters, saved):
+            t.copy_(s)
+        grown = max(grow * cap, round_up(deferred + deferred // 8, 1024))
+        if max_cap is not None and (cap >= max_cap if clamp else grown > max_cap):
+            return deferred, cap
+        cap = min(grown, max_cap) if clamp else grown
+
+
 # ------------------------------------------------------------------------------------------------ eval sweeps
 def sim_write(X: torch.Tensor, Y: torch.Tensor, xn: torch.Tensor | None, yn: torch.Tensor | None, n1: int, n2: int,
               mode: int) -> torch.Tensor:
@@ -301,7 +344,9 @@ def rank_judge(X, Y, xn, yn, nv1, nv2, g_row, g_col, row_gid0: int, col_gid0: in
                R, Rp, C, Cp, row_ok, col_ok, eps: float, cnt_row: torch.Tensor, cnt_col: torch.Tensor):
     """Settle the streamed rank candidates of eval_onepass against the final constants (snag_rank_judge) and re-score
     the elements inside the band canonically (snag_band_rescore); counts are accumulated into cnt_row / cnt_col.
+    X, Y are the canonical rows of the re-score (bf16 operands or fp32 rows).
     Returns (overflow int32[1] device tensor — a rank stream was full, the counts are incomplete —, deferred count)."""
+    sfx = _suffix(X, Y)
     _need(rk_stream, torch.int64, "rk_stream", 2)
     _need(rk_stream_row, torch.int32, "rk_stream_row", 2)
     _need(rk_cnt, torch.int32, "rk_cnt", 1)
@@ -309,50 +354,45 @@ def rank_judge(X, Y, xn, yn, nv1, nv2, g_row, g_col, row_gid0: int, col_gid0: in
         _need(t, torch.float32, name, 1)
     _need(row_ok, torch.uint8, "row_ok", 1)
     _need(col_ok, torch.uint8, "col_ok", 1)
-    dev = X.device
     n_ctas, rk_cap = rk_stream.shape
     st = current_stream()
-    overflow = torch.zeros((1,), dtype=torch.int32, device=dev)
-    cap = max(RANK_BAND_MIN_CAP, RANK_BAND_PER_ROW * (R.numel() + C.numel()))
-    row_save, col_save = cnt_row.clone(), cnt_col.clone()
-    while True:
-        band = torch.empty((cap,), dtype=torch.int64, device=dev)
-        band_cnt = torch.zeros((1,), dtype=torch.int32, device=dev)
+    overflow = torch.zeros((1,), dtype=torch.int32, device=X.device)
+
+    def attempt(band, band_cnt, cap):
         call("snag_rank_judge", ptr(rk_stream), ptr(rk_stream_row), ptr(rk_cnt), n_ctas, rk_cap, ptr(R), ptr(Rp), ptr(C), ptr(Cp),
              ptr(row_ok), ptr(col_ok), float(eps), row_gid0, col_gid0, ptr(cnt_row), ptr(cnt_col), ptr(band), ptr(band_cnt), cap,
              ptr(overflow), st)
-        call("snag_band_rescore", ptr(X), ptr(Y), X.shape[1], ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col),
-             row_gid0, col_gid0, 1, ptr(band), ptr(band_cnt), cap, ptr(cnt_row), ptr(cnt_col), st)
-        deferred = int(band_cnt.item()) & 0xFFFFFFFF
-        if deferred <= cap:
-            return overflow, deferred
-        cnt_row.copy_(row_save)
-        cnt_col.copy_(col_save)
-        cap = round_up(deferred + deferred // 8, 1024)
+        call("snag_band_rescore" + sfx, ptr(X), ptr(Y), X.shape[1], ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row),
+             ptr(g_col), row_gid0, col_gid0, 1, ptr(band), ptr(band_cnt), cap, ptr(cnt_row), ptr(cnt_col), st)
+
+    deferred, _ = _band_retry(attempt, max(RANK_BAND_MIN_CAP, RANK_BAND_PER_ROW * (R.numel() + C.numel())), (cnt_row, cnt_col))
+    return overflow, deferred
 
 
 def rank_exhaustive(A, B, an, bn, nva, nvb, g, rows: torch.Tensor, a_gid0: int, b_gid0: int, use_csls: bool, swapped: bool,
                     cnt: torch.Tensor, n_b: int | None = None) -> None:
     """cnt[row] += canonical rank count of every listed row of A against the first n_b rows of B (snag_rank_exhaustive)."""
-    _check_operand(A, "A")
-    _check_operand(B, "B")
+    sfx = _suffix(A, B, "AB")
     _need(rows, torch.int32, "rows", 1)
     _need(cnt, torch.int32, "cnt", 1)
     if rows.numel() == 0:
         return
-    call("snag_rank_exhaustive", ptr(A), ptr(B), A.shape[1], B.shape[0] if n_b is None else n_b, ptr(an), ptr(bn), ptr(nva),
-         ptr(nvb), ptr(g), ptr(rows), rows.numel(), a_gid0, b_gid0, int(use_csls), int(swapped), ptr(cnt), current_stream())
+    call("snag_rank_exhaustive" + sfx, ptr(A), ptr(B), A.shape[1], B.shape[0] if n_b is None else n_b, ptr(an), ptr(bn),
+         ptr(nva), ptr(nvb), ptr(g), ptr(rows), rows.numel(), a_gid0, b_gid0, int(use_csls), int(swapped), ptr(cnt), current_stream())
 
 
 def rank_recount_rows(A, B, an, bn, nva, nvb, g_a, g_b, rows: torch.Tensor, a_gid0: int, b_gid0: int, n_b: int,
-                      swapped: bool, eps: float) -> torch.Tensor:
+                      swapped: bool, eps: float, canon: tuple | None = None) -> torch.Tensor:
     """Rank counts of the listed rows of A against the first n_b rows of B by a tensor-core sweep over the gathered
     sub-panel (snag_eval_rank_band_rows + snag_band_rescore_rows): the recount of entities whose one-pass guess failed.
     A = sources and B = targets (swapped False: l2r ranks of the listed sources), or A = targets and B = sources
     (swapped True: r2l ranks of the listed targets). an / nva / g_a are indexed like A, bn / nvb / g_b like B.
+    canon: the canonical rows (of A, of B) of the re-score when they are not A and B (the fp32 rows of split operands).
     Returns int32 [len(rows)]."""
     _check_operand(A, "A")
     _check_operand(B, "B")
+    Ac, Bc = (A, B) if canon is None else canon
+    sfx = _suffix(Ac, Bc, "AB")
     _need(rows, torch.int32, "rows", 1)
     f = rows.numel()
     dev = A.device
@@ -361,24 +401,21 @@ def rank_recount_rows(A, B, an, bn, nva, nvb, g_a, g_b, rows: torch.Tensor, a_gi
         return cnt
     idx = rows.long()
     Af = A.index_select(0, idx)
+    Acf = Af if canon is None else Ac.index_select(0, idx)
     anf, nvaf, gf = an.index_select(0, idx), nva.index_select(0, idx), g_a.index_select(0, idx)
     gids = (rows + a_gid0).contiguous()
     scratch = torch.zeros((n_b,), dtype=torch.int32, device=dev)
     st = current_stream()
-    cap = max(RANK_BAND_MIN_CAP, RANK_BAND_PER_ROW * (f + n_b))
-    while True:
-        band = torch.empty((cap,), dtype=torch.int64, device=dev)
-        band_cnt = torch.zeros((1,), dtype=torch.int32, device=dev)
+
+    def attempt(band, band_cnt, cap):
         with _SweepTimer("sim_kernel<EpiRank>[recount]", f, n_b):
             call("snag_eval_rank_band_rows", ptr(Af), ptr(B), ptr(anf), ptr(bn), ptr(nvaf), ptr(nvb), ptr(gf), ptr(g_b), ptr(gids),
                  b_gid0, f, n_b, A.shape[1], 1, float(eps), ptr(cnt), ptr(scratch), ptr(band), ptr(band_cnt), cap, st)
-        call("snag_band_rescore_rows", ptr(Af), ptr(B), A.shape[1], ptr(anf), ptr(bn), ptr(nvaf), ptr(nvb), ptr(gf), ptr(g_b),
+        call("snag_band_rescore_rows" + sfx, ptr(Acf), ptr(Bc), Bc.shape[1], ptr(anf), ptr(bn), ptr(nvaf), ptr(nvb), ptr(gf), ptr(g_b),
              ptr(gids), b_gid0, 1, int(swapped), ptr(band), ptr(band_cnt), cap, ptr(cnt), ptr(scratch), st)
-        deferred = int(band_cnt.item()) & 0xFFFFFFFF
-        if deferred <= cap:
-            return cnt
-        cnt.zero_()
-        cap = round_up(deferred + deferred // 8, 1024)
+
+    _band_retry(attempt, max(RANK_BAND_MIN_CAP, RANK_BAND_PER_ROW * (f + n_b)), (cnt,))
+    return cnt
 
 
 def col_cand_reduce(stream: torch.Tensor, stream_row: torch.Tensor, stream_cnt: torch.Tensor, n_cols: int, k: int):
@@ -472,19 +509,21 @@ LAST_TOPK_INFO: dict = {}
 
 def topk_rescore(A, B, an, bn, cand_idx: torch.Tensor, cand_val: torch.Tensor, k: int, n_b: int, tag: str = "rows",
                  want_best: bool = False, outsider_bound: torch.Tensor | None = None, norm_bound: float | None = None,
-                 lazy: bool = False):
-    """Canonical CSLS neighbourhood means of the rows of A from their KT tensor-core candidates (rows of B); rows the
-    candidates cannot vouch for are completed by an exhaustive scan of B (within TOPK_EXHAUSTIVE_BUDGET; beyond it the
-    candidate-based value stays and the count is reported in LAST_TOPK_INFO[tag]['unverified']).
+                 lazy: bool = False, margin: float | None = None, info: dict | None = None):
+    """Canonical CSLS neighbourhood means of the rows of A from their KT tensor-core candidates (rows of B; bf16
+    operands or fp32 rows); rows the candidates cannot vouch for are completed by an exhaustive scan of B (within
+    TOPK_EXHAUSTIVE_BUDGET; beyond it the candidate-based value stays and the count is reported in
+    info[tag]['unverified'], info defaulting to LAST_TOPK_INFO).
+    margin: the verification half-width in s of the caller's error model (default: tc_margin of these bf16 operands).
     want_best: return (nv, best_d, best_idx) — every row's nearest row of B under the canonical squared distance, lowest
     index on ties (the argmin of link mining).
     outsider_bound [n_rows]: the admission threshold the lists were collected under, if any (see snag_topk_rescore).
     norm_bound: an upper bound of ||a|| ||b|| the caller vouches for (saves the host round trip that measures it).
     lazy: no host synchronisation at all — the exhaustive completion is enqueued unconditionally (it reads the flagged
     count on the device and does nothing when it is zero) for at most the budgeted number of rows, and
-    LAST_TOPK_INFO[tag] holds the DEVICE counter ('flagged_dev') and 'budget_rows' for the caller to check later."""
-    _check_operand(A, "A")
-    _check_operand(B, "B")
+    info[tag] holds the DEVICE counter ('flagged_dev') and 'budget_rows' for the caller to check later."""
+    sfx = _suffix(A, B, "AB")
+    info = LAST_TOPK_INFO if info is None else info
     _need(cand_idx, torch.int32, "cand_idx", 2)
     _need(cand_val, torch.float32, "cand_val", 2)
     n_rows = cand_idx.shape[0]
@@ -500,40 +539,39 @@ def topk_rescore(A, B, an, bn, cand_idx: torch.Tensor, cand_val: torch.Tensor, k
     cap = n_rows
     flagged = torch.empty((cap,), dtype=torch.int32, device=dev)
     fcnt = torch.zeros((1,), dtype=torch.int32, device=dev)
-    margin = tc_margin(A.shape[1], norm_bound) if norm_bound is not None else _error_scale(an, bn, A.shape[1])
-    call("snag_topk_rescore", ptr(A), ptr(B), A.shape[1], n_rows, ptr(an), ptr(bn), ptr(cand_idx), ptr(cand_val), k,
+    if margin is None:
+        margin = tc_margin(A.shape[1], norm_bound) if norm_bound is not None else _error_scale(an, bn, A.shape[1])
+    call("snag_topk_rescore" + sfx, ptr(A), ptr(B), A.shape[1], n_rows, ptr(an), ptr(bn), ptr(cand_idx), ptr(cand_val), k,
          TOPK_VERIFY_DELTA * margin, ptr(outsider_bound), ptr(nv), ptr(flagged), ptr(fcnt), cap,
          ptr(best_d), ptr(best_i), st)
     if lazy:
         budget_rows = int(min(cap, TOPK_EXHAUSTIVE_BUDGET // max(1, n_b * A.shape[1])))
         if budget_rows > 0:
-            call("snag_topk_exhaustive", ptr(A), ptr(B), A.shape[1], n_b, ptr(an), ptr(bn), ptr(flagged), ptr(fcnt), budget_rows,
+            call("snag_topk_exhaustive" + sfx, ptr(A), ptr(B), A.shape[1], n_b, ptr(an), ptr(bn), ptr(flagged), ptr(fcnt), budget_rows,
                  k, ptr(nv), ptr(best_d), ptr(best_i), st)
-        LAST_TOPK_INFO[tag] = {"flagged_dev": fcnt, "budget_rows": budget_rows}
+        info[tag] = {"flagged_dev": fcnt, "budget_rows": budget_rows}
         return (nv, best_d, best_i) if want_best else nv
     n_flag = int(fcnt.item())
-    info = {"flagged": n_flag, "unverified": 0}
+    info[tag] = {"flagged": n_flag, "unverified": 0}
     if n_flag:
         if float(n_flag) * n_b * A.shape[1] <= TOPK_EXHAUSTIVE_BUDGET:
-            call("snag_topk_exhaustive", ptr(A), ptr(B), A.shape[1], n_b, ptr(an), ptr(bn), ptr(flagged), ptr(fcnt), cap, k,
+            call("snag_topk_exhaustive" + sfx, ptr(A), ptr(B), A.shape[1], n_b, ptr(an), ptr(bn), ptr(flagged), ptr(fcnt), cap, k,
                  ptr(nv), ptr(best_d), ptr(best_i), st)
         else:
-            info["unverified"] = n_flag
+            info[tag]["unverified"] = n_flag
             import warnings
             warnings.warn(f"snag_b200: {n_flag} {tag} neighbourhoods could not be verified against the canonical arithmetic "
                           f"within the exhaustive budget (plateaus of near-equal similarities wider than {KT} - k); their "
                           f"CSLS means come from the tensor-core candidates and may differ from the reference in the last "
                           f"bits", RuntimeWarning, stacklevel=2)
-    LAST_TOPK_INFO[tag] = info
     return (nv, best_d, best_i) if want_best else nv
 
 
 def pair_score(X, Y, n: int, xn, yn, nv1, nv2, use_csls: bool, want_dot: bool = False):
-    _check_operand(X, "X")
-    _check_operand(Y, "Y")
+    sfx = _suffix(X, Y)
     g = torch.empty((n,), dtype=torch.float32, device=X.device)
     s = torch.empty((n,), dtype=torch.float32, device=X.device) if want_dot else None
-    call("snag_pair_score", ptr(X), ptr(Y), X.shape[1], n, ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), int(use_csls), ptr(g),
+    call("snag_pair_score" + sfx, ptr(X), ptr(Y), X.shape[1], n, ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), int(use_csls), ptr(g),
          ptr(s), current_stream())
     return (g, s) if want_dot else g
 
@@ -565,16 +603,24 @@ RANK_BAND_MAX_CAP = 1 << 28    # beyond this many deferred elements (2 GB list) 
 
 def eval_rank(X, Y, xn, yn, nv1, nv2, g_row, g_col, row_gid0: int, col_gid0: int, n1: int, n2: int, use_csls: bool,
               cnt_row: torch.Tensor, cnt_col: torch.Tensor, want_top3: bool = False, exact_chain: bool = False,
-              norm_bound: float | None = None, lazy: bool = False):
+              norm_bound: float | None = None, lazy: bool = False, eps: float | None = None, canon: tuple | None = None,
+              info: dict | None = None):
     """Rank counters of sweep 2, accumulated into cnt_row / cnt_col. Default: s-space sweep with a deferral band
     (snag_eval_rank_band) followed by the canonical re-score of the deferred elements (snag_band_rescore); a band list
     that overflows is retried with a larger list, and degenerate inputs (almost everything tied) fall back to the
     in-kernel fp32 chain (snag_eval_rank, `exact_chain=True`). Returns the per-list nearest-candidate lists
-    ([n_lists, n1, 4] values, ids) when want_top3, else (None, None).
-    lazy: one attempt with the initial list capacity and no host synchronisation; LAST_RANK_INFO holds the DEVICE
+    ([n_lists, n1, 4] values, ids) when want_top3, else (None, None). info (default LAST_RANK_INFO) reports the attempt.
+    eps: half-width of the band in s from the caller's error model (default: rank_band_eps of these bf16 operands).
+    canon: the canonical rows (Xr, Yr) of the re-score when they are not X and Y (the fp32 rows of split operands).
+    There is no chain on fp32 rows (its verdicts come from the tensor-core scores): their band list is clamped to
+    RANK_BAND_MAX_CAP, and past it this raises.
+    lazy: one attempt with the initial list capacity and no host synchronisation; info holds the DEVICE
     counter ('deferred_dev') and 'cap' — the caller must check deferred <= cap before trusting the counters."""
     _check_operand(X, "X")
     _check_operand(Y, "Y")
+    Xc, Yc = (X, Y) if canon is None else canon
+    sfx = _suffix(Xc, Yc)
+    info = LAST_RANK_INFO if info is None else info
     _need(cnt_row, torch.int32, "cnt_row", 1)
     _need(cnt_col, torch.int32, "cnt_col", 1)
     t3v = t3i = None
@@ -583,42 +629,38 @@ def eval_rank(X, Y, xn, yn, nv1, nv2, g_row, g_col, row_gid0: int, col_gid0: int
         t3v = torch.empty((nch, n1, 4), dtype=torch.float32, device=X.device)
         t3i = torch.empty((nch, n1, 4), dtype=torch.int32, device=X.device)
     st = current_stream()
+    if sfx and exact_chain:
+        raise ValueError("the in-kernel chain ranks bf16 operands only")
     if not exact_chain:
-        eps = RANK_BAND_EPS * (tc_margin(X.shape[1], norm_bound) if norm_bound is not None else _error_scale(xn, yn, X.shape[1]))
+        if eps is None:
+            eps = RANK_BAND_EPS * (tc_margin(X.shape[1], norm_bound) if norm_bound is not None else _error_scale(xn, yn, X.shape[1]))
         cap = max(RANK_BAND_MIN_CAP, RANK_BAND_PER_ROW * (n1 + n2))
+
+        def attempt(band, band_cnt, cap):
+            with _SweepTimer("sim_kernel<EpiRank>", n1, n2):
+                call("snag_eval_rank_band", ptr(X), ptr(Y), ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col),
+                     row_gid0, col_gid0, n1, n2, X.shape[1], int(use_csls), eps, ptr(cnt_row), ptr(cnt_col),
+                     ptr(t3v), ptr(t3i), ptr(band), ptr(band_cnt), cap, st)
+            call("snag_band_rescore" + sfx, ptr(Xc), ptr(Yc), Xc.shape[1], ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row),
+                 ptr(g_col), row_gid0, col_gid0, int(use_csls), ptr(band), ptr(band_cnt), cap, ptr(cnt_row), ptr(cnt_col), st)
+
         if lazy:
-            band = torch.empty((cap,), dtype=torch.int64, device=X.device)
-            band_cnt = torch.zeros((1,), dtype=torch.int32, device=X.device)
-            with _SweepTimer("sim_kernel<EpiRank>", n1, n2):
-                call("snag_eval_rank_band", ptr(X), ptr(Y), ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col),
-                     row_gid0, col_gid0, n1, n2, X.shape[1], int(use_csls), eps, ptr(cnt_row), ptr(cnt_col),
-                     ptr(t3v), ptr(t3i), ptr(band), ptr(band_cnt), cap, st)
-            call("snag_band_rescore", ptr(X), ptr(Y), X.shape[1], ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row),
-                 ptr(g_col), row_gid0, col_gid0, int(use_csls), ptr(band), ptr(band_cnt), cap, ptr(cnt_row), ptr(cnt_col), st)
-            LAST_RANK_INFO.clear()
-            LAST_RANK_INFO.update(deferred_dev=band_cnt, cap=cap, mode="band", eps=eps)
+            band_cnt, cap = _band_retry(attempt, cap, (cnt_row, cnt_col), sync=False)
+            info.clear()
+            info.update(deferred_dev=band_cnt, cap=cap, mode="band", eps=eps)
             return t3v, t3i
-        row_save = col_save = None
-        while cap <= RANK_BAND_MAX_CAP:
-            band = torch.empty((cap,), dtype=torch.int64, device=X.device)
-            band_cnt = torch.zeros((1,), dtype=torch.int32, device=X.device)
-            if row_save is None:
-                row_save, col_save = cnt_row.clone(), cnt_col.clone()
-            with _SweepTimer("sim_kernel<EpiRank>", n1, n2):
-                call("snag_eval_rank_band", ptr(X), ptr(Y), ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col),
-                     row_gid0, col_gid0, n1, n2, X.shape[1], int(use_csls), eps, ptr(cnt_row), ptr(cnt_col),
-                     ptr(t3v), ptr(t3i), ptr(band), ptr(band_cnt), cap, st)
-            call("snag_band_rescore", ptr(X), ptr(Y), X.shape[1], ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row),
-                 ptr(g_col), row_gid0, col_gid0, int(use_csls), ptr(band), ptr(band_cnt), cap, ptr(cnt_row), ptr(cnt_col), st)
-            deferred = int(band_cnt.item()) & 0xFFFFFFFF
-            LAST_RANK_INFO.update(deferred=deferred, cap=cap, mode="band", eps=eps)
+        if sfx or cap <= RANK_BAND_MAX_CAP:
+            deferred, cap = _band_retry(attempt, cap, (cnt_row, cnt_col), grow=8, max_cap=RANK_BAND_MAX_CAP, clamp=bool(sfx))
+            if sfx:
+                info.clear()
+            info.update(deferred=deferred, cap=cap, mode="band", eps=eps)
             if deferred <= cap:
                 return t3v, t3i
-            cnt_row.copy_(row_save)          # the list overflowed: undo the partial counts and retry
-            cnt_col.copy_(col_save)
-            cap = max(cap * 8, round_up(deferred + deferred // 8, 1024))
+            if sfx:
+                raise SnagError(f"{deferred} elements of the fp32 rank sweep are within the error bound of a ground-truth "
+                                f"distance (nearly all ties): more than the deferral list can hold")
         # hopeless (nearly everything within the band: duplicated / constant embeddings): in-kernel chain with exact ties
-    LAST_RANK_INFO.update(mode="chain")
+    info.update(mode="chain")
     with _SweepTimer("sim_kernel<EpiRank>", n1, n2):
         call("snag_eval_rank", ptr(X), ptr(Y), ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), ptr(g_row), ptr(g_col), row_gid0,
              col_gid0, n1, n2, X.shape[1], int(use_csls), ptr(cnt_row), ptr(cnt_col), ptr(t3v), ptr(t3i), st)
@@ -633,16 +675,16 @@ LAST_RANK_INFO: dict = {}
 
 
 def pairs_dot(X, Y, rows: torch.Tensor, cols: torch.Tensor) -> torch.Tensor:
-    """Canonical dot products X[rows[p]] . Y[cols[p]] (fp64 index-order accumulation, one rounding) of listed pairs."""
-    _check_operand(X, "X")
-    _check_operand(Y, "Y")
+    """Canonical dot products X[rows[p]] . Y[cols[p]] (fp64 index-order accumulation, one rounding) of listed pairs of
+    bf16 operands or fp32 rows."""
+    sfx = _suffix(X, Y)
     _need(rows, torch.int32, "rows", 1)
     _need(cols, torch.int32, "cols", 1)
     if rows.numel() != cols.numel():
         raise ValueError("rows and cols must pair up")
     out = torch.empty((rows.numel(),), dtype=torch.float32, device=X.device)
     if rows.numel():
-        call("snag_pairs_dot", ptr(X), ptr(Y), X.shape[1], ptr(rows), ptr(cols), rows.numel(), ptr(out), current_stream())
+        call("snag_pairs_dot" + sfx, ptr(X), ptr(Y), X.shape[1], ptr(rows), ptr(cols), rows.numel(), ptr(out), current_stream())
     return out
 
 
@@ -660,13 +702,12 @@ def top4_merge(val: torch.Tensor, idx: torch.Tensor):
 def top3_rescore(X, Y, xn, yn, nv1, nv2, use_csls: bool, cand: torch.Tensor):
     """Canonical distances of each row's candidate columns [n_rows, 4] (ids into Y), sorted ascending with the lower id
     first on ties: columns 0..2 are ret1..ret3 of the prediction file. Returns (val [n_rows, 4], idx [n_rows, 4])."""
-    _check_operand(X, "X")
-    _check_operand(Y, "Y")
+    sfx = _suffix(X, Y)
     _need(cand, torch.int32, "cand", 2)
     n_rows = cand.shape[0]
     oval = torch.empty((n_rows, 4), dtype=torch.float32, device=cand.device)
     oidx = torch.empty((n_rows, 4), dtype=torch.int32, device=cand.device)
-    call("snag_top3_rescore", ptr(X), ptr(Y), X.shape[1], n_rows, ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), int(use_csls),
+    call("snag_top3_rescore" + sfx, ptr(X), ptr(Y), X.shape[1], n_rows, ptr(xn), ptr(yn), ptr(nv1), ptr(nv2), int(use_csls),
          ptr(cand), ptr(oval), ptr(oidx), current_stream())
     return oval, oidx
 
