@@ -1,5 +1,6 @@
-"""Kernel backend of the fp32 evaluation (evaluate.evaluate_alignment(precision="fp32")): the entry points
-evaluate._align_ranks_steps calls, over the UNROUNDED fp32 normalised rows.
+"""Kernel backend of the fp32 evaluation (evaluate.evaluate_alignment(precision="fp32")) and of the fp32 link searches
+(mining / seeds with precision="fp32"): the entry points evaluate._align_ranks_steps, mining.mutual_nearest and
+seeds.topk_similarity_entries call, over the UNROUNDED fp32 rows.
 
 Every table is carried as a SplitOperand: its fp32 rows [n, Dpad] (what the canonical re-scores read, through the
 snag_*_f32 entry points) and a three-term bf16 split of them [n, 3 Dpad] (what the existing tcgen05 sweeps of
@@ -116,9 +117,10 @@ def eval_onepass(X, Y, *args, **kw):
     return ops.eval_onepass(X.split, Y.split, *args, **kw)
 
 
-def topk_rescore(A, B, an, bn, cand_idx, cand_val, k: int, n_b: int, tag: str = "rows", outsider_bound=None):
-    return ops.topk_rescore(A.rows, B.rows, an, bn, cand_idx, cand_val, k, n_b, tag, outsider_bound=outsider_bound,
-                            margin=_error_scale(an, bn, A.shape[1]), info=LAST_TOPK_INFO)
+def topk_rescore(A, B, an, bn, cand_idx, cand_val, k: int, n_b: int, tag: str = "rows", want_best: bool = False,
+                 outsider_bound=None):
+    return ops.topk_rescore(A.rows, B.rows, an, bn, cand_idx, cand_val, k, n_b, tag, want_best=want_best,
+                            outsider_bound=outsider_bound, margin=_error_scale(an, bn, A.shape[1]), info=LAST_TOPK_INFO)
 
 
 def pair_score(X, Y, *args, **kw):

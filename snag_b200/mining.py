@@ -4,18 +4,42 @@ driver main.py:214-223): mutual nearest neighbours between the non-train entitie
 The reference concatenates pairwise_distances over 1000-row slabs into a [n_left, n_right] fp32 matrix, takes
 torch.argmin along both axes and filters the pairs with Python list logic (O(n * |links|) membership tests).
 Here one fused tcgen05 sweep produces both argmin vectors (the matrix is never formed) and the link filtering is
-integer tensor work. Same arithmetic contract as the evaluation: operands are the bf16-rounded rows, d_ij follows
-src/utils.py:210-218 op by op in fp32, ties go to the lowest index like torch.argmin.
+integer tensor work. Same arithmetic contract as the evaluation: d_ij follows src/utils.py:210-218 op by op in fp32,
+ties go to the lowest index like torch.argmin, and the operands are the bf16-rounded rows (precision="bf16") or the
+unrounded fp32 rows (precision="fp32", the snag_b200.fp32 backend: split-bf16 sweeps, canonical re-scores on the fp32
+rows), as the reference mines them.
 """
 from __future__ import annotations
 
 import torch
 
+from . import fp32 as _fp32
 from . import ops as _cuda_ops
 from ._lib import KT, SnagError
+from .evaluate import _check_precision
+
+# What the trainer's link searches run on: Iter_new_links here and seeds.visual_pivot_induction
+# (python -m snag_b200.patch --link-precision fp32 sets it).
+LINK_PRECISION = "bf16"
 
 
-def mutual_nearest(x: torch.Tensor, y: torch.Tensor, normalize: bool = False, _backend=None, canonical: bool = True):
+def _backend_for(precision: str, _backend=None):
+    """The kernel backend of `precision`; _backend is a test seam (tests/oracle_backend.py), the product never passes it."""
+    if _backend is not None:
+        return _backend
+    return _fp32 if precision == "fp32" else _cuda_ops
+
+
+def _prep(be, precision: str, t: torch.Tensor, normalize: bool, side: int):
+    """(operand, ||row||^2) of `t` for the backend of `precision`; side 0 = the sweeps' sources, 1 = their targets (the
+    layout of fp32.prep's split operand; bf16 operands have one layout)."""
+    if precision == "fp32":
+        return be.prep(t.contiguous().float(), None, normalize, side)
+    return be.prep_bf16(t.contiguous().float(), None, normalize)
+
+
+def mutual_nearest(x: torch.Tensor, y: torch.Tensor, normalize: bool = False, _backend=None, canonical: bool = True,
+                   precision: str = "bf16"):
     """(preds_l int64 [n1], preds_r int64 [n2], dmin_l fp32 [n1], dmin_r fp32 [n2]): for every row of x its nearest row
     of y under the squared distance of src/utils.pairwise_distances, and vice versa.
 
@@ -24,11 +48,16 @@ def mutual_nearest(x: torch.Tensor, y: torch.Tensor, normalize: bool = False, _b
     the argmin — lowest index on ties, like torch.argmin — is taken over them, with the same verification bound and
     exhaustive completion as the CSLS neighbourhoods. The result does not depend on the MMA accumulation order.
     canonical=False: the single fused sweep (sim_kernel<EpiMutualNN>) that takes both argmins straight from the
-    tensor-core distances — exact ties still go to the lowest index, near-ties (< 1e-6) follow the tensor core."""
-    be = _cuda_ops if _backend is None else _backend     # test seam (tests/oracle_backend.py); the product never passes it
+    tensor-core distances — exact ties still go to the lowest index, near-ties (< 1e-6) follow the tensor core.
+    precision: "bf16" (default) mines the rows rounded to bf16; "fp32" mines the unrounded fp32 rows (canonical only):
+    argmins and minima are the oracle's on those rows."""
+    _check_precision(precision)
+    if precision == "fp32" and not canonical:
+        raise ValueError("canonical=False (the fused EpiMutualNN sweep) mines bf16 operands only")
+    be = _backend_for(precision, _backend)
     n1, n2 = x.shape[0], y.shape[0]
-    X, xn = be.prep_bf16(x.contiguous().float(), None, normalize)
-    Y, yn = be.prep_bf16(y.contiguous().float(), None, normalize)
+    X, xn = _prep(be, precision, x, normalize, 0)
+    Y, yn = _prep(be, precision, y, normalize, 1)      # the split pairing is positional: the swapped sweep works as well
     if canonical and hasattr(be, "topk_rescore"):
         out = []
         for A, B, an, bn, na, nb, tag in ((X, Y, xn, yn, n1, n2, "mine_rows"), (Y, X, yn, xn, n2, n1, "mine_cols")):
@@ -61,16 +90,19 @@ def mutual_nearest(x: torch.Tensor, y: torch.Tensor, normalize: bool = False, _b
     return preds_l, preds_r, dmin_l, dmin_r
 
 
-def iter_new_links(left_non_train, right_non_train, final_emb: torch.Tensor, new_links, refresh: bool, _backend=None):
+def iter_new_links(left_non_train, right_non_train, final_emb: torch.Tensor, new_links, refresh: bool, _backend=None,
+                   precision: str = "bf16"):
     """Body of Iter_new_links: mutual nearest pairs; when `refresh` is False only those already in `new_links` survive
     (model/SNAG.py:203-206). Entity ids in, list of (left id, right id) tuples out, in increasing order of the position
-    in `left_non_train` (the order of the reference's list comprehension)."""
+    in `left_non_train` (the order of the reference's list comprehension). precision: as mutual_nearest."""
+    _check_precision(precision)
     if len(left_non_train) == 0 or len(right_non_train) == 0:
         return new_links
     dev = final_emb.device
     left = torch.as_tensor(list(left_non_train), dtype=torch.int64, device=dev)
     right = torch.as_tensor(list(right_non_train), dtype=torch.int64, device=dev)
-    preds_l, preds_r, _, _ = mutual_nearest(final_emb.index_select(0, left), final_emb.index_select(0, right), _backend=_backend)
+    preds_l, preds_r, _, _ = mutual_nearest(final_emb.index_select(0, left), final_emb.index_select(0, right),
+                                            _backend=_backend, precision=precision)
     pos = torch.arange(left.numel(), device=dev)
     keep = preds_r[preds_l] == pos
     pl, pr = left[keep], right[preds_l[keep]]
@@ -83,6 +115,8 @@ def iter_new_links(left_non_train, right_non_train, final_emb: torch.Tensor, new
 
 
 def Iter_new_links(self, epoch, left_non_train, final_emb, right_non_train, new_links=[]):
-    """Drop-in for SNAG.Iter_new_links (same signature; installed on the reference class by snag_b200.patch)."""
+    """Drop-in for SNAG.Iter_new_links (same signature; installed on the reference class by snag_b200.patch). Mines in
+    LINK_PRECISION."""
     step = self.args.semi_learn_step
-    return iter_new_links(left_non_train, right_non_train, final_emb, new_links, (epoch + 1) % (step * 5) == step)
+    return iter_new_links(left_non_train, right_non_train, final_emb, new_links, (epoch + 1) % (step * 5) == step,
+                          precision=LINK_PRECISION)

@@ -1,13 +1,17 @@
 """Drop-in installation into an UNMODIFIED checkout of zjukg/SNAG (SNAG_MMEA).
 
-    python -m snag_b200.patch [--eval-precision fp32] /path/to/SNAG_MMEA [main.py flags ...]
+    python -m snag_b200.patch [--eval-precision fp32] [--link-precision fp32] /path/to/SNAG_MMEA [main.py flags ...]
                                                       # runs main.py with the hot path replaced
 or, from Python:
     import snag_b200.patch as sp; sp.patch()         # after SNAG_MMEA is on sys.path, before Runner is built
 
 --eval-precision fp32 (patch(eval_precision="fp32")): Runner._test ranks the unrounded fp32 embeddings, as the reference
-does, instead of their bf16 rounding (snag_b200.evaluate.EVAL_PRECISION); the flag is consumed before main.py parses
-its arguments.
+does, instead of their bf16 rounding (snag_b200.evaluate.EVAL_PRECISION). It governs Runner._test only.
+--link-precision fp32 (patch(link_precision="fp32")): the two searches that choose training links — the
+iterative-learning mining of SNAG.Iter_new_links and the seed induction of visual_pivot_induction (--unsup) — run on
+the unrounded fp32 rows instead of their bf16 rounding (snag_b200.mining.LINK_PRECISION), so that the links are the
+reference's. Both options come before the reference directory, in either order, and are consumed before main.py
+parses its arguments.
 
 patch() assigns attributes — main.py, model/*.py and src/*.py stay byte-identical:
     model.SNAG_loss.icl_loss / ial_loss / CustomMultiLossLayer            -> snag_b200.loss
@@ -47,13 +51,19 @@ def unpatch() -> int:
     return n
 
 
-def patch(main_module: types.ModuleType | None = None, eval_precision: str | None = None) -> list[str]:
+def patch(main_module: types.ModuleType | None = None, eval_precision: str | None = None,
+          link_precision: str | None = None) -> list[str]:
     """Install the replacements into whichever reference modules are importable; returns what was patched.
-    eval_precision ("bf16" or "fp32", None = leave as is): what Runner._test evaluates with."""
+    eval_precision ("bf16" or "fp32", None = leave as is): what Runner._test evaluates with.
+    link_precision (likewise): what Iter_new_links and visual_pivot_induction search with."""
     done = []
+    for precision in (eval_precision, link_precision):
+        if precision is not None:
+            evaluate._check_precision(precision)
     if eval_precision is not None:
-        evaluate._check_precision(eval_precision)
         evaluate.EVAL_PRECISION = eval_precision
+    if link_precision is not None:
+        mining.LINK_PRECISION = link_precision
 
     def _set(mod, name, value, label=None):
         # obj.__dict__ rather than getattr: a function stored on a class must be put back as the plain function
@@ -105,26 +115,42 @@ def patch(main_module: types.ModuleType | None = None, eval_precision: str | Non
     return done
 
 
-def parse_args(argv: list[str]) -> tuple[str | None, str, list[str]]:
-    """(eval_precision or None, reference directory, main.py's arguments) from this module's command line: the options
-    of snag_b200.patch precede the reference directory; everything after it belongs to main.py."""
-    precision = None
+class Options(tuple):
+    """(eval_precision or None, reference directory, main.py's arguments), with the link precision (or None) as the
+    attribute link_precision: a three-tuple, so that callers which unpack parse_args' result keep working."""
+
+    def __new__(cls, eval_precision: str | None, reference_dir: str, argv: list[str], link_precision: str | None = None):
+        self = super().__new__(cls, (eval_precision, reference_dir, argv))
+        self.link_precision = link_precision
+        return self
+
+
+_OPTIONS = ("--eval-precision", "--link-precision")
+
+
+def parse_args(argv: list[str]) -> Options:
+    """Options from this module's command line: the options of snag_b200.patch (--eval-precision, --link-precision, in
+    any order) precede the reference directory; everything after it belongs to main.py."""
+    values = dict.fromkeys(_OPTIONS)
     i = 0
-    while i < len(argv) and argv[i].startswith("--eval-precision"):
-        if argv[i] == "--eval-precision":
+    while i < len(argv) and argv[i].split("=", 1)[0] in _OPTIONS:
+        name = argv[i].split("=", 1)[0]
+        if argv[i] == name:
             if i + 1 >= len(argv):
-                raise SystemExit("--eval-precision needs a value (bf16 or fp32)")
-            precision, i = argv[i + 1], i + 2
+                raise SystemExit(f"{name} needs a value (bf16 or fp32)")
+            value, i = argv[i + 1], i + 2
         else:
-            precision, i = argv[i].split("=", 1)[1], i + 1
-        if precision not in evaluate.PRECISIONS:
-            raise SystemExit(f"--eval-precision {precision}: expected one of {evaluate.PRECISIONS}")
+            value, i = argv[i].split("=", 1)[1], i + 1
+        if value not in evaluate.PRECISIONS:
+            raise SystemExit(f"{name} {value}: expected one of {evaluate.PRECISIONS}")
+        values[name] = value
     if i >= len(argv):
         raise SystemExit(__doc__)
-    return precision, argv[i], list(argv[i + 1:])
+    return Options(values["--eval-precision"], argv[i], list(argv[i + 1:]), values["--link-precision"])
 
 
-def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = None) -> None:
+def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = None,
+             link_precision: str | None = None) -> None:
     """Execute the reference's main.py (unchanged on disk) with the hot path patched in: the module body is executed
     first, the patch is applied (Runner now exists), then the `if __name__ == "__main__":` block runs."""
     reference_dir = os.path.abspath(reference_dir)
@@ -132,7 +158,7 @@ def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = N
     sys.path.insert(0, reference_dir)
     os.chdir(reference_dir)
     sys.argv = [path] + list(argv)
-    patch(eval_precision=eval_precision)              # model.*, src.* before main.py binds their names
+    patch(eval_precision=eval_precision, link_precision=link_precision)    # model.*, src.* before main.py binds them
     tree = ast.parse(open(path).read(), filename=path)
     body, tail = [], []
     for node in tree.body:
@@ -149,5 +175,5 @@ def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = N
 
 
 if __name__ == "__main__":
-    _precision, _ref_dir, _argv = parse_args(sys.argv[1:])
-    run_main(_ref_dir, _argv, _precision)
+    _opts = parse_args(sys.argv[1:])
+    run_main(_opts[1], _opts[2], _opts[0], _opts.link_precision)

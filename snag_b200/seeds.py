@@ -4,34 +4,50 @@
 The reference forms the full [n_left, n_right] similarity matrix of the (L2-normalised) image / name / char features,
 takes the K = 100 * unsup_k largest entries with torch.topk over the flattened matrix and greedily keeps pairs whose
 entities are still unused. Here the matrix is never formed:
-  1. one top-k sweep (sim_kernel<EpiRowTopK>) gives every left entity's 16 best scores; the K-th largest of that pool is
-     a lower bound of the K-th largest entry of the whole matrix (the pool is a subset of it);
+  1. one top-k sweep (sim_kernel<EpiRowTopK>) gives every left entity's 16 best scores; the K-th largest of that pool,
+     lowered by the tensor-core error bound, is a lower bound of the tensor-core score of every entry whose canonical
+     score is among the K largest of the whole matrix (see _admission_threshold);
   2. one thresholded sweep (sim_kernel<EpiRowColTopK> with that bound as every column's admission threshold) streams
      out every entry at or above it — a superset of the global top K;
   3. the collected entries are re-scored with the canonical dot product (fp64, index order), sorted by
      (similarity descending, flat index ascending) and cut to K;
   4. the greedy matching runs on the host exactly as in the reference (sets instead of list scans).
-Operands are the bf16-rounded features (the same contract as the evaluation path).
+Operands are the bf16-rounded features (precision="bf16", the same contract as the evaluation path) or the unrounded
+fp32 features (precision="fp32": split-bf16 sweeps and fp32 canonical re-scores of snag_b200.fp32), as the reference
+ranks them.
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
+from . import mining
 from . import ops as _cuda_ops
 from ._lib import KT, SnagError
+from .evaluate import _check_precision
 
 
-def topk_similarity_entries(left_f: torch.Tensor, right_f: torch.Tensor, K: int, _backend=None):
+def _admission_threshold(pool_kth: torch.Tensor, eps: float) -> torch.Tensor:
+    """Admission threshold (in the sweep's score c = 2 s - 1) of the thresholded sweep, from the K-th largest
+    tensor-core score of the pool and eps, the backend's bound of |s_tensor_core - s_canonical| (tc_margin of the real
+    operands). The pool holds K entries with c_tc >= pool_kth, so K entries have s_canonical >= (1 + pool_kth)/2 - eps
+    and every entry of the canonical top K has at least that s_canonical, hence s_tc >= (1 + pool_kth)/2 - 2 eps:
+    c_tc >= pool_kth - 4 eps (a margin eps in s is 2 eps in c). eps includes 1e-6 for the fp32 roundings of c."""
+    return pool_kth - 4.0 * eps
+
+
+def topk_similarity_entries(left_f: torch.Tensor, right_f: torch.Tensor, K: int, _backend=None, precision: str = "bf16"):
     """(rows int64 [K'], cols int64 [K'], sims fp32 [K']) — the K' = min(K, n_l * n_r) largest entries of
-    left_f @ right_f.T in descending order, ties by ascending flat index (get_topk_indices, src/utils.py:437-443)."""
-    be = _cuda_ops if _backend is None else _backend     # test seam (tests/oracle_backend.py); the product never passes it
+    left_f @ right_f.T in descending order, ties by ascending flat index (get_topk_indices, src/utils.py:437-443).
+    precision: "bf16" (default) ranks the features rounded to bf16, "fp32" the unrounded fp32 features."""
+    _check_precision(precision)
+    be = mining._backend_for(precision, _backend)
     n_l, n_r = left_f.shape[0], right_f.shape[0]
     K = min(int(K), n_l * n_r)
     if K <= 0:
         raise ValueError("K must be positive")
-    X, _ = be.prep_bf16(left_f.contiguous().float(), None, normalize=False)
-    Y, _ = be.prep_bf16(right_f.contiguous().float(), None, normalize=False)
+    X, xn = mining._prep(be, precision, left_f, False, 0)
+    Y, yn = mining._prep(be, precision, right_f, False, 1)
     dev = X.device
     # with unit "norms" the sweep's score c = 1 - clamp(2 - 2 s, 0) = 2 s - 1 is monotone in s (s <= 1)
     one_l = torch.ones((n_l,), dtype=torch.float32, device=dev)
@@ -44,11 +60,13 @@ def topk_similarity_entries(left_f: torch.Tensor, right_f: torch.Tensor, K: int,
         # more entries requested than the per-row pools hold (K > 16 * n_left): every entry qualifies
         thr = torch.tensor(float("-inf"), device=dev)
     else:
-        thr = torch.topk(pool, K).values[-1] - 4e-6
+        eps = be.tc_margin(X.shape[1], float(torch.sqrt(xn.max() * yn.max()).item()))
+        thr = _admission_threshold(torch.topk(pool, K).values[-1], eps)
     colthr = torch.full((n_r,), float(thr), dtype=torch.float32, device=dev)
     colb = (0.5 * colthr - 4e-6).contiguous()                                       # s > (yn - 1 + thr)/2 with yn = 1
     n_ctas = int(_cuda_ops._lib.load().snag_num_sms()) if _backend is None else 148
     cap = _cuda_ops.round_up(int(2.5 * max(K, 4096) / n_ctas) + 4096, 1024)
+    # 12 bytes per stream entry (int64 column + c, int32 row) in n_ctas CTA-private streams, whatever the width
     while True:
         _, _, stream, stream_row, stream_cnt = be.eval_rowcoltopk(X, Y, one_l, one_r, n_l, n_r, colthr, colb, cap)
         cnt = stream_cnt.to(torch.int64)
@@ -72,13 +90,14 @@ def topk_similarity_entries(left_f: torch.Tensor, right_f: torch.Tensor, K: int,
 
 
 def visual_pivot_induction(args, left_ents, right_ents, img_features, ills, logger):
-    """Drop-in for src/data.visual_pivot_induction (same signature, same log lines, same int32 [n, 2] result)."""
+    """Drop-in for src/data.visual_pivot_induction (same signature, same log lines, same int32 [n, 2] result); ranks in
+    mining.LINK_PRECISION."""
     dev = torch.device("cuda", torch.cuda.current_device())
     feats = torch.as_tensor(img_features, dtype=torch.float32)
     l_img_f = feats[torch.as_tensor(list(left_ents), dtype=torch.int64)].to(dev)
     r_img_f = feats[torch.as_tensor(list(right_ents), dtype=torch.int64)].to(dev)
     topk = args.unsup_k
-    rows, cols, sims = topk_similarity_entries(l_img_f, r_img_f, topk * 100)
+    rows, cols, sims = topk_similarity_entries(l_img_f, r_img_f, topk * 100, precision=mining.LINK_PRECISION)
     print("highest sim:", sims[0].item(), "lowest sim:", sims[-1].item())              # src/utils.py:441
     rows, cols = rows.cpu().tolist(), cols.cpu().tolist()
     visual_links = []
