@@ -472,6 +472,35 @@ int snag_icl_bwd_logits(const uint16_t* X, const uint16_t* Y, int32_t B, int32_t
                         int32_t Dpad, float inv_tau, const float* cr, const float* cc, const float* dg, uint16_t* G,
                         int32_t self_cols, float ebar, void* stream);
 
+/* ---- fp32 loss route (icl_loss with precision "fp32") ----------------------------------------- */
+/* The contraction operands are a three-term bf16 split of the UNROUNDED normalised rows (as snag_prep_split): h = bf16(z),
+ * m = bf16(z - h). One split stack per table, [3 Bp, 5 Dpad] bf16 (128-byte aligned): row r of [a ; b ; a] (each part
+ * zero padded to Bp rows) laid out [m | h | h | m | h]; its side-0 window (columns [0, 3 Dpad)) is [m | h | h], its side-1
+ * window (columns [2 Dpad, 5 Dpad)) is [h | m | h], so a side-0 row contracted with a side-1 row over 3 Dpad gives
+ * m_i h_j + h_i m_j + h_i h_j (symmetric in i, j; |z_i z_j - that| <= 3 * 2^-16 |z_i| |z_j|). Dpad arguments below are
+ * the table's Dpad (a multiple of 64), not the stack's width.
+ * snag_icl_stack_prep_split : snag_icl_stack_prep with split stacks as out[p]; h is bit for bit snag_icl_stack_prep's
+ *                             output, m bit for bit snag_prep_split's.
+ * snag_icl_fwd_sym_split    : snag_icl_fwd_sym on split stacks S5[p] (no esave: a bf16 E would cap dL/dlogits at 2^-9);
+ *                             same plan, workspaces, unit ranges and snag_icl_sym_finalize.
+ * snag_icl_rowsum_split     : snag_icl_rowsum with X the side-0 window of the anchors' rows and Y the side-1 window of
+ *                             [other ; this] (rows 5 Dpad apart); snag_icl_finalize as usual.
+ * snag_icl_bwd_logits_split : snag_icl_bwd_logits (self_cols = 1, ebar = 0) on the same windows; G is formed in fp32 and
+ *                             written as G3 [nx, 6 Bp] bf16 (32-byte aligned) = [G_h | G_h | G_m], G_h = bf16(G),
+ *                             G_m = bf16(G - G_h). snag_sim_write_t_mn(XT = the K-stacked rows [Y_h ; Y_m ; Y_h]
+ *                             ([6 Bp, Dpad]), Y = G3, contraction 6 Bp) then gives G_h Y_h + G_h Y_m + G_m Y_h. */
+int snag_icl_stack_prep_split(int32_t n_prob, const float* const* emb, const int64_t* ld, const int32_t* D, uint16_t* const* out,
+                              const int32_t* Dpad, const int64_t* idx_l, const int64_t* idx_r, int32_t B, int32_t Bp,
+                              int32_t normalize, void* stream);
+int snag_icl_fwd_sym_split(int32_t n_prob, const uint16_t* const* S5, float* const* rowpart, float* const* colpart, float* pos,
+                           int32_t B, int32_t Bp, int32_t Dpad, float inv_tau, int32_t unit_begin, int32_t unit_end,
+                           float* total, void* stream);
+int snag_icl_rowsum_split(const uint16_t* X, const uint16_t* Y, int32_t B, int32_t Bp, int32_t row0, int32_t nx, int32_t Dpad,
+                          float inv_tau, float* rowsum_part, float* pos, void* stream);
+int snag_icl_bwd_logits_split(const uint16_t* X, const uint16_t* Y, int32_t B, int32_t Bp, int32_t row0, int32_t nx,
+                              int32_t Dpad, float inv_tau, const float* cr, const float* cc, const float* dg, uint16_t* G3,
+                              void* stream);
+
 #ifdef __cplusplus
 }
 #endif

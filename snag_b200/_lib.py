@@ -99,6 +99,10 @@ _SIGNATURES = {
     "snag_icl_g_from_e": [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _f32, _vp, _vp],
     "snag_icl_sym_finalize": [_vp, _vp, _i32, _i32, _i32, _f32, _vp, _vp],
     "snag_icl_bwd_logits": [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _f32, _vp, _vp, _vp, _vp, _i32, _f32, _vp],
+    "snag_icl_stack_prep_split": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp],
+    "snag_icl_fwd_sym_split": [_i32, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _f32, _i32, _i32, _vp, _vp],
+    "snag_icl_rowsum_split": [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _f32, _vp, _vp, _vp],
+    "snag_icl_bwd_logits_split": [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _f32, _vp, _vp, _vp, _vp, _vp],
 }
 EXPORTED_SYMBOLS = sorted(list(_SIGNATURES) + ["snag_error_string", "snag_csls_workspace_bytes", "snag_sim_write_t_splits",
                                                 "snag_icl_bwd_fused_splits"])

@@ -95,6 +95,14 @@ int snag_icl_stack_prep(int32_t n_prob, const float* const* emb, const int64_t* 
                                reinterpret_cast<__nv_bfloat16* const*>(out), Dpad, reinterpret_cast<const long long*>(idx_l),
                                reinterpret_cast<const long long*>(idx_r), B, Bp, normalize, S(stream));
 }
+int snag_icl_stack_prep_split(int32_t n_prob, const float* const* emb, const int64_t* ld, const int32_t* D, uint16_t* const* out,
+                              const int32_t* Dpad, const int64_t* idx_l, const int64_t* idx_r, int32_t B, int32_t Bp,
+                              int32_t normalize, void* stream) {
+  return launch_icl_stack_prep_split(n_prob, emb, reinterpret_cast<const long long*>(ld), D,
+                                     reinterpret_cast<__nv_bfloat16* const*>(out), Dpad,
+                                     reinterpret_cast<const long long*>(idx_l), reinterpret_cast<const long long*>(idx_r), B,
+                                     Bp, normalize, S(stream));
+}
 int snag_normalize_bwd_scatter_many(int32_t n_prob, const float* const* emb, const int64_t* ld, const int32_t* D,
                                     const float* const* dz_a, const float* const* dz_b, const int64_t* ld_dz,
                                     const int32_t* n_parts, const int64_t* part_stride, float* const* demb,
@@ -182,6 +190,12 @@ int snag_icl_fwd_sym(int32_t n_prob, const uint16_t* const* S3, float* const* ro
                      uint16_t* const* esave, void* stream) {
   return launch_icl_fwd_sym(n_prob, reinterpret_cast<const __nv_bfloat16* const*>(S3), rowpart, colpart, pos, B, Bp, Dpad,
                             inv_tau, unit_begin, unit_end, total, reinterpret_cast<__nv_bfloat16* const*>(esave), S(stream));
+}
+int snag_icl_fwd_sym_split(int32_t n_prob, const uint16_t* const* S5, float* const* rowpart, float* const* colpart, float* pos,
+                           int32_t B, int32_t Bp, int32_t Dpad, float inv_tau, int32_t unit_begin, int32_t unit_end,
+                           float* total, void* stream) {
+  return launch_icl_fwd_sym(n_prob, reinterpret_cast<const __nv_bfloat16* const*>(S5), rowpart, colpart, pos, B, Bp, Dpad,
+                            inv_tau, unit_begin, unit_end, total, nullptr, S(stream), 1);
 }
 int snag_icl_g_from_e(const uint16_t* E, int32_t side, int32_t B, int32_t Bp, const float* cr_this, const float* cr_other,
                       const float* diag, float inv_tau, uint16_t* G, void* stream) {
@@ -422,6 +436,17 @@ int snag_icl_bwd_logits(const uint16_t* X, const uint16_t* Y, int32_t B, int32_t
                         int32_t self_cols, float ebar, void* stream) {
   return launch_icl_bwd_logits(BF(X), BF(Y), B, Bp, row0, nx, Dpad, inv_tau, cr, cc, dg,
                                reinterpret_cast<__nv_bfloat16*>(G), self_cols, ebar, S(stream));
+}
+
+int snag_icl_rowsum_split(const uint16_t* X, const uint16_t* Y, int32_t B, int32_t Bp, int32_t row0, int32_t nx, int32_t Dpad,
+                          float inv_tau, float* rowsum_part, float* pos, void* stream) {
+  return launch_icl_rowsum_split(BF(X), BF(Y), B, Bp, row0, nx, Dpad, inv_tau, rowsum_part, pos, S(stream));
+}
+int snag_icl_bwd_logits_split(const uint16_t* X, const uint16_t* Y, int32_t B, int32_t Bp, int32_t row0, int32_t nx,
+                              int32_t Dpad, float inv_tau, const float* cr, const float* cc, const float* dg, uint16_t* G3,
+                              void* stream) {
+  return launch_icl_bwd_logits_split(BF(X), BF(Y), B, Bp, row0, nx, Dpad, inv_tau, cr, cc, dg,
+                                     reinterpret_cast<__nv_bfloat16*>(G3), S(stream));
 }
 
 }  // extern "C"

@@ -432,6 +432,55 @@ __global__ void __launch_bounds__(256) icl_stack_prep_kernel(const __grid_consta
   prep_row<KEEP, false>(src, D, Dpad, normalize, dst, dst2, lane, vec4);
 }
 
+// Split stacks of the fp32 loss route: row r of [a ; b ; a] as [m | h | h | m | h] (5 Dpad bf16 per row), h = bf16(z),
+// m = bf16(z - h), z normalised with prep_split_kernel's arithmetic step for step (so h is bit for bit what
+// icl_stack_prep_kernel writes and m what prep_split_kernel writes). The side-0 window (columns [0, 3 Dpad)) is
+// [m | h | h], the side-1 window (columns [2 Dpad, 5 Dpad)) is [h | m | h]: a contraction of a side-0 row with a side-1
+// row forms m_i h_j + h_i m_j + h_i h_j. One warp per row of [a ; b]; the warp of row i of part a also writes the repeated
+// row 2 Bp + i. a.Dpad[p] is the width of one block (Dpad of the table).
+__global__ void __launch_bounds__(256) icl_stack_prep_split_kernel(const __grid_constant__ StackPrepArgs a,
+                                                                   const long long* __restrict__ idx_l,
+                                                                   const long long* __restrict__ idx_r, int B, int Bp,
+                                                                   int normalize) {
+  const int p = blockIdx.y;
+  const int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (r >= 2 * Bp) return;
+  const int part = r >= Bp ? 1 : 0, i = r - part * Bp;
+  const int D = a.D[p], Dpad = a.Dpad[p];
+  const long long ld = 5ll * Dpad;
+  __nv_bfloat16* dst = a.out[p] + static_cast<long long>(r) * ld;
+  __nv_bfloat16* dst2 = part == 0 ? dst + 2ll * Bp * ld : nullptr;
+  const float* src = i < B ? a.emb[p] + (part == 1 ? idx_r[i] : idx_l[i]) * a.ld[p] : nullptr;
+  float denom = 1.0f;
+  if (src && normalize) {
+    const bool vec4 = (D % 4 == 0) && (a.ld[p] % 4 == 0) && ((reinterpret_cast<uintptr_t>(a.emb[p]) & 15) == 0);
+    float ss = 0.f;
+    if (vec4) {
+      const float4* s4 = reinterpret_cast<const float4*>(src);
+      for (int c4 = lane; c4 < (D >> 2); c4 += 32) {
+        const float4 t = __ldg(s4 + c4);
+        ss = __fmaf_rn(t.x, t.x, ss); ss = __fmaf_rn(t.y, t.y, ss); ss = __fmaf_rn(t.z, t.z, ss); ss = __fmaf_rn(t.w, t.w, ss);
+      }
+    } else {
+      for (int c = lane; c < D; c += 32) { const float v = __ldg(src + c); ss = __fmaf_rn(v, v, ss); }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    denom = fmaxf(sqrtf(ss), 1e-12f);
+  }
+  for (int c = lane; c < Dpad; c += 32) {
+    float v = 0.f;
+    if (src && c < D) v = normalize ? __fdiv_rn(__ldg(src + c), denom) : __ldg(src + c);
+    const __nv_bfloat16 h = __float2bfloat16_rn(v);
+    const __nv_bfloat16 m = __float2bfloat16_rn(__fsub_rn(v, __bfloat162float(h)));
+    dst[c] = m; dst[Dpad + c] = h; dst[2 * Dpad + c] = h; dst[3 * Dpad + c] = m; dst[4 * Dpad + c] = h;
+    if (dst2) {
+      dst2[c] = m; dst2[Dpad + c] = h; dst2[2 * Dpad + c] = h; dst2[3 * Dpad + c] = m; dst2[4 * Dpad + c] = h;
+    }
+  }
+}
+
 struct ScatterManyArgs {
   const float* emb[MANY_MAX];
   long long ld[MANY_MAX];
@@ -1852,6 +1901,22 @@ int launch_icl_stack_prep(int n_prob, const float* const* emb, const long long* 
   const unsigned gx = static_cast<unsigned>((2ll * Bp * 32 + 255) / 256);
   if (n_narrow) icl_stack_prep_kernel<4><<<dim3(gx, static_cast<unsigned>(n_narrow)), 256, 0, st>>>(narrow, idx_l, idx_r, B, Bp, normalize);
   if (n_wide) icl_stack_prep_kernel<16><<<dim3(gx, static_cast<unsigned>(n_wide)), 256, 0, st>>>(wide, idx_l, idx_r, B, Bp, normalize);
+  return static_cast<int>(cudaGetLastError());
+}
+int launch_icl_stack_prep_split(int n_prob, const float* const* emb, const long long* ld, const int* D, __nv_bfloat16* const* out,
+                                const int* Dpad, const long long* idx_l, const long long* idx_r, int B, int Bp, int normalize,
+                                cudaStream_t st) {
+  if (n_prob < 1 || n_prob > MANY_MAX || !emb || !ld || !D || !out || !Dpad || !idx_l || !idx_r) return SNAG_ERR_ARG;
+  if (B <= 0 || Bp < B || (Bp % 256) != 0) return SNAG_ERR_ARG;
+  StackPrepArgs a{};
+  for (int p = 0; p < n_prob; ++p) {
+    if (!emb[p] || !out[p] || D[p] <= 0 || ld[p] < D[p]) return SNAG_ERR_ARG;
+    if (Dpad[p] < D[p] || (Dpad[p] % 64) != 0) return SNAG_ERR_SHAPE;
+    if (reinterpret_cast<uintptr_t>(out[p]) & 127) return SNAG_ERR_ALIGN;
+    a.emb[p] = emb[p]; a.ld[p] = ld[p]; a.out[p] = out[p]; a.D[p] = D[p]; a.Dpad[p] = Dpad[p];
+  }
+  const unsigned gx = static_cast<unsigned>((2ll * Bp * 32 + 255) / 256);
+  icl_stack_prep_split_kernel<<<dim3(gx, static_cast<unsigned>(n_prob)), 256, 0, st>>>(a, idx_l, idx_r, B, Bp, normalize);
   return static_cast<int>(cudaGetLastError());
 }
 int launch_normalize_bwd_scatter_many(int n_prob, const float* const* emb, const long long* ld, const int* D,

@@ -23,6 +23,7 @@
 // Mainloop as sim_kernel (simgemm.cuh): TMA producer warp -> 4-stage ring of (128 x 64 | 256 x 64) bf16 k-blocks,
 // single-thread tcgen05.mma 128x256x16 issuer, fp32 accumulator double-buffered in TMEM, FS_WG epilogue warpgroups
 // owning 256 / FS_WG columns each.
+#include <cstddef>
 #include <mutex>
 #include "common.cuh"
 #include "snag_internal.h"
@@ -76,8 +77,10 @@ struct FsParams {
   int n_prob, kblocks;
   int unit_begin, unit_end;    // this launch's share of the n_prob * units_per_prob units
   float scale_log2;            // log2(e) / tau
+  int koff_b;                  // split stacks: column of the side-1 window (2 Dpad); fits the padding before prob
   FsProblem prob[FS_MAX_PROB];
 };
+static_assert(offsetof(FsParams, prob) == 64, "FsParams header");
 
 // ---- closed-form enumeration of the staircase --------------------------------------------------
 // Column tiles are cut into G = ceil(C / T) chunks of T tiles, aligned globally: chunk gch = tiles [gch T, (gch + 1) T).
@@ -127,7 +130,13 @@ __device__ __forceinline__ float fs_transpose_sum(float (&v)[32], int lane) {
   return v[0];
 }
 
-__global__ void __launch_bounds__(FS_THREADS, 1) icl_fwd_sym_kernel(const __grid_constant__ FsParams p) {
+// kSplit: the tables are split stacks (snag_icl_stack_prep_split, [m | h | h | m | h] rows of 5 Dpad): the A rows of a
+// tile are read from the side-0 window (columns [0, 3 Dpad)) and the B rows from the side-1 window (columns
+// [2 Dpad, 5 Dpad), p.koff_b further), so every element is m_i h_j + h_i m_j + h_i h_j — symmetric in (i, j), like the
+// bf16 Gram matrix, so the staircase, both sums and pos are unchanged. No E is saved (bf16 E would cap dL/dlogits at
+// 2^-9 relative).
+template <bool kSplit>
+__device__ __forceinline__ void icl_fwd_sym_body(const FsParams& p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
   const uint32_t base = (raw_addr + 1023u) & ~1023u;
@@ -179,8 +188,9 @@ __global__ void __launch_bounds__(FS_THREADS, 1) icl_fwd_sym_kernel(const __grid
             mbar_expect_tx(full_bar(stage), FS_STAGE_BYTES);
             const uint32_t sa = base + stage * FS_STAGE_BYTES;
             tma_load_2d(sa, tm, full_bar(stage), kb * FS_BK, u.rb * FS_BM);
-            tma_load_2d(sa + FS_A_BYTES, tm, full_bar(stage), kb * FS_BK, ct * FS_BN);
-            tma_load_2d(sa + FS_A_BYTES + FS_A_BYTES, tm, full_bar(stage), kb * FS_BK, ct * FS_BN + FS_BM);
+            const int kb_b = kb * FS_BK + (kSplit ? p.koff_b : 0);
+            tma_load_2d(sa + FS_A_BYTES, tm, full_bar(stage), kb_b, ct * FS_BN);
+            tma_load_2d(sa + FS_A_BYTES + FS_A_BYTES, tm, full_bar(stage), kb_b, ct * FS_BN + FS_BM);
           }
           __syncwarp();
           if (++stage == FS_STAGES) { stage = 0; phase ^= 1; }
@@ -284,7 +294,7 @@ __global__ void __launch_bounds__(FS_THREADS, 1) icl_fwd_sym_kernel(const __grid
               if (has_pos && row_ok && j == i + g.Bp) pr.pos[idx_i] = sv;
             }
           }
-          if (pr.esave != nullptr) {
+          if (!kSplit && pr.esave != nullptr) {
             uint32_t pk[16];
 #pragma unroll
             for (int q = 0; q < 32; q += 2) {
@@ -318,6 +328,13 @@ __global__ void __launch_bounds__(FS_THREADS, 1) icl_fwd_sym_kernel(const __grid
     tc_fence_after();
     tmem_dealloc(tmem_base, FS_ACC * FS_BN);
   }
+}
+
+__global__ void __launch_bounds__(FS_THREADS, 1) icl_fwd_sym_kernel(const __grid_constant__ FsParams p) {
+  icl_fwd_sym_body<false>(p);
+}
+__global__ void __launch_bounds__(FS_THREADS, 1) icl_fwd_sym_split_kernel(const __grid_constant__ FsParams p) {
+  icl_fwd_sym_body<true>(p);
 }
 
 // total[prob][r] = sum of the row partials of r's chunks + sum of the column partials of the row blocks whose tile
@@ -401,8 +418,9 @@ int icl_fwd_sym_plan(int n_prob, int B, int Bp, long long* out) {
 
 int launch_icl_fwd_sym(int n_prob, const __nv_bfloat16* const* S3, float* const* rowpart, float* const* colpart, float* pos,
                        int B, int Bp, int Dpad, float inv_tau, int unit_begin, int unit_end, float* total,
-                       __nv_bfloat16* const* esave, cudaStream_t st) {
+                       __nv_bfloat16* const* esave, cudaStream_t st, int split) {
   if (!S3 || !rowpart || !colpart || !pos || !total) return SNAG_ERR_ARG;
+  if (split && esave) return SNAG_ERR_ARG;
   if (Dpad <= 0 || (Dpad % FS_BK) != 0) return SNAG_ERR_SHAPE;
   if (!device_is_sm100()) return SNAG_ERR_DEVICE;
   FsParams p{};
@@ -411,14 +429,15 @@ int launch_icl_fwd_sym(int n_prob, const __nv_bfloat16* const* S3, float* const*
   const int n_units = p.g.units_per_prob * n_prob;
   if (unit_begin < 0 || unit_end > n_units || unit_begin > unit_end) return SNAG_ERR_ARG;
   p.n_prob = n_prob;
-  p.kblocks = Dpad / FS_BK;
+  p.kblocks = (split ? 3 : 1) * Dpad / FS_BK;
+  p.koff_b = split ? 2 * Dpad : 0;
   p.unit_begin = unit_begin;
   p.unit_end = unit_end;
   p.scale_log2 = inv_tau * 1.4426950408889634f;
   FsTotalArgs ta{};
   for (int i = 0; i < n_prob; ++i) {
     if (!S3[i] || !rowpart[i] || !colpart[i]) return SNAG_ERR_ARG;
-    if ((rc = make_operand_map(&p.prob[i].tm, S3[i], 2ll * Bp, Dpad, FS_BM))) return rc;
+    if ((rc = make_operand_map(&p.prob[i].tm, S3[i], 2ll * Bp, (split ? 5 : 1) * Dpad, FS_BM))) return rc;
     p.prob[i].rowpart = rowpart[i];
     p.prob[i].colpart = colpart[i];
     p.prob[i].pos = pos + static_cast<long long>(i) * Bp;
@@ -428,12 +447,12 @@ int launch_icl_fwd_sym(int n_prob, const __nv_bfloat16* const* S3, float* const*
     ta.colpart[i] = colpart[i];
   }
   if (unit_end > unit_begin) {
-    const cudaError_t attr_err =
-        cudaFuncSetAttribute(icl_fwd_sym_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FS_SMEM_BYTES);
+    auto* kern = split ? icl_fwd_sym_split_kernel : icl_fwd_sym_kernel;
+    const cudaError_t attr_err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FS_SMEM_BYTES);
     if (attr_err != cudaSuccess) return static_cast<int>(attr_err);
     const int span = unit_end - unit_begin;
     const int grid = span < num_sms() ? span : num_sms();
-    icl_fwd_sym_kernel<<<grid, FS_THREADS, FS_SMEM_BYTES, st>>>(p);
+    kern<<<grid, FS_THREADS, FS_SMEM_BYTES, st>>>(p);
   }
   icl_sym_total_kernel<<<dim3((2 * Bp + 255) / 256, n_prob), 256, 0, st>>>(ta, p.g, unit_begin, unit_end, total);
   return static_cast<int>(cudaGetLastError());

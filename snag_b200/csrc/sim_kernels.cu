@@ -130,13 +130,15 @@ static void load_encode() {
     g_encode = reinterpret_cast<EncodeTiledFn>(fn);
 }
 
-// bf16 row-major [rows, Dpad] operand, box = [box_rows x 64 elements], 128-byte swizzle, zero OOB fill
-int make_operand_map(CUtensorMap* m, const __nv_bfloat16* ptr, long long rows, int Dpad, int box_rows) {
+// bf16 row-major [rows, Dpad] operand whose rows lie ld >= Dpad elements apart (a column window of a wider matrix),
+// box = [box_rows x 64 elements], 128-byte swizzle, zero OOB fill
+static int make_operand_map_ld(CUtensorMap* m, const __nv_bfloat16* ptr, long long rows, int Dpad, long long ld, int box_rows) {
   std::call_once(g_encode_once, load_encode);
   if (!g_encode) return SNAG_ERR_DRIVER;
   if (reinterpret_cast<uintptr_t>(ptr) & 127) return SNAG_ERR_ALIGN;
+  if (ld != Dpad && (ld < Dpad || (ld % 8) != 0)) return SNAG_ERR_SHAPE;     // TMA: 16-byte row strides
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(Dpad), static_cast<cuuint64_t>(rows)};
-  const cuuint64_t strides[1] = {static_cast<cuuint64_t>(Dpad) * 2};
+  const cuuint64_t strides[1] = {static_cast<cuuint64_t>(ld) * 2};
   const cuuint32_t box[2] = {static_cast<cuuint32_t>(BK), static_cast<cuuint32_t>(box_rows)};
   const cuuint32_t estr[2] = {1, 1};
   const CUresult r = g_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(ptr), dims, strides, box,
@@ -144,27 +146,31 @@ int make_operand_map(CUtensorMap* m, const __nv_bfloat16* ptr, long long rows, i
                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? SNAG_OK : SNAG_ERR_DRIVER;
 }
+int make_operand_map(CUtensorMap* m, const __nv_bfloat16* ptr, long long rows, int Dpad, int box_rows) {
+  return make_operand_map_ld(m, ptr, rows, Dpad, Dpad, box_rows);
+}
 
 // development aid: when set (snag_debug_counters), every sweep's UMMA issuer records its wait cycles per CTA
 static unsigned long long* g_dbg_counters = nullptr;
 void set_debug_counters(unsigned long long* p) { g_dbg_counters = p; }
 
 // xt_ld > 0: X is given transposed, as a [Dpad rows, xt_ld columns] matrix whose first n1 columns are the operand
-// (SimShape::a_mn)
+// (SimShape::a_mn). row_ld > 0: the rows of X and Y lie row_ld elements apart (column windows of the loss's split stacks)
 template <class Epi>
 static int launch_sim(const __nv_bfloat16* X, const __nv_bfloat16* Y, int n1, int n2, int Dpad,
-                      const typename Epi::Params& ep, cudaStream_t st, int ksplits = 1, int xt_ld = 0) {
+                      const typename Epi::Params& ep, cudaStream_t st, int ksplits = 1, int xt_ld = 0, int row_ld = 0) {
   if (!X || !Y) return SNAG_ERR_ARG;
   if (!device_is_sm100()) return SNAG_ERR_DEVICE;
   SimPlan pl;
   int rc = make_plan(n1, n2, Dpad, &pl);
   if (rc) return rc;
   CUtensorMap tmX, tmY;
+  const int ld = row_ld > 0 ? row_ld : Dpad;
   if (xt_ld > 0) {
-    if ((xt_ld % 64) != 0 || xt_ld < n1) return SNAG_ERR_SHAPE;
+    if ((xt_ld % 64) != 0 || xt_ld < n1 || row_ld > 0) return SNAG_ERR_SHAPE;
     if ((rc = make_operand_map(&tmX, X, Dpad, xt_ld, 64))) return rc;
-  } else if ((rc = make_operand_map(&tmX, X, n1, Dpad, BM))) return rc;
-  if ((rc = make_operand_map(&tmY, Y, n2, Dpad, BN))) return rc;
+  } else if ((rc = make_operand_map_ld(&tmX, X, n1, Dpad, ld, BM))) return rc;
+  if ((rc = make_operand_map_ld(&tmY, Y, n2, Dpad, ld, BN))) return rc;
   // the attribute is per device; setting it on every call is cheap and covers multi-device processes
   const cudaError_t attr_err =
       cudaFuncSetAttribute(sim_kernel<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, SIM_SMEM_BYTES);
@@ -311,6 +317,16 @@ int launch_icl_rowsum(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B, int
   return launch_sim<EpiIclFwd>(X, Y, nx, 2 * Bp, Dpad, p, st);
 }
 
+// launch_icl_rowsum on split stacks (rows of 5 Dpad, see snag_icl_stack_prep_split): X at a side-0 window, Y at a
+// side-1 window, contraction width 3 Dpad
+int launch_icl_rowsum_split(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B, int Bp, int row0, int nx, int Dpad,
+                            float inv_tau, float* rowsum_part, float* pos, cudaStream_t st) {
+  if (!rowsum_part || !pos || B <= 0 || Bp < B || (Bp % BN) != 0 || Dpad <= 0 || (Dpad % 64) != 0) return SNAG_ERR_ARG;
+  if (row0 < 0 || nx <= 0 || row0 + nx > Bp) return SNAG_ERR_ARG;
+  EpiIclFwd::Params p{inv_tau * 1.4426950408889634f, B, Bp, row0, nx, rowsum_part, pos};
+  return launch_sim<EpiIclFwd>(X, Y, nx, 2 * Bp, 3 * Dpad, p, st, 1, 0, 5 * Dpad);
+}
+
 int launch_eval_rowcoltopk(const __nv_bfloat16* X, const __nv_bfloat16* Y, const float* xn, const float* yn, int n1, int n2,
                            int Dpad, float* part, int* part_idx, const float* rowthr, const float* colthr, const float* colb,
                            uint2* stream, int* stream_row, int* stream_cnt, int cta_cap, float norm2_max, cudaStream_t st) {
@@ -363,6 +379,17 @@ int launch_icl_bwd_logits(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B,
   if (reinterpret_cast<uintptr_t>(G) & 15) return SNAG_ERR_ALIGN;
   EpiIclBwd::Params p{inv_tau * 1.4426950408889634f, inv_tau, B, Bp, row0, nx, cr, cc, dg, G, self_cols, ebar};
   return launch_sim<EpiIclBwd>(X, Y, nx, 2 * Bp, Dpad, p, st);
+}
+
+// dL/dlogits on split stacks (windows as launch_icl_rowsum_split), written as G3 = [G_h | G_h | G_m] [nx, 6 Bp]
+int launch_icl_bwd_logits_split(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B, int Bp, int row0, int nx, int Dpad,
+                                float inv_tau, const float* cr, const float* cc, const float* dg, __nv_bfloat16* G3,
+                                cudaStream_t st) {
+  if (!cr || !cc || !dg || !G3 || B <= 0 || Bp < B || (Bp % BN) != 0 || Dpad <= 0 || (Dpad % 64) != 0) return SNAG_ERR_ARG;
+  if (row0 < 0 || nx <= 0 || row0 + nx > Bp) return SNAG_ERR_ARG;
+  if (reinterpret_cast<uintptr_t>(G3) & 31) return SNAG_ERR_ALIGN;
+  EpiIclBwdSplit::Params p{inv_tau * 1.4426950408889634f, inv_tau, B, Bp, row0, nx, cr, cc, dg, G3, 1, 0.f};
+  return launch_sim<EpiIclBwdSplit>(X, Y, nx, 2 * Bp, 3 * Dpad, p, st, 1, 0, 5 * Dpad);
 }
 
 }  // namespace snag

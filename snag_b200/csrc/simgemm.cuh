@@ -1678,4 +1678,69 @@ struct EpiIclBwd {
   static __device__ __forceinline__ void unit_end(const Params&, const SimShape&, const EpiCtx&, State&) {}
 };
 
+// ------------------------------------------------------------------------------------------------
+// Epilogue: ICL backward of the fp32 loss route. The logits tile comes from split operands (X rows [m | h | h], Y rows
+// [h | m | h]), G is formed in fp32 registers exactly as EpiIclBwd forms it (the cross diagonal -dg/tau included), and
+// stored as two bf16 terms, G3 = [G_h | G_h | G_m] ([nx, 6 Bp], G_h = bf16(G), G_m = bf16(G - G_h), the difference exact
+// in fp32): the gradient GEMM over K = 6 Bp against the K-stacked rows [Y_h ; Y_m ; Y_h] then forms
+// G_h Y_h + G_h Y_m + G_m Y_h, which leaves out G_m Y_m (<= 2^-16 |G| |Y|) and the residual of the two-term split of G
+// (<= 2^-16 |G|). Every 32-byte piece is written with one 256-bit store, as in EpiIclBwd.
+// ------------------------------------------------------------------------------------------------
+struct EpiIclBwdSplit : EpiIclBwd {
+  // EpiIclBwd::half_strip without the rounding: the 16 fp32 values of G
+  static __device__ __forceinline__ void half_strip_f32(const Params& p, const State& st, const float* cc_s,
+                                                        const uint32_t (&r)[32], int q0, int idx0, int part, bool plain,
+                                                        float (&v)[16]) {
+    const float nb = -p.scale_log2;
+    float cc[16];
+#pragma unroll
+    for (int q = 0; q < 16; q += 4) {
+      const float4 t = *reinterpret_cast<const float4*>(cc_s + q0 + q);
+      cc[q] = t.x; cc[q + 1] = t.y; cc[q + 2] = t.z; cc[q + 3] = t.w;
+    }
+#pragma unroll
+    for (int q = 0; q < 16; ++q) {
+      const float E = ex2_approx(__fmaf_rn(__uint_as_float(r[q0 + q]), p.scale_log2, nb)) - p.ebar;
+      float gval = (st.cr + cc[q]) * E;
+      if (!plain) {
+        const int idx = idx0 + q0 + q;
+        if (idx == st.gr) gval = part ? 0.f : gval - st.dg;
+        if (!st.ok || idx >= p.B) gval = 0.f;
+      }
+      v[q] = gval;
+    }
+  }
+  static __device__ __forceinline__ void chunk(const Params& p, const SimShape&, const EpiCtx& cx, State& st, int ct,
+                                               int c, const uint32_t (&r)[32], int buf) {
+    const float* cc_s = cx.scratch + buf * BN + c * 32;
+    const int col0 = ct * BN + c * 32;
+    const int part = col0 >= p.Bp ? 1 : 0;
+    const int idx0 = col0 - part * p.Bp;
+    const int gr0 = p.row0 + cx.rb * BM;
+    const bool plain = (gr0 + BM <= p.B) && ((cx.rb + 1) * BM <= p.nx) && (idx0 + 32 <= p.B) &&
+                       (idx0 + 31 < gr0 || idx0 > gr0 + BM - 1);
+    const long long twoBp_bytes = 4ll * p.Bp;                  // bytes between the three column blocks of G3
+    uint8_t* dst = reinterpret_cast<uint8_t*>(p.G + static_cast<long long>(cx.row) * (6 * p.Bp) + col0);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      float v[16];
+      half_strip_f32(p, st, cc_s, r, 16 * h, idx0, part, plain, v);
+      uint32_t hi[8], lo[8];
+#pragma unroll
+      for (int q = 0; q < 16; q += 2) {
+        const __nv_bfloat162 g2 = __floats2bfloat162_rn(v[q], v[q + 1]);
+        const __nv_bfloat162 m2 = __floats2bfloat162_rn(__fsub_rn(v[q], __low2float(g2)), __fsub_rn(v[q + 1], __high2float(g2)));
+        hi[q / 2] = *reinterpret_cast<const uint32_t*>(&g2);
+        lo[q / 2] = *reinterpret_cast<const uint32_t*>(&m2);
+      }
+      if (cx.row_ok) {
+        const uint4 h0 = make_uint4(hi[0], hi[1], hi[2], hi[3]), h1 = make_uint4(hi[4], hi[5], hi[6], hi[7]);
+        st_global_256(dst + 32 * h, h0, h1);
+        st_global_256(dst + twoBp_bytes + 32 * h, h0, h1);
+        st_global_256(dst + 2 * twoBp_bytes + 32 * h, make_uint4(lo[0], lo[1], lo[2], lo[3]), make_uint4(lo[4], lo[5], lo[6], lo[7]));
+      }
+    }
+  }
+};
+
 }  // namespace snag

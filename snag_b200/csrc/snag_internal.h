@@ -87,7 +87,7 @@ int launch_icl_bwd_fused(int n_prob, const __nv_bfloat16* const* S3, const float
 int icl_fwd_sym_plan(int n_prob, int B, int Bp, long long* out);
 int launch_icl_fwd_sym(int n_prob, const __nv_bfloat16* const* S3, float* const* rowpart, float* const* colpart, float* pos,
                        int B, int Bp, int Dpad, float inv_tau, int unit_begin, int unit_end, float* total,
-                       __nv_bfloat16* const* esave, cudaStream_t st);
+                       __nv_bfloat16* const* esave, cudaStream_t st, int split = 0);
 int launch_icl_g_from_e(const __nv_bfloat16* E, int side, int B, int Bp, const float* cr_this, const float* cr_other,
                         const float* diag, float inv_tau, __nv_bfloat16* G, cudaStream_t st);
 int launch_icl_sym_finalize(const float* total, const float* pos, int n_prob, int B, int Bp, float inv_tau, float* out,
@@ -182,5 +182,14 @@ int launch_col_cand_finalize(const long long* offs, const int* hist, const float
                              float* nv, float* cand_val, int* cand_idx, int* overflow, cudaStream_t st);
 int launch_icl_bwd_logits(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B, int Bp, int row0, int nx, int Dpad, float inv_tau,
                           const float* cr, const float* cc, const float* dg, __nv_bfloat16* G, int self_cols, float ebar, cudaStream_t st);
+// the fp32 loss route: split stacks [3 Bp, 5 Dpad] rows [m | h | h | m | h] (bw_kernels.cu / sim_kernels.cu)
+int launch_icl_stack_prep_split(int n_prob, const float* const* emb, const long long* ld, const int* D, __nv_bfloat16* const* out,
+                                const int* Dpad, const long long* idx_l, const long long* idx_r, int B, int Bp, int normalize,
+                                cudaStream_t st);
+int launch_icl_rowsum_split(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B, int Bp, int row0, int nx, int Dpad,
+                            float inv_tau, float* rowsum_part, float* pos, cudaStream_t st);
+int launch_icl_bwd_logits_split(const __nv_bfloat16* X, const __nv_bfloat16* Y, int B, int Bp, int row0, int nx, int Dpad,
+                                float inv_tau, const float* cr, const float* cc, const float* dg, __nv_bfloat16* G3,
+                                cudaStream_t st);
 
 }  // namespace snag

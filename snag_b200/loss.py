@@ -17,6 +17,7 @@ of both sets, the target probabilities written once in bf16 and contracted with 
 """
 from __future__ import annotations
 
+import copy
 import os
 
 import numpy as np
@@ -165,6 +166,20 @@ SYM_FORWARD = os.environ.get("SNAG_SYM_FORWARD", "1") != "0"
 # matrix in bf16 ([2Bp, 2Bp]: 2 GB per table at B = 16 384) and the backward forms dL/dlogits from it with a bandwidth
 # kernel instead of a second pass over the 1200- / 1800-wide contraction. Single rank only (off: recompute).
 SAVE_E = os.environ.get("SNAG_SAVE_E", "1") != "0"
+
+# What icl_loss contracts (read at every call; icl_loss.forward_many(precision=) and SnagLossLayer(precision=) override
+# it per call / per layer): "bf16" rounds the normalised rows to bf16 before every contraction (losses within ~5e-3
+# relative of the reference's fp32 arithmetic, gradients within ~2e-2); "fp32" contracts a three-term bf16 split of the
+# unrounded rows (snag_b200.loss_fp32: 3x the contraction width, two-kernel backward at every width). ial_loss stays bf16
+# (SNAG never calls it).
+TRAIN_PRECISION = "bf16"
+PRECISIONS = ("bf16", "fp32")
+
+
+def _check_precision(precision: str) -> str:
+    if precision not in PRECISIONS:
+        raise ValueError(f"precision={precision!r}: expected one of {PRECISIONS}")
+    return precision
 
 
 class _IclMany(torch.autograd.Function):
@@ -396,12 +411,28 @@ class icl_loss(nn.Module):
         self.inversion = inversion
         self.neg_cross_kg = neg_cross_kg
         self.shard = None            # AnchorShard, see distribute()
+        self.fp32_be = None          # kernel backend of the fp32 route (None: snag_b200.loss_fp32; tests: a CPU stand-in)
+        self._fp32_shard = None      # (shard it was made from, the same shard with the fp32 backend)
 
     def distribute(self, group, grads: str = "gather", be=None):
         """Shard the anchors of every following forward over the ranks of `group` (SURVEY 8(e); BASELINE configs[4]).
         Every rank must call forward with the same batch; the returned loss is identical on all ranks."""
         self.shard = None if group is None else AnchorShard(group, grads, be)
+        self._fp32_shard = None
         return self
+
+    def _shard_for(self, precision: str) -> AnchorShard:
+        """The anchor shard of this loss with the kernel backend of `precision`."""
+        base = self.shard or _unsharded()
+        if precision == "bf16":
+            return base
+        from . import loss_fp32
+        be = loss_fp32 if self.fp32_be is None else self.fp32_be
+        if self._fp32_shard is None or self._fp32_shard[0] is not base or self._fp32_shard[1].be is not be:
+            sh = copy.copy(base)                  # same group, ranks and exchanges; only the kernels differ
+            sh.be = be
+            self._fp32_shard = (base, sh)
+        return self._fp32_shard[1]
 
     def forward(self, emb, train_links, neg_l=None, neg_r=None, weight_norm=None, norm=True):
         if neg_l is not None or neg_r is not None:
@@ -414,10 +445,12 @@ class icl_loss(nn.Module):
                                f"(model/SNAG_loss.py:84-89 raises as well)")
         return self.forward_many([emb], train_links, [weight_norm], norm=norm)[0]
 
-    def forward_many(self, embs, train_links, weight_norms=None, norm=True):
+    def forward_many(self, embs, train_links, weight_norms=None, norm=True, precision=None):
         """The same loss for several embedding tables that share the batch `train_links` (what one SNAG step does 2 + 2M
         times, model/SNAG.py:106,147-159): returns one scalar per table, each equal to forward(emb, train_links,
-        weight_norm=w). One autograd node covers all tables, so their backward sweeps are batched into one launch."""
+        weight_norm=w). One autograd node covers all tables, so their backward sweeps are batched into one launch.
+        precision: "bf16" or "fp32" (None: TRAIN_PRECISION at the time of the call)."""
+        precision = _check_precision(TRAIN_PRECISION if precision is None else precision)
         if self.inversion:
             raise NotImplementedError("inversion=True is unreachable from SNAG (model/SNAG.py:50-51)")
         if self.n_view != 2:
@@ -442,7 +475,7 @@ class icl_loss(nn.Module):
                                  f"{inv_tau:.3g}, beyond the fused kernels' range of {MAX_INV_TAU:g}")
             embs = [e * (2.0 ** -e2) for e in embs]
         # normalising only the 2B gathered rows equals normalising all N first (model/SNAG_loss.py:60-64), row by row
-        nll = _IclMany.apply(idx_l, idx_r, inv_tau, self.shard or _unsharded(), bool(norm), *embs)
+        nll = _IclMany.apply(idx_l, idx_r, inv_tau, self._shard_for(precision), bool(norm), *embs)
         batch = idx_l.numel()
         alpha = self.weight
         # softXEnt (:42-54) and the alpha mix (:126) for all tables at once — the same elementwise operations and one
@@ -628,9 +661,11 @@ class SnagLossLayer(nn.Module):
 
     WEIGHT_COLUMN = (3, 2, 1, 0, 4, 5)      # model/SNAG.py:145-150: gph<-w[:,3], rel<-w[:,2], att<-w[:,1], img<-w[:,0], ...
 
-    def __init__(self, tau=0.1, ab_weight=0.5, awloss=False):
+    def __init__(self, tau=0.1, ab_weight=0.5, awloss=False, precision=None):
         super().__init__()
         self.awloss = awloss
+        # what the icl_loss calls contract ("bf16" / "fp32"; None: loss.TRAIN_PRECISION at the time of each call)
+        self.precision = None if precision is None else _check_precision(precision)
         self.multi_loss_layer = CustomMultiLossLayer(loss_num=6)                         # model/SNAG.py:48
         self.multi_loss_layer_2 = AutomaticWeightedLoss(num=7)                           # :49
         self.criterion_cl = icl_loss(tau=tau, ab_weight=ab_weight, n_view=2)             # :50
@@ -647,7 +682,8 @@ class SnagLossLayer(nn.Module):
             present = [(emb, col) for emb, col in zip(streams, self.WEIGHT_COLUMN) if emb is not None]
             wn = None if weight_norm is None else weight_norm * weight_norm.shape[1]
             vals = self.criterion_cl.forward_many([e for e, _ in present], train_ill,
-                                                  [None if wn is None else wn[:, c] for _, c in present])
+                                                  [None if wn is None else wn[:, c] for _, c in present],
+                                                  precision=self.precision)
             it = iter(vals)
             losses = [0 if emb is None else next(it) for emb in streams]
         return self.multi_loss_layer(losses)
@@ -659,7 +695,8 @@ class SnagLossLayer(nn.Module):
         s_pres = [(e, c) for e, c in zip(streams, self.WEIGHT_COLUMN) if e is not None]
         h_pres = [h for h in hidden if h is not None]
         vals = self.criterion_cl.forward_many([joint_emb, joint_emb_fz] + [e for e, _ in s_pres] + h_pres, batch,
-                                              [None, None] + [wn[:, c] for _, c in s_pres] + [None] * len(h_pres))
+                                              [None, None] + [wn[:, c] for _, c in s_pres] + [None] * len(h_pres),
+                                              precision=self.precision)
         gmi = vals[0] + vals[1]
         it = iter(vals[2:])
         ecia = self.inner_view_loss(streams, batch, losses=[0 if e is None else next(it) for e in streams])

@@ -782,17 +782,20 @@ ICL_SYM_MAX_PROBLEMS = 16
 
 
 def icl_fwd_sym(S3s, B: int, Bp: int, inv_tau: float, rank: int = 0, world: int = 1, all_reduce=None,
-                esave=None) -> torch.Tensor:
+                esave=None, split: bool = False) -> torch.Tensor:
     """Forward statistics of icl_loss for several tables that share the batch, on half the Gram matrix of the stacked
     rows (snag_icl_fwd_sym): S3s[p] = [a ; b ; ...] as [>= 2 Bp, Dpad] bf16 (same Dpad). Returns fp32 [n_prob, 4, B] =
     (lse_a, nll_a, lse_b, nll_b) per table. With world > 1 this rank processes its contiguous share of the work units
     and `all_reduce(tensor) -> tensor` (sum over the ranks) combines the partial sums before the logarithm.
     esave: optional list (one entry per table, None to skip) of bf16 [2 Bp, 2 Bp] buffers that receive E of every computed
-    element for icl_g_from_e (single rank only: the buffer must see all work units)."""
+    element for icl_g_from_e (single rank only: the buffer must see all work units).
+    split: S3s are the split stacks of the fp32 loss route ([3 Bp, 5 Dpad], snag_icl_fwd_sym_split; no esave)."""
     import ctypes
     n_prob = len(S3s)
     if not 1 <= n_prob <= ICL_SYM_MAX_PROBLEMS:
         raise ValueError(f"1..{ICL_SYM_MAX_PROBLEMS} tables per launch")
+    if split and esave is not None:
+        raise ValueError("esave is not available for split stacks: a bf16 E would cap dL/dlogits at 2^-9 relative")
     dpad = S3s[0].shape[1]
     for t in S3s:
         _check_operand(t, "S3")
@@ -820,10 +823,18 @@ def icl_fwd_sym(S3s, B: int, Bp: int, inv_tau: float, rank: int = 0, world: int 
         es = arr(esave)
     tiles = (2 * Bp // 256) ** 2 + 2 * Bp // 256            # per table: the staircase of 128-row blocks x 256-column tiles
     share = (u1 - u0) / max(1, units)
-    with _SweepTimer("icl_fwd_sym_kernel", int(n_prob * tiles * share) * 128, 256, dpad):
-        call("snag_icl_fwd_sym", n_prob, arr(S3s), arr([rowpart[i] for i in range(n_prob)]),
-             arr([colpart[i] for i in range(n_prob)]), ptr(pos), B, Bp, dpad, float(inv_tau), u0, u1, ptr(total), es,
-             current_stream())
+    if split:
+        if dpad % 320:
+            raise ValueError("split stacks are [3 Bp, 5 Dpad] with Dpad a multiple of 64")
+        with _SweepTimer("icl_fwd_sym_split_kernel", int(n_prob * tiles * share) * 128, 256, dpad // 5 * 3):
+            call("snag_icl_fwd_sym_split", n_prob, arr(S3s), arr([rowpart[i] for i in range(n_prob)]),
+                 arr([colpart[i] for i in range(n_prob)]), ptr(pos), B, Bp, dpad // 5, float(inv_tau), u0, u1, ptr(total),
+                 current_stream())
+    else:
+        with _SweepTimer("icl_fwd_sym_kernel", int(n_prob * tiles * share) * 128, 256, dpad):
+            call("snag_icl_fwd_sym", n_prob, arr(S3s), arr([rowpart[i] for i in range(n_prob)]),
+                 arr([colpart[i] for i in range(n_prob)]), ptr(pos), B, Bp, dpad, float(inv_tau), u0, u1, ptr(total), es,
+                 current_stream())
     if world > 1:
         buf = all_reduce(buf)
         total, pos = buf[:n_prob * 2 * Bp], buf[n_prob * 2 * Bp:]

@@ -1,6 +1,7 @@
 """Drop-in installation into an UNMODIFIED checkout of zjukg/SNAG (SNAG_MMEA).
 
-    python -m snag_b200.patch [--eval-precision fp32] [--link-precision fp32] /path/to/SNAG_MMEA [main.py flags ...]
+    python -m snag_b200.patch [--eval-precision fp32] [--link-precision fp32] [--train-precision fp32]
+                              /path/to/SNAG_MMEA [main.py flags ...]
                                                       # runs main.py with the hot path replaced
 or, from Python:
     import snag_b200.patch as sp; sp.patch()         # after SNAG_MMEA is on sys.path, before Runner is built
@@ -10,8 +11,11 @@ does, instead of their bf16 rounding (snag_b200.evaluate.EVAL_PRECISION). It gov
 --link-precision fp32 (patch(link_precision="fp32")): the two searches that choose training links — the
 iterative-learning mining of SNAG.Iter_new_links and the seed induction of visual_pivot_induction (--unsup) — run on
 the unrounded fp32 rows instead of their bf16 rounding (snag_b200.mining.LINK_PRECISION), so that the links are the
-reference's. Both options come before the reference directory, in either order, and are consumed before main.py
-parses its arguments.
+reference's.
+--train-precision fp32 (patch(train_precision="fp32")): the icl_loss calls of the training step contract a split of the
+unrounded fp32 rows instead of their bf16 rounding (snag_b200.loss.TRAIN_PRECISION), as the reference's fp32 training
+does. It governs icl_loss only: ial_loss stays bf16 (SNAG never calls it).
+The options come before the reference directory, in any order, and are consumed before main.py parses its arguments.
 
 patch() assigns attributes — main.py, model/*.py and src/*.py stay byte-identical:
     model.SNAG_loss.icl_loss / ial_loss / CustomMultiLossLayer            -> snag_b200.loss
@@ -52,14 +56,18 @@ def unpatch() -> int:
 
 
 def patch(main_module: types.ModuleType | None = None, eval_precision: str | None = None,
-          link_precision: str | None = None) -> list[str]:
+          link_precision: str | None = None, train_precision: str | None = None) -> list[str]:
     """Install the replacements into whichever reference modules are importable; returns what was patched.
     eval_precision ("bf16" or "fp32", None = leave as is): what Runner._test evaluates with.
-    link_precision (likewise): what Iter_new_links and visual_pivot_induction search with."""
+    link_precision (likewise): what Iter_new_links and visual_pivot_induction search with.
+    train_precision (likewise): what the icl_loss calls of the training step contract."""
     done = []
     for precision in (eval_precision, link_precision):
         if precision is not None:
             evaluate._check_precision(precision)
+    if train_precision is not None:
+        loss._check_precision(train_precision)
+        loss.TRAIN_PRECISION = train_precision
     if eval_precision is not None:
         evaluate.EVAL_PRECISION = eval_precision
     if link_precision is not None:
@@ -116,21 +124,24 @@ def patch(main_module: types.ModuleType | None = None, eval_precision: str | Non
 
 
 class Options(tuple):
-    """(eval_precision or None, reference directory, main.py's arguments), with the link precision (or None) as the
-    attribute link_precision: a three-tuple, so that callers which unpack parse_args' result keep working."""
+    """(eval_precision or None, reference directory, main.py's arguments), with the link and training precisions (or
+    None) as the attributes link_precision and train_precision: a three-tuple, so that callers which unpack parse_args'
+    result keep working."""
 
-    def __new__(cls, eval_precision: str | None, reference_dir: str, argv: list[str], link_precision: str | None = None):
+    def __new__(cls, eval_precision: str | None, reference_dir: str, argv: list[str], link_precision: str | None = None,
+                train_precision: str | None = None):
         self = super().__new__(cls, (eval_precision, reference_dir, argv))
         self.link_precision = link_precision
+        self.train_precision = train_precision
         return self
 
 
-_OPTIONS = ("--eval-precision", "--link-precision")
+_OPTIONS = ("--eval-precision", "--link-precision", "--train-precision")
 
 
 def parse_args(argv: list[str]) -> Options:
-    """Options from this module's command line: the options of snag_b200.patch (--eval-precision, --link-precision, in
-    any order) precede the reference directory; everything after it belongs to main.py."""
+    """Options from this module's command line: the options of snag_b200.patch (--eval-precision, --link-precision,
+    --train-precision, in any order) precede the reference directory; everything after it belongs to main.py."""
     values = dict.fromkeys(_OPTIONS)
     i = 0
     while i < len(argv) and argv[i].split("=", 1)[0] in _OPTIONS:
@@ -146,11 +157,12 @@ def parse_args(argv: list[str]) -> Options:
         values[name] = value
     if i >= len(argv):
         raise SystemExit(__doc__)
-    return Options(values["--eval-precision"], argv[i], list(argv[i + 1:]), values["--link-precision"])
+    return Options(values["--eval-precision"], argv[i], list(argv[i + 1:]), values["--link-precision"],
+                   values["--train-precision"])
 
 
 def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = None,
-             link_precision: str | None = None) -> None:
+             link_precision: str | None = None, train_precision: str | None = None) -> None:
     """Execute the reference's main.py (unchanged on disk) with the hot path patched in: the module body is executed
     first, the patch is applied (Runner now exists), then the `if __name__ == "__main__":` block runs."""
     reference_dir = os.path.abspath(reference_dir)
@@ -158,7 +170,8 @@ def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = N
     sys.path.insert(0, reference_dir)
     os.chdir(reference_dir)
     sys.argv = [path] + list(argv)
-    patch(eval_precision=eval_precision, link_precision=link_precision)    # model.*, src.* before main.py binds them
+    patch(eval_precision=eval_precision, link_precision=link_precision,     # model.*, src.* before main.py binds them
+          train_precision=train_precision)
     tree = ast.parse(open(path).read(), filename=path)
     body, tail = [], []
     for node in tree.body:
@@ -176,4 +189,4 @@ def run_main(reference_dir: str, argv: list[str], eval_precision: str | None = N
 
 if __name__ == "__main__":
     _opts = parse_args(sys.argv[1:])
-    run_main(_opts[1], _opts[2], _opts[0], _opts.link_precision)
+    run_main(_opts[1], _opts[2], _opts[0], _opts.link_precision, _opts.train_precision)
